@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: maze env-steps/s including pixel-change + returns (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--obs-dtype f32|u8]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--obs-dtype f32|u8] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1], per GPU): 4096 batched maze envs; one *step* = one pass of
@@ -19,7 +19,12 @@ scaling).  Prints ONE JSON line (rank 0).
 `cpu_baseline` the numpy oracle port of the reference path on this box's host cores.
 
 --impl reference  times the reference's CPU implementation of the path (the oracle port: the
-reference is Python and /root/reference does not exist on the GPU box) on all host cores.
+reference is Python and is not part of this repository) on all host cores.
+
+--dump-outputs DIR  after the timed steps, writes what the last timed pass of rank 0 computed as
+DIR/<name>.npy (float32 / float64, fixed samples of the larger buffers, at most about 41 MB), so
+that two builds can be compared output for output: the inputs are seeded, identical for identical
+arguments.
 """
 import argparse
 import json
@@ -60,7 +65,12 @@ def parse():
   p.add_argument("--agent-obs", default="cells", choices=["cells", "s2d", "f32"],
                  help="full-agent observations: agent cells (conv1 renders its tiles in shared memory, no frame in HBM), "
                       "K1-rendered x'' planes, or f32 frames")
-  return p.parse_args()
+  p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                 help="write the outputs of the last timed pass as DIR/<name>.npy (see dump_outputs)")
+  args = p.parse_args()
+  if args.steps < 1:
+    p.error("--steps must be at least 1")
+  return args
 
 
 def workload_config(args):
@@ -359,6 +369,35 @@ def parity_check(torch, eng, envs=64):
     return "error: " + repr(e)[:200], ""
 
 
+def dump_outputs(torch, eng, out_dir, max_envs=4096, map_envs=256, frames=256):
+  """Writes the buffers the last pass of `eng` left for its caller as out_dir/<name>.npy, about 41 MB at most.
+  reward, terminal, R, adv and frame_rec ([T, S, 2]: its low and high 32 bits, as float64 holds 53) for a sample of
+  `max_envs` envs (all of them up to that many); pc and pc_tgt for a sample of `map_envs` envs ([T, S, 20, 20]); obs
+  for a sample of `frames` (step, env) pairs in ascending order of step * N + env.  The samples are sorted and drawn
+  from RandomState(0), so they depend on N and T only."""
+  import numpy as np
+  t, n = eng.t, eng.n
+  rs = np.random.RandomState(0)
+
+  def pick(m, k):
+    return torch.from_numpy(np.sort(rs.choice(m, min(m, k), replace=False))).to(eng.device)
+
+  envs, map_sel, rows = pick(n, max_envs), pick(n, map_envs), pick(t * n, frames)
+  torch.cuda.synchronize(eng.device)
+  rec = eng.frame_rec.index_select(1, envs).cpu().numpy().view(np.uint64)
+  outs = {
+      "reward": eng.reward.index_select(1, envs), "terminal": eng.terminal.index_select(1, envs),
+      "R": eng.R.index_select(1, envs), "adv": eng.adv.index_select(1, envs),
+      "pc": eng.pc.index_select(1, map_sel), "pc_tgt": eng.pc_tgt.index_select(1, map_sel),
+      "obs": eng.obs.view(t * n, 84, 84, 3).index_select(0, rows),
+  }
+  os.makedirs(out_dir, exist_ok=True)
+  for name, v in outs.items():
+    np.save(os.path.join(out_dir, name + ".npy"), v.float().cpu().numpy())
+  np.save(os.path.join(out_dir, "frame_rec.npy"),
+          np.stack([rec & np.uint64(0xFFFFFFFF), rec >> np.uint64(32)], -1).astype(np.float64))
+
+
 def measure_pc_stress(torch, dev, peak, seq=50000, dtype_name="u8"):
   """BASELINE configs[3]: pixel-control target stress -- synthetic 84x84x3 frame stream (u8, scaled by /255 on load like
   lab / indoor / gym frames), 20x20 cells, n = 20, gamma_pc = 0.9, 1 M frames per batch: K2 (stream pixel change, every
@@ -581,6 +620,8 @@ def run_b200(args):
   k1_ms = sum(e[0].elapsed_time(e[1]) for e in evs) / (K * (1 if window else t))    # per K1 launch
   k3_ms = sum(e[1].elapsed_time(e[2]) for e in evs) / K
   k4_ms = sum(e[2].elapsed_time(e[3]) for e in evs) / K
+  if args.dump_outputs and rank == 0:
+    dump_outputs(torch, eng, args.dump_outputs)
 
   # ---- host-buffer (e2e) arm: same pass through run_host() ----
   # the caller's host buffers are the engine's pinned staging arrays (filled in place once)
@@ -590,7 +631,7 @@ def run_b200(args):
   h_act, h_val, h_bv, h_bq = hbuf["actions"], hbuf["values"], hbuf["boot_value"], hbuf["boot_q"]
   for _ in range(3):
     out = eng.run_host(h_act, h_val, h_bv, h_bq)
-  ke = max(3, min(K, 200))
+  ke = K
   e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
   barrier()
   e0.record()

@@ -1,5 +1,5 @@
-import sys, json
-sys.path.insert(0, "/root/repo")
+import sys, os, json
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from unreal_b200 import kernels as K
 dev = torch.device("cuda", 0)

@@ -212,10 +212,10 @@ def gen_trainer(name, H, n_iter, n_step_TD, seed, net_seed):
       base_adv=np.array(base_adv, np.float64), base_R=np.array(base_R, np.float64),
       pc_len=np.array(pc_len), pc_pos=np.array(pc_pos, np.uint8), pc_lar=np.array(pc_lar, np.float64),
       pc_a=np.array(pc_a, np.float64),
-      # full maps only for the first frames (size); sums + 16 probe cells for all
+      # full maps only for the first frames (size); float64 sums + 16 float32 probe cells for all
       pc_R_head=np.array(pc_R[:PC_FULL], np.float32),
       pc_R_sum=np.array([np.sum(m, dtype=np.float64) for m in pc_R]),
-      pc_R_probe=np.array([np.asarray(m, np.float64).reshape(-1)[PC_PROBE] for m in pc_R]),
+      pc_R_probe=np.array([np.asarray(m, np.float64).reshape(-1)[PC_PROBE] for m in pc_R], np.float32),
       vr_len=np.array(vr_len), vr_pos=np.array(vr_pos, np.uint8), vr_lar=np.array(vr_lar, np.float64),
       vr_R=np.array(vr_R, np.float64),
       rp_pos=np.array(rp_pos, np.uint8), rp_c=np.array(rp_c, np.float64),
@@ -329,7 +329,7 @@ def gen_lar():
   print("lar", with_obj.shape, with_obj.dtype, without.shape)
 
 
-PC_FULL = 400
+PC_FULL = 160          # keeps each trainer_*.npz under 1 MB
 PC_PROBE = np.array([0, 19, 21, 63, 105, 147, 168, 189, 210, 231, 252, 294, 336, 378, 380, 399])
 
 
