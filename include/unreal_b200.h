@@ -227,6 +227,28 @@ int unreal_rollout_post(const float* reward, const uint8_t* terminal, const uint
                         uint8_t* ended, uint64_t* last_rec, float* episode_reward, float* lstm_c, float* lstm_h,
                         double* stats, void* stream);
 
+/* ---- evaluation of a frozen policy on the maze (Evaluator, unreal_b200/train/evaluator.py) -----------------------
+ * Everything of one evaluation step after the policy, for N mazes in one launch (per-env logic in csrc/eval_core.cuh).
+ * For every env with active[e] != 0:
+ *   action    greedy != 0: argmax of pi [N,a] f32 (lowest index on ties), no draw; else RandomState.choice(a, p=pi) on
+ *             the env's stream mt [624,N] / mt_pos [N] (trainer.py:147-148, two words, as unreal_choose_action);
+ *   step      maze_environment.py:98-128 on the map of unreal_maze_set_map; pos [N,2], last_action, last_reward [N]
+ *             updated like :125-127;
+ *   episode   ep_score [N] += reward, ep_length [N] += 1; at a terminal or at max_steps steps the result row
+ *             (e, ep_index[e]) of res_score / res_length / res_finished [N,episodes] is written (finished = terminal),
+ *             ep_index advances, the env is reset as after a terminal (trainer.py:201-202, :279-296: start cell, last
+ *             action / reward 0, lstm_c / lstm_h rows [N,256] f32 zeroed, local_network.reset_state :293), and after its
+ *             `episodes`-th episode active[e] = 0;
+ *   operand   row e of the next step's GEMM operand xh bf16 [N, ld_xh] is written: columns [0,256) = fc_tab [49,256]
+ *             bf16 row of the new cell, [256, kx) = one-hot(last_action, a) ++ [last_reward] ++ zeros (objective size 0),
+ *             [kx, kx+256) = lstm_h row rounded to bf16 (nearest even).
+ * Inactive envs are not touched: no draw, no state, result, LSTM or operand write. */
+int unreal_maze_eval_act(const float* pi, int a, int greedy, uint32_t* mt, int32_t* mt_pos, int32_t* pos,
+                         int32_t* last_action, float* last_reward, float* ep_score, int32_t* ep_length, int32_t* ep_index,
+                         uint8_t* active, float* res_score, int32_t* res_length, uint8_t* res_finished, int episodes,
+                         int max_steps, float* lstm_c, float* lstm_h, const void* fc_tab_bf16, void* xh_bf16, int64_t ld_xh,
+                         int kx, int n, void* stream);
+
 /* ---- K6: shared RMSProp with global-norm clip, train/rmsprop_applier.py ---------------
  * _apply_gradients (:109-132): g <- grad * clip / max(||grad||, clip)  (tf.clip_by_global_norm :121)
  * _apply_dense (:83-93) = TF ApplyRMSProp:  ms += (g*g - ms)*(1-decay);

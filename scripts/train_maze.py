@@ -6,7 +6,10 @@ Logs finished episodes and mean episode score (+1 goal, -1 per wall hit) per 100
     {"learning_check": {"seeds": [...], "solved": k, "criterion": "..."}}
 
     python scripts/train_maze.py --envs 1024 --updates 2500 --lr 1e-2 --seeds 0,1,2,3 [--warmup 300] [--entropy-beta 0.001]
-                                 [--obs cells|s2d|f32] [--out file.jsonl]
+                                 [--obs cells|s2d|f32] [--out file.jsonl] [--eval-episodes K]
+
+--eval-episodes K: after each seed's run the final weights are evaluated (unreal_b200.train.evaluator): K sampled episodes
+per env and the greedy episode, added to that seed's result as `eval`.
 """
 import argparse
 import json
@@ -21,6 +24,7 @@ import torch
 from unreal_b200.environment.environment import Environment
 from unreal_b200.model.model import UnrealModel
 from unreal_b200.train.rmsprop_applier import RMSPropApplier
+from unreal_b200.train.evaluator import Evaluator
 from unreal_b200.train.trainer import Trainer
 
 
@@ -65,7 +69,15 @@ def run(args, seed, out):
         break
   tr.stop()
   solved = bool(final and final["mean_score"] is not None and final["mean_score"] >= 0.9 and final["steps_per_episode"] <= 25)
-  return solved, final
+  ev = None
+  if args.eval_episodes > 0:
+    # the final weights on their own: sampled (K episodes per env, own streams) and the greedy path (deterministic: one env)
+    ev = {"sample": Evaluator(net, 'maze', '', num_envs=n, seeds=np.arange(n) + 1000 * seed, mode='sample',
+                              max_episode_steps=args.eval_max_steps).run(args.eval_episodes)["summary"],
+          "greedy": Evaluator(net, 'maze', '', num_envs=1, mode='greedy',
+                              max_episode_steps=args.eval_max_steps).run(1)["summary"]}
+    out.write(json.dumps({"seed": seed, "eval": ev}) + "\n"); out.flush()
+  return solved, final, ev
 
 
 def main():
@@ -84,22 +96,25 @@ def main():
   p.add_argument("--seeds", default="0")
   p.add_argument("--obs", default="cells", choices=["cells", "s2d", "f32"])
   p.add_argument("--out", default="-")
+  p.add_argument("--eval-episodes", type=int, default=0, help="evaluate the final weights: K sampled episodes per env + greedy")
+  p.add_argument("--eval-max-steps", type=int, default=2000, help="step cap of an evaluation episode")
   args = p.parse_args()
   out = sys.stdout if args.out == "-" else open(args.out, "w")
   seeds = [int(s) for s in args.seeds.split(",")]
   results = []
   for s in seeds:
-    solved, final = run(args, s, out)
-    results.append((s, solved, final))
+    solved, final, ev = run(args, s, out)
+    results.append((s, solved, final, ev))
     torch.cuda.empty_cache()
   out.write(json.dumps({"learning_check": {
-      "seeds": seeds, "solved": sum(1 for _, ok, _ in results if ok),
+      "seeds": seeds, "solved": sum(1 for _, ok, _, _ in results if ok),
       "criterion": "mean episode score >= 0.9 at <= 25 steps per episode (optimum: +1 in 20 moves) in the last logging window",
       "config": {"envs": args.envs, "max_updates": args.updates, "lr": args.lr, "warmup_updates": args.warmup,
                  "entropy_beta": args.entropy_beta, "clip": args.clip, "gradient": "sum over envs" if args.grad_sum else "mean over envs",
                  "obs": args.obs},
-      "per_seed": [{"seed": s, "solved": ok, "updates": (f or {}).get("updates"), "mean_score": (f or {}).get("mean_score"),
-                    "steps_per_episode": (f or {}).get("steps_per_episode")} for s, ok, f in results]}}) + "\n")
+      "per_seed": [dict({"seed": s, "solved": ok, "updates": (f or {}).get("updates"), "mean_score": (f or {}).get("mean_score"),
+                         "steps_per_episode": (f or {}).get("steps_per_episode")}, **({"eval": ev} if ev else {}))
+                   for s, ok, f, ev in results]}}) + "\n")
   out.flush()
 
 

@@ -72,6 +72,8 @@ SIGNATURES = {
     "unreal_replay_gather": (c_int, [c_void_p, P, c_int64, P, P, c_int, c_int, P, P]),
     "unreal_rollout_lar": (c_int, [P, P, P, c_int, c_int, c_int, P, P]),
     "unreal_rollout_post": (c_int, [P, P, P, c_int, P, P, P, P, P, P, P, P]),
+    "unreal_maze_eval_act": (c_int, [P, c_int, c_int, P, P, P, P, P, P, P, P, P, P, P, P, c_int, c_int, P, P, P, P, c_int64,
+                                     c_int, c_int, P]),
     "unreal_grad_sumsq": (c_int, [P, c_int64, P, P]),
     "unreal_rmsprop_update": (c_int, [P, P, P, P, c_int64, P, c_float, c_float, c_float, c_float, c_float,
                                       c_float, P, P]),

@@ -738,6 +738,14 @@ int maze_walls49(uint64_t* out) {
   *out = w;
   return UNREAL_OK;
 }
+
+// the layout K1 steps with (the host copy of c_maze), for kernels of other translation units (evaluate.cu)
+int maze_layout_host(MazeLayout* out) {
+  int rc = ensure_map();
+  if (rc != UNREAL_OK) return rc;
+  *out = h_maze;
+  return UNREAL_OK;
+}
 }  // namespace unreal
 
 extern "C" int unreal_maze_get_layout(int* sx, int* sy, int* gx, int* gy, uint8_t* walls49_host) {

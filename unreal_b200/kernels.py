@@ -986,6 +986,36 @@ def rollout_post(reward, terminal, frame_rec, active, ended, last_rec, episode_r
        ptr(lstm_h, torch.float32, "lstm_h"), ptr(stats, torch.float64, "stats"), stream_ptr())
 
 
+def maze_eval_act(pi, greedy, streams, state, ep, res, lstm_c, lstm_h, fc_tab, xh, kx, max_steps):
+  """One evaluation step after the policy, in place (unreal_maze_eval_act, include/unreal_b200.h): pi f32 [N,A];
+  streams: MtStreams (None when greedy); state: MazeState; ep: dict(score f32, length i32, index i32, active u8) [N];
+  res: dict(score f32, length i32, finished u8) [N,E]; lstm_c / lstm_h f32 [N,256]; fc_tab bf16 [49,256]; xh bf16
+  [N, >= kx + 256] with contiguous rows."""
+  n, a = pi.shape
+  e = res["score"].shape[1]
+  for k, t in res.items():
+    if tuple(t.shape) != (n, e):
+      raise _lib.UnrealError("maze_eval_act: result %s must be [%d,%d]" % (k, n, e))
+  for k, t in ep.items():
+    if t.numel() != n:
+      raise _lib.UnrealError("maze_eval_act: %s must hold %d entries" % (k, n))
+  if state.n != n or tuple(lstm_c.shape) != (n, 256) or tuple(lstm_h.shape) != (n, 256) or tuple(fc_tab.shape) != (49, 256):
+    raise _lib.UnrealError("maze_eval_act: maze state [%d], LSTM state [%d,256] and table [49,256] expected" % (n, n))
+  xp, ld = _rows2d(xh, xh.shape[1], torch.bfloat16, "xh")
+  if xh.shape[0] != n:
+    raise _lib.UnrealError("maze_eval_act: xh must have %d rows" % n)
+  if streams is None and not greedy:
+    raise _lib.UnrealError("maze_eval_act: sampling needs the MT19937 streams")
+  call("unreal_maze_eval_act", ptr(pi, torch.float32, "pi"), int(a), 1 if greedy else 0,
+       None if streams is None else ptr(streams.mt), None if streams is None else ptr(streams.pos),
+       ptr(state.pos, torch.int32), ptr(state.last_action, torch.int32), ptr(state.last_reward, torch.float32),
+       ptr(ep["score"], torch.float32, "score"), ptr(ep["length"], torch.int32, "length"),
+       ptr(ep["index"], torch.int32, "index"), ptr(ep["active"], torch.uint8, "active"),
+       ptr(res["score"], torch.float32, "res score"), ptr(res["length"], torch.int32, "res length"),
+       ptr(res["finished"], torch.uint8, "res finished"), int(e), int(max_steps), ptr(lstm_c, torch.float32, "lstm_c"),
+       ptr(lstm_h, torch.float32, "lstm_h"), ptr(fc_tab, torch.bfloat16, "fc_tab"), xp, ld, int(kx), n, stream_ptr())
+
+
 def lstm_cell_act_heads(gates, c_state, h_state, wp, bp, wv, bv, active=None, v_out=None):
   """Acting step of the cell + the policy / value heads in one launch: gates bf16 [N,1024], state f32 [N,256] in place for
   the active envs; wp [256,A], bp [A], wv [256], bv [1] f32 -> (pi f32 [N,A], v f32 [N]; v_out: a caller-owned [N] row)."""

@@ -371,14 +371,17 @@ class UnrealModel(object):
       (h, c1, h1), _ = self._tower(p32, img, self._lar(last_action_reward, n), state[0], state[1])
       return p32, h[0], (c1, h1)
 
-  def _step_gates(self, p32, images, lar, h_prev):
+  def _step_gates(self, p32, images, lar, h_prev, xh=None):
     """One acting step up to the LSTM gate pre-activations, without the training path's glue: fc1 writes straight
-    into the [x, h] operand of the step GEMM (`_act_xh`, persistent, padding columns stay zero), the last action /
-    reward vector and h are cast into their columns, one GEMM gives the gates [N,1024] f32."""
+    into the [x, h] operand of the step GEMM (`xh`; None: the model's `_act_xh`, persistent, padding columns stay zero),
+    the last action / reward vector and h are cast into their columns, one GEMM gives the gates [N,1024] f32."""
     n = images.shape[0]
-    xh = self._act_xh.get(n)
     if xh is None:
-      xh = self._act_xh[n] = torch.zeros(n, self.kx + 256, dtype=torch.bfloat16, device=self._device)
+      xh = self._act_xh.get(n)
+      if xh is None:
+        xh = self._act_xh[n] = torch.zeros(n, self.kx + 256, dtype=torch.bfloat16, device=self._device)
+    elif tuple(xh.shape) != (n, self.kx + 256) or xh.dtype != torch.bfloat16:
+      raise _lib.UnrealError("xh must be bf16 [%d, %d] with zero padding columns" % (n, self.kx + 256))
     if self._use_tables(images):      # maze cells: fc1's output is a row of the 49-entry table (refresh_shadow)
       K.cell_gather(self._fc_tab_act, images.reshape(n, 2), out=xh[:, :256])
     else:
@@ -387,37 +390,51 @@ class UnrealModel(object):
       K.gemm_bf16(h2.view(n, 2592), self.v16["W_base_fc1"], out=xh[:, :256], b_mn_major=True, bias=p32["b_base_fc1"], relu=True)
     xh[:, 256:self.lstm_in].copy_(lar)
     xh[:, self.kx:].copy_(h_prev)
-    return K.gemm_bf16(xh, self.wcat16, b_mn_major=True, bias=p32["lstm_bias"], out_dtype=self._gates_dtype())
+    return self._xh_gates(p32, xh)
+
+  def _xh_gates(self, p32, xh, out=None):
+    """The acting step's GEMM: gate pre-activations [N,1024] of a filled [x, h] operand."""
+    return K.gemm_bf16(xh, self.wcat16, b_mn_major=True, bias=p32["lstm_bias"], out_dtype=self._gates_dtype(), out=out)
+
+  def _act_cell_heads(self, p32, gates, c, h, active=None, v_out=None):
+    """The acting step after the GEMM: the cell in place on the state rows (c, h) [N,256] of the active envs, then the
+    policy / value heads -> (pi [N,A], v [N])."""
+    if self.fused_heads and self.fused_act_heads and gates.dtype == torch.bfloat16 and self._action_size <= 7:
+      # the cell and the heads in one launch: the warp that computes an env's h reduces its logits and value as well
+      return K.lstm_cell_act_heads(gates, c, h, p32["W_base_fc_p"].contiguous(), p32["b_base_fc_p"],
+                                   p32["W_base_fc_v"].reshape(256).contiguous(), p32["b_base_fc_v"], active, v_out)
+    hh = torch.empty(gates.shape[0], 256, device=self._device)
+    K.lstm_cell_act(gates, c, h, hh, active)      # in place on the state of the active envs
+    return self._policy_value(p32, hh, v_out)
+
+  def act_step(self, s_t, last_action_reward, c, h, active=None, v_out=None, xh=None):
+    """run_base_policy_and_value on caller-owned state: the LSTM state rows c, h (f32 [N,256], updated in place for
+    the active envs) and, optionally, the step GEMM's operand xh (bf16 [N, kx + 256], zero-initialised; None: the
+    model's own per-batch-size operand) -> (pi [N,A], v [N])."""
+    if self.fused_conv and self.fused_encoder:
+      with torch.no_grad():
+        p32 = self._views(self.flat)
+        img = self._images(s_t)
+        n = img.shape[1]
+        gates = self._step_gates(p32, img[0], self._lar(last_action_reward, n)[0], h, xh)
+        return self._act_cell_heads(p32, gates, c, h, active, v_out)
+    p32, hh, new_state = self._step(s_t, last_action_reward, (c, h))
+    with torch.no_grad():
+      pi, v = self._policy_value(p32, hh, v_out)
+      if active is None:
+        c.copy_(new_state[0]); h.copy_(new_state[1])
+      else:
+        m = active.to(torch.bool).unsqueeze(1)
+        c.copy_(torch.where(m, new_state[0], c))
+        h.copy_(torch.where(m, new_state[1], h))
+    return pi, v
 
   def run_base_policy_and_value(self, sess, s_t, last_action_reward, active=None, mode="", v_out=None):
     """model.py:630-660: one acting step; advances the LSTM state of the active envs.  `v_out` (f32 [N], contiguous): the
     values are written there (the batched rollout's history row) and returned as that tensor."""
     if v_out is not None and not (v_out.is_contiguous() and v_out.dtype == torch.float32):
       raise _lib.UnrealError("v_out must be a contiguous float32 [N] tensor")
-    if self.fused_conv and self.fused_encoder:
-      with torch.no_grad():
-        p32 = self._views(self.flat)
-        img = self._images(s_t)
-        n = img.shape[1]
-        gates = self._step_gates(p32, img[0], self._lar(last_action_reward, n)[0], self._lstm_h)
-        if self.fused_heads and self.fused_act_heads and gates.dtype == torch.bfloat16 and self._action_size <= 7:
-          # the cell and the heads in one launch: the warp that computes an env's h reduces its logits and value as well
-          pi, v = K.lstm_cell_act_heads(gates, self._lstm_c, self._lstm_h, p32["W_base_fc_p"].contiguous(), p32["b_base_fc_p"],
-                                        p32["W_base_fc_v"].reshape(256).contiguous(), p32["b_base_fc_v"], active, v_out)
-          return pi, v, None
-        h = torch.empty(n, 256, device=self._device)
-        K.lstm_cell_act(gates, self._lstm_c, self._lstm_h, h, active)      # in place on the state of the active envs
-        pi, v = self._policy_value(p32, h, v_out)
-      return pi, v, None
-    p32, h, new_state = self._step(s_t, last_action_reward, self.base_lstm_state_out)
-    with torch.no_grad():
-      pi, v = self._policy_value(p32, h, v_out)
-      if active is None:
-        self._lstm_c.copy_(new_state[0]); self._lstm_h.copy_(new_state[1])
-      else:
-        m = active.to(torch.bool).unsqueeze(1)
-        self._lstm_c.copy_(torch.where(m, new_state[0], self._lstm_c))
-        self._lstm_h.copy_(torch.where(m, new_state[1], self._lstm_h))
+    pi, v = self.act_step(s_t, last_action_reward, self._lstm_c, self._lstm_h, active, v_out)
     return pi, v, None
 
   def run_base_value(self, sess, s_t, last_action_reward):
