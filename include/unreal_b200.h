@@ -395,6 +395,23 @@ int unreal_conv1_wgrad(const void* xpp_bf16, const void* dy_planes_bf16, float* 
 int unreal_conv1_fwd_maze(const int32_t* pos, const void* w_taps_bf16, const float* bias, void* out_bf16, int s,
                           void* stream);
 int unreal_conv1_wgrad_maze(const int32_t* pos, const void* dy_planes21_bf16, float* dw_taps, int s, void* stream);
+/* Split-bf16 ("bf16x3") encoder forward, for reference-grade (fp32-like) products on the bf16 tensor path: every fp32
+ * operand a is carried as a_hi = bf16(a) and a_lo = bf16(a - a_hi), and a.b is accumulated as
+ * a_hi.b_hi + a_hi.b_lo + a_lo.b_hi in fp32.  Layouts are those of the bf16 entry points above; *_lo filters are the
+ * same tap layouts of bf16(W - bf16(W)).
+ *   unreal_s2d_frames_split    : as unreal_s2d_frames, plus the lo planes.
+ *   unreal_conv1_fwd_split     : x'' hi / lo planes (xpp_lo NULL: the input is exactly bf16, two passes)
+ *                                -> h1 = relu(conv + bias) as a hi / lo pair of bf16 [S,20,20,16].
+ *   unreal_conv1_fwd_maze_split: render-fused (the rendered frames are exactly 0 / 1: two passes) -> h1 hi / lo.
+ *   unreal_conv2_fwd_split     : h1 hi / lo -> h2 bf16 [S,9,9,32] = relu(conv + bias).
+ * With zero lo filters and a zero (or NULL) lo input the results equal the bf16 entry points bit for bit. */
+int unreal_s2d_frames_split(const void* frames, int dtype, void* out_hi_bf16, void* out_lo_bf16, int s, void* stream);
+int unreal_conv1_fwd_split(const void* xpp_hi_bf16, const void* xpp_lo_bf16, const void* w_hi_bf16, const void* w_lo_bf16,
+                           const float* bias, void* out_hi_bf16, void* out_lo_bf16, int s, void* stream);
+int unreal_conv1_fwd_maze_split(const int32_t* pos, const void* w_hi_bf16, const void* w_lo_bf16, const float* bias,
+                                void* out_hi_bf16, void* out_lo_bf16, int s, void* stream);
+int unreal_conv2_fwd_split(const void* h1_hi_bf16, const void* h1_lo_bf16, const void* w_hi_bf16, const void* w_lo_bf16,
+                           const float* bias, void* out_bf16, int s, void* stream);
 int unreal_conv1_wgrad_p21(const void* xpp_bf16, const void* dy_planes21_bf16, float* dw_taps, int s, void* stream);
 /* conv2 filter gradient from h1 [S,20,20,16] bf16 and the masked dY2 [S*81,32] bf16, both read once through
  * TMA boxes: dw_taps f32 [4 ky][64 (kx,c)][32 out] = HWIO [4,4,16,32] += ... (caller zeroes dw_taps). */

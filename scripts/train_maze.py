@@ -6,10 +6,12 @@ Logs finished episodes and mean episode score (+1 goal, -1 per wall hit) per 100
     {"learning_check": {"seeds": [...], "solved": k, "criterion": "..."}}
 
     python scripts/train_maze.py --envs 1024 --updates 2500 --lr 1e-2 --seeds 0,1,2,3 [--warmup 300] [--entropy-beta 0.001]
-                                 [--obs cells|s2d|f32] [--out file.jsonl] [--eval-episodes K]
+                                 [--obs cells|s2d|f32] [--out file.jsonl] [--eval-episodes K] [--encoder-precision bf16x3]
 
 --eval-episodes K: after each seed's run the final weights are evaluated (unreal_b200.train.evaluator): K sampled episodes
 per env and the greedy episode, added to that seed's result as `eval`.
+--encoder-precision bf16x3: conv1 and conv2 forward on split-bf16 operands (UnrealModel(encoder_precision=...)); the
+summary's config names it when it is not the default.
 """
 import argparse
 import json
@@ -32,7 +34,7 @@ def run(args, seed, out):
   n, dev = args.envs, torch.device("cuda", 0)
   Environment.action_size = -1
   net = UnrealModel(4, 0, -1, True, True, True, True, 0.05, args.entropy_beta, dev, {'segnet_mode': 0}, (84, 84), True, 0, 0.0,
-                    0.0, num_envs=n, seed=seed)
+                    0.0, num_envs=n, seed=seed, encoder_precision=args.encoder_precision)
   if args.grad_sum:
     net.grad_scale = 1.0
   applier = RMSPropApplier(args.lr, decay=0.99, momentum=0.0, epsilon=0.1, clip_norm=args.clip)
@@ -98,9 +100,16 @@ def main():
   p.add_argument("--out", default="-")
   p.add_argument("--eval-episodes", type=int, default=0, help="evaluate the final weights: K sampled episodes per env + greedy")
   p.add_argument("--eval-max-steps", type=int, default=2000, help="step cap of an evaluation episode")
+  p.add_argument("--encoder-precision", default="bf16", choices=["bf16", "bf16x3"],
+                 help="bf16x3: split-bf16 operands in the encoder's forward convolutions (fp32-grade products)")
   args = p.parse_args()
   out = sys.stdout if args.out == "-" else open(args.out, "w")
   seeds = [int(s) for s in args.seeds.split(",")]
+  config = {"envs": args.envs, "max_updates": args.updates, "lr": args.lr, "warmup_updates": args.warmup,
+            "entropy_beta": args.entropy_beta, "clip": args.clip, "gradient": "sum over envs" if args.grad_sum else "mean over envs",
+            "obs": args.obs}
+  if args.encoder_precision != "bf16":
+    config["encoder_precision"] = args.encoder_precision
   results = []
   for s in seeds:
     solved, final, ev = run(args, s, out)
@@ -109,9 +118,7 @@ def main():
   out.write(json.dumps({"learning_check": {
       "seeds": seeds, "solved": sum(1 for _, ok, _, _ in results if ok),
       "criterion": "mean episode score >= 0.9 at <= 25 steps per episode (optimum: +1 in 20 moves) in the last logging window",
-      "config": {"envs": args.envs, "max_updates": args.updates, "lr": args.lr, "warmup_updates": args.warmup,
-                 "entropy_beta": args.entropy_beta, "clip": args.clip, "gradient": "sum over envs" if args.grad_sum else "mean over envs",
-                 "obs": args.obs},
+      "config": config,
       "per_seed": [dict({"seed": s, "solved": ok, "updates": (f or {}).get("updates"), "mean_score": (f or {}).get("mean_score"),
                          "steps_per_episode": (f or {}).get("steps_per_episode")}, **({"eval": ev} if ev else {}))
                    for s, ok, f, ev in results]}}) + "\n")

@@ -106,6 +106,10 @@ SIGNATURES = {
     "unreal_conv1_wgrad_p21": (c_int, [P, P, P, c_int, P]),
     "unreal_conv1_fwd_maze": (c_int, [P, P, P, P, c_int, P]),
     "unreal_conv1_wgrad_maze": (c_int, [P, P, P, c_int, P]),
+    "unreal_s2d_frames_split": (c_int, [P, c_int, P, P, c_int, P]),
+    "unreal_conv1_fwd_split": (c_int, [P, P, P, P, P, P, P, c_int, P]),
+    "unreal_conv1_fwd_maze_split": (c_int, [P, P, P, P, P, P, c_int, P]),
+    "unreal_conv2_fwd_split": (c_int, [P, P, P, P, P, P, c_int, P]),
     "unreal_a3c_head_loss": (c_int, [P, P, P, P, P, P, P, P, P, c_int64, c_int, c_float, c_float, P, P, P, P, P, P]),
     "unreal_a3c_head_bwd": (c_int, [P, P, P, P, P, P, c_int64, c_int, P, P, P, P, P, P]),
     "unreal_pc_loss": (c_int, [P, P, P, P, c_int, c_float, c_int64, c_int, P, P, P, P]),

@@ -113,25 +113,32 @@ __device__ __forceinline__ void tma_store_3d(const CUtensorMap* m, uint32_t src,
 // MASKED: the result is the gradient w.r.t. a ReLU layer's output `mask_y` (pc_fc1 seen as [S,9,9,32] behind the pixel-control
 // deconv): the epilogue zeroes it where mask_y <= 0 and sums the rounded values over items into db -- the ReLU-gradient /
 // bias-gradient pass over the [S,2592] gradient (2.5 GB of traffic per update at 8192 envs) disappears.
-template <int N, int MODE, bool MASKED = false, int C = 16>   // N output channels: 32 (conv2, MODE 2); C input channels
+// SPLIT (split-bf16 conv2, C = 16 only): tma_alo / tma_alo2 are the boxes of h1_lo, tma_wlo the filter residual; a stage
+// holds the hi box then the lo box (two stages keep two CTAs per SM), the filters are resident as hi then lo, and every
+// K step accumulates a_hi.w_hi + a_hi.w_lo + a_lo.w_hi.  Other builds ignore the three extra maps.
+template <int N, int MODE, bool MASKED = false, int C = 16, bool SPLIT = false>   // N output channels: 32 (conv2, MODE 2); C input channels
 __global__ void __launch_bounds__(kConvThreads, 2)
 conv_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_a2,
                         const __grid_constant__ CUtensorMap tma_w, const __grid_constant__ CUtensorMap tma_c,
-                        const ConvArgs g) {
+                        const ConvArgs g, const __grid_constant__ CUtensorMap tma_alo,
+                        const __grid_constant__ CUtensorMap tma_alo2, const __grid_constant__ CUtensorMap tma_wlo) {
   using Cfg = ConvCfg<MODE, C>;
+  static_assert(!SPLIT || (C == 16 && !MASKED), "split conv2: the encoder's geometry only");
+  constexpr int kStages = SPLIT ? 2 : Cfg::kStages;
+  constexpr int kStageBytes = SPLIT ? 2 * Cfg::kStageBytes : Cfg::kStageBytes;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   constexpr int kWTileBytes = N * Cfg::kRowBytes;          // one resident filter slice [N rows x kRowBytes]
   constexpr int kWBytes = (Cfg::kSteps * kWTileBytes + 1023) / 1024 * 1024;
   const uint32_t w_smem = smem_base;
-  const uint32_t a_smem = smem_base + kWBytes;
-  const uint32_t bar_base = a_smem + Cfg::kStages * Cfg::kStageBytes;
+  const uint32_t a_smem = smem_base + (SPLIT ? 2 : 1) * kWBytes;
+  const uint32_t bar_base = a_smem + kStages * kStageBytes;
   auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (Cfg::kStages + s); };
-  auto tfull_bar = [&](int a) { return bar_base + 8u * (2 * Cfg::kStages + a); };
-  auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * Cfg::kStages + kConvAcc + a); };
-  const uint32_t w_bar = bar_base + 8u * (2 * Cfg::kStages + 2 * kConvAcc);
-  const uint32_t tmem_slot = bar_base + 8u * (2 * Cfg::kStages + 2 * kConvAcc + 1);
+  auto empty_bar = [&](int s) { return bar_base + 8u * (kStages + s); };
+  auto tfull_bar = [&](int a) { return bar_base + 8u * (2 * kStages + a); };
+  auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * kStages + kConvAcc + a); };
+  const uint32_t w_bar = bar_base + 8u * (2 * kStages + 2 * kConvAcc);
+  const uint32_t tmem_slot = bar_base + 8u * (2 * kStages + 2 * kConvAcc + 1);
   const uint32_t ebuf_base = bar_base + 1024u;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -140,7 +147,8 @@ conv_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_
     prefetch_tensormap(&tma_a2);
     prefetch_tensormap(&tma_w);
     prefetch_tensormap(&tma_c);
-    for (int s = 0; s < Cfg::kStages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
+    if constexpr (SPLIT) { prefetch_tensormap(&tma_alo); prefetch_tensormap(&tma_alo2); prefetch_tensormap(&tma_wlo); }
+    for (int s = 0; s < kStages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     for (int a = 0; a < kConvAcc; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 4); }
     mbar_init(w_bar, 1);
     fence_mbar_init();
@@ -156,20 +164,23 @@ conv_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_
   if (warp == 0) {
     if (lane == 0) {
       // ===== TMA producer: resident filter slices once, then one box per (item, step) =====
-      mbar_arrive_expect_tx(w_bar, Cfg::kSteps * kWTileBytes);
+      mbar_arrive_expect_tx(w_bar, (SPLIT ? 2 : 1) * Cfg::kSteps * kWTileBytes);
 #pragma unroll
-      for (int t = 0; t < Cfg::kSteps; ++t)
+      for (int t = 0; t < Cfg::kSteps; ++t) {
         tma_load_2d(w_smem + t * kWTileBytes, &tma_w, w_bar, t * (Cfg::kRowBytes / 2), 0);
+        if constexpr (SPLIT) tma_load_2d(w_smem + kWBytes + t * kWTileBytes, &tma_wlo, w_bar, t * (Cfg::kRowBytes / 2), 0);
+      }
       int stage = 0; uint32_t phase = 0;
       for (int it = blockIdx.x; it < g.items; it += gridDim.x) {
 #pragma unroll 1
         for (int st = 0; st < Cfg::kSteps; ++st) {
           mbar_wait(empty_bar(stage), phase ^ 1u);
-          mbar_arrive_expect_tx(full_bar(stage), g.box_bytes);
-          const uint32_t dst = a_smem + stage * Cfg::kStageBytes;
+          mbar_arrive_expect_tx(full_bar(stage), (SPLIT ? 2 : 1) * g.box_bytes);
+          const uint32_t dst = a_smem + stage * kStageBytes;
           const int by = st >> 1, dy = st & 1;
           tma_load_4d(dst, dy ? &tma_a2 : &tma_a, full_bar(stage), 0, 0, by, it);
-          if (++stage == Cfg::kStages) { stage = 0; phase ^= 1u; }
+          if constexpr (SPLIT) tma_load_4d(dst + Cfg::kStageBytes, dy ? &tma_alo2 : &tma_alo, full_bar(stage), 0, 0, by, it);
+          if (++stage == kStages) { stage = 0; phase ^= 1u; }
         }
       }
     }
@@ -191,13 +202,18 @@ conv_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_
           fence_after_sync();
           // SW64 K-major descriptors as (lo, hi) words: hi is constant (SBO 512 B, version 1, 64-byte swizzle),
           // lo = (address >> 4) | LBO field; one add per UMMA instead of rebuilding 64-bit descriptors
-          const uint32_t a_lo = ((a_smem + stage * Cfg::kStageBytes) >> 4) | (1u << 16);
+          const uint32_t a_lo = ((a_smem + stage * kStageBytes) >> 4) | (1u << 16);
           const uint32_t b_lo = ((w_smem + st * kWTileBytes) >> 4) | (1u << 16);
 #pragma unroll
-          for (int k = 0; k < Cfg::kMmaPerStep; ++k)
+          for (int k = 0; k < Cfg::kMmaPerStep; ++k) {
             mma_f16_lohi(tmem_d, a_lo + 2u * k, kDescHiSw64, b_lo + 2u * k, kDescHiSw64, idesc, (st > 0 || k > 0) ? 1u : 0u);
+            if constexpr (SPLIT) {
+              mma_f16_lohi(tmem_d, a_lo + 2u * k, kDescHiSw64, b_lo + (uint32_t)(kWBytes >> 4) + 2u * k, kDescHiSw64, idesc, 1u);
+              mma_f16_lohi(tmem_d, a_lo + (uint32_t)(Cfg::kStageBytes >> 4) + 2u * k, kDescHiSw64, b_lo + 2u * k, kDescHiSw64, idesc, 1u);
+            }
+          }
           mma_commit(empty_bar(stage));
-          if (++stage == Cfg::kStages) { stage = 0; phase ^= 1u; }
+          if (++stage == kStages) { stage = 0; phase ^= 1u; }
         }
         mma_commit(tfull_bar(acc));
         if (++acc == kConvAcc) { acc = 0; acc_phase ^= 1u; }
@@ -297,30 +313,36 @@ conv_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_
 // pixel-change kernel (csrc/pixel_change84.cu: PRMT into the mantissa of 2^23, one FADD2, fma(v, hi, RN(v * lo)) on the
 // packed fp32x2 pipe; exhaustively checked by unreal_selfcheck_arith) -- the kernel was instruction-bound on 48
 // __fdiv_rn per thread (0.39 of HBM).  `magic` = 0x4B000000 arrives as a kernel parameter so the PRMT selectors stay immediates.
-__device__ __forceinline__ uint32_t u8pair_to_bf16x2(uint32_t word, int byte0, uint32_t magic) {
+__device__ __forceinline__ float2 u8pair_to_f32x2(uint32_t word, int byte0, uint32_t magic) {
   float2 m;
   m.x = __uint_as_float(__byte_perm(word, magic, 0x7540u | (uint32_t)byte0));
   m.y = __uint_as_float(__byte_perm(word, magic, 0x7540u | (uint32_t)(byte0 + 1)));
   const float2 v = __fadd2_rn(m, make_float2(-8388608.0f, -8388608.0f));
-  const float2 q = __ffma2_rn(v, make_float2(0x1.010102p-8f, 0x1.010102p-8f),
-                              __fmul2_rn(v, make_float2(-0x1.fdfdfep-33f, -0x1.fdfdfep-33f)));
+  return __ffma2_rn(v, make_float2(0x1.010102p-8f, 0x1.010102p-8f),
+                    __fmul2_rn(v, make_float2(-0x1.fdfdfep-33f, -0x1.fdfdfep-33f)));
+}
+__device__ __forceinline__ uint32_t u8pair_to_bf16x2(uint32_t word, int byte0, uint32_t magic) {
+  const float2 q = u8pair_to_f32x2(word, byte0, magic);
   __nv_bfloat162 p2 = __floats2bfloat162_rn(q.x, q.y);
   return *reinterpret_cast<uint32_t*>(&p2);
 }
 
-template <typename T>
+// LO (split-bf16 encoder): also writes the residual planes out_lo = bf16(x - bf16(x)) in the same layout, so that
+// hi + lo carries the frame to about 16 mantissa bits.
+template <typename T, bool LO = false>
 __global__ void __launch_bounds__(256) s2d_frames_kernel(const T* __restrict__ in, __nv_bfloat16* __restrict__ out,
-                                                         int64_t total, uint32_t magic) {
+                                                         int64_t total, uint32_t magic, __nv_bfloat16* __restrict__ out_lo) {
   for (int64_t id = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; id < total; id += (int64_t)gridDim.x * blockDim.x) {
     const int X = (int)(id % 21);
     const int Y = (int)((id / 21) % 21);
     const int64_t s = id / 441;
     const T* src = in + ((s * 84 + 4 * Y) * 84 + 4 * X) * 3;
     uint32_t pk[24];
+    uint32_t pl[LO ? 24 : 1];
 #pragma unroll
     for (int dy = 0; dy < 4; ++dy) {
       float v[12];
-      if (sizeof(T) == 1) {
+      if (sizeof(T) == 1 && !LO) {
         const uint32_t* p = reinterpret_cast<const uint32_t*>(src + dy * 252);   // 12 bytes, 4-byte aligned
 #pragma unroll
         for (int w = 0; w < 3; ++w) {
@@ -335,6 +357,14 @@ __global__ void __launch_bounds__(256) s2d_frames_kernel(const T* __restrict__ i
         const float4 a = __ldcs(p), b = __ldcs(p + 1), c = __ldcs(p + 2);
         v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
         v[8] = c.x; v[9] = c.y; v[10] = c.z; v[11] = c.w;
+      } else if (LO) {
+        const uint32_t* p = reinterpret_cast<const uint32_t*>(src + dy * 252);   // 12 bytes, 4-byte aligned
+#pragma unroll
+        for (int w = 0; w < 3; ++w) {
+          const uint32_t u = __ldcs(p + w);
+          const float2 a = u8pair_to_f32x2(u, 0, magic), b = u8pair_to_f32x2(u, 2, magic);
+          v[4 * w] = a.x; v[4 * w + 1] = a.y; v[4 * w + 2] = b.x; v[4 * w + 3] = b.y;
+        }
       } else {
         const uint32_t* p = reinterpret_cast<const uint32_t*>(src + dy * 252);   // 12 bytes, 4-byte aligned
 #pragma unroll
@@ -348,6 +378,11 @@ __global__ void __launch_bounds__(256) s2d_frames_kernel(const T* __restrict__ i
       for (int j = 0; j < 6; ++j) {
         __nv_bfloat162 p2 = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);
         pk[dy * 6 + j] = *reinterpret_cast<uint32_t*>(&p2);
+        if constexpr (LO) {
+          const float2 h = __bfloat1622float2(p2);
+          __nv_bfloat162 l2 = __floats2bfloat162_rn(v[2 * j] - h.x, v[2 * j + 1] - h.y);
+          pl[dy * 6 + j] = *reinterpret_cast<uint32_t*>(&l2);
+        }
       }
     }
     // plane-major: x'' [S][6 chunks of 8 channels][441 pixels][8]; consecutive threads (pixels) write
@@ -356,6 +391,11 @@ __global__ void __launch_bounds__(256) s2d_frames_kernel(const T* __restrict__ i
     uint4* dst = reinterpret_cast<uint4*>(out) + (s * 6) * 441 + pix;
 #pragma unroll
     for (int j = 0; j < 6; ++j) dst[(int64_t)j * 441] = make_uint4(pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
+    if constexpr (LO) {
+      uint4* dlo = reinterpret_cast<uint4*>(out_lo) + (s * 6) * 441 + pix;
+#pragma unroll
+      for (int j = 0; j < 6; ++j) dlo[(int64_t)j * 441] = make_uint4(pl[4 * j], pl[4 * j + 1], pl[4 * j + 2], pl[4 * j + 3]);
+    }
   }
 }
 
@@ -375,26 +415,39 @@ constexpr int kC1BoxBytes = 6 * kC1PlaneBytes;      // 12096
 constexpr int kC1StageBytes = 12288;
 constexpr int kC1WBytes = 4 * 6 * 16 * 16;          // [tap][chunk][16 out rows][8 ch] bf16
 constexpr int kC1Smem = kC1WBytes + kC1Stages * kC1StageBytes + 1024 /*barriers*/ + 1024 /*tail reads*/ + 1024 /*align*/;
+// SPLIT (split-bf16, "bf16x3"): operands a = a_hi + a_lo as two bf16 tensors; a stage holds the hi tile then the lo
+// tile, the filters are resident as hi then lo, and a.b ~ a_hi.b_hi + a_hi.b_lo + a_lo.b_hi accumulates in the same
+// TMEM columns (the a_lo.b_lo term is below fp32 rounding).  Four stages keep two CTAs per SM.
+constexpr int kC1SplitStages = 4;
+constexpr int kC1SplitSmem = 2 * kC1WBytes + kC1SplitStages * 2 * kC1StageBytes + 1024 + 1024 + 1024;
 
+template <bool SPLIT>
 __global__ void __launch_bounds__(kConvThreads, 2)
 conv1_fwd_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfloat16* __restrict__ w_planes,
                          const float* __restrict__ bias, __nv_bfloat16* __restrict__ out, int items,
-                         const int32_t* __restrict__ maze_pos, uint64_t walls49) {
+                         const int32_t* __restrict__ maze_pos, uint64_t walls49,
+                         const __nv_bfloat16* __restrict__ xpp_lo, const __nv_bfloat16* __restrict__ w_planes_lo,
+                         __nv_bfloat16* __restrict__ out_lo) {
+  // SPLIT: xpp_lo may be NULL (input exactly bf16: rendered maze tiles, pre-converted planes): two passes instead of three
+  constexpr int kStages = SPLIT ? kC1SplitStages : kC1Stages;
+  constexpr int kStageBytes = SPLIT ? 2 * kC1StageBytes : kC1StageBytes;
+  constexpr int kWB = SPLIT ? 2 * kC1WBytes : kC1WBytes;
+  const bool has_lo = SPLIT && xpp_lo != nullptr;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t w_smem = smem_base;
-  const uint32_t a_smem = smem_base + kC1WBytes;
-  const uint32_t bar_base = a_smem + kC1Stages * kC1StageBytes;
+  const uint32_t a_smem = smem_base + kWB;
+  const uint32_t bar_base = a_smem + kStages * kStageBytes;
   auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (kC1Stages + s); };
-  auto tfull_bar = [&](int a) { return bar_base + 8u * (2 * kC1Stages + a); };
-  auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * kC1Stages + kC1Acc + a); };
-  const uint32_t w_bar = bar_base + 8u * (2 * kC1Stages + 2 * kC1Acc);
-  const uint32_t tmem_slot = bar_base + 8u * (2 * kC1Stages + 2 * kC1Acc + 1);
+  auto empty_bar = [&](int s) { return bar_base + 8u * (kStages + s); };
+  auto tfull_bar = [&](int a) { return bar_base + 8u * (2 * kStages + a); };
+  auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * kStages + kC1Acc + a); };
+  const uint32_t w_bar = bar_base + 8u * (2 * kStages + 2 * kC1Acc);
+  const uint32_t tmem_slot = bar_base + 8u * (2 * kStages + 2 * kC1Acc + 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (warp == 0 && lane == 0) {
-    for (int s = 0; s < kC1Stages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
+    for (int s = 0; s < kStages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     for (int a = 0; a < kC1Acc; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 4); }
     mbar_init(w_bar, 1);
     fence_mbar_init();
@@ -410,40 +463,54 @@ conv1_fwd_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfloa
   if (warp == 0 && maze_pos != nullptr) {
     // ===== render-fused producer (maze): the warp WRITES each item's x'' tile from the agent cell =====
     if (lane == 0) {
-      mbar_arrive_expect_tx(w_bar, kC1WBytes);
+      mbar_arrive_expect_tx(w_bar, kWB);
       asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                    ::"r"(w_smem), "l"(w_planes), "r"(kC1WBytes), "r"(w_bar) : "memory");
+      if constexpr (SPLIT)
+        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                     ::"r"(w_smem + kC1WBytes), "l"(w_planes_lo), "r"(kC1WBytes), "r"(w_bar) : "memory");
     }
     int stage = 0; uint32_t phase = 0;
     for (int it = blockIdx.x; it < items; it += gridDim.x) {
       const int2 cell = __ldg(reinterpret_cast<const int2*>(maze_pos) + (it >> 2));
       mbar_wait(empty_bar(stage), phase ^ 1u);
-      maze_tile_to_smem(a_smem + stage * kC1StageBytes, walls49, cell.x, cell.y, it & 3, lane);
+      maze_tile_to_smem(a_smem + stage * kStageBytes, walls49, cell.x, cell.y, it & 3, lane);
       fence_proxy_async_smem();            // generic-proxy writes -> visible to the tensor core's async-proxy reads
       __syncwarp();
       if (lane == 0) mbar_arrive(full_bar(stage));
-      if (++stage == kC1Stages) { stage = 0; phase ^= 1u; }
+      if (++stage == kStages) { stage = 0; phase ^= 1u; }
     }
   } else if (warp == 0) {
     if (lane == 0) {
       // ===== producer: resident filters (one bulk copy), then ONE box per item =====
-      mbar_arrive_expect_tx(w_bar, kC1WBytes);
+      mbar_arrive_expect_tx(w_bar, kWB);
       asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                    ::"r"(w_smem), "l"(w_planes), "r"(kC1WBytes), "r"(w_bar) : "memory");
+      if constexpr (SPLIT)
+        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                     ::"r"(w_smem + kC1WBytes), "l"(w_planes_lo), "r"(kC1WBytes), "r"(w_bar) : "memory");
       int stage = 0; uint32_t phase = 0;
       for (int it = blockIdx.x; it < items; it += gridDim.x) {
         mbar_wait(empty_bar(stage), phase ^ 1u);
-        mbar_arrive_expect_tx(full_bar(stage), kC1BoxBytes);
+        mbar_arrive_expect_tx(full_bar(stage), has_lo ? 2 * kC1BoxBytes : kC1BoxBytes);
         // each plane's 126 pixel rows are 2016 contiguous bytes in x'': six 1-D bulk copies (a tensor
         // box with a 16-byte inner dimension costs the TMA engine one request per row: measured 2.3x slower)
         const uint8_t* src = reinterpret_cast<const uint8_t*>(xpp) + ((int64_t)(it >> 2) * 6 * 441 + (it & 3) * 105) * 16;
-        const uint32_t dst = a_smem + stage * kC1StageBytes;
+        const uint32_t dst = a_smem + stage * kStageBytes;
 #pragma unroll
         for (int q = 0; q < 6; ++q)
           asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                        ::"r"(dst + q * kC1PlaneBytes), "l"(src + (int64_t)q * 441 * 16), "r"(kC1PlaneBytes),
                          "r"(full_bar(stage)) : "memory");
-        if (++stage == kC1Stages) { stage = 0; phase ^= 1u; }
+        if (has_lo) {
+          const uint8_t* src_lo = reinterpret_cast<const uint8_t*>(xpp_lo) + (src - reinterpret_cast<const uint8_t*>(xpp));
+#pragma unroll
+          for (int q = 0; q < 6; ++q)
+            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                         ::"r"(dst + kC1StageBytes + q * kC1PlaneBytes), "l"(src_lo + (int64_t)q * 441 * 16),
+                           "r"(kC1PlaneBytes), "r"(full_bar(stage)) : "memory");
+        }
+        if (++stage == kStages) { stage = 0; phase ^= 1u; }
       }
     }
   } else if (warp == 1) {
@@ -461,18 +528,24 @@ conv1_fwd_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfloa
         fence_after_sync();
         const uint32_t tmem_d = tmem_base + (uint32_t)(acc * 32);
         // descriptor low words: (address >> 4) | LBO field; every offset below is a multiple of 16 bytes
-        const uint32_t a_lo0 = ((a_smem + stage * kC1StageBytes) >> 4) | ((uint32_t)(kC1PlaneBytes >> 4) << 16);
+        const uint32_t a_lo0 = ((a_smem + stage * kStageBytes) >> 4) | ((uint32_t)(kC1PlaneBytes >> 4) << 16);
 #pragma unroll
         for (int tap = 0; tap < 4; ++tap) {
           const uint32_t shift16 = (uint32_t)((tap >> 1) * 21 + (tap & 1));
 #pragma unroll
-          for (int j = 0; j < 3; ++j)
-            mma_f16_lohi(tmem_d, a_lo0 + (uint32_t)(2 * j * kC1PlaneBytes >> 4) + shift16, desc_hi,
-                         w_lo0 + (uint32_t)((tap * 1536 + 2 * j * 256) >> 4), desc_hi, idesc, (tap > 0 || j > 0) ? 1u : 0u);
+          for (int j = 0; j < 3; ++j) {
+            const uint32_t a = a_lo0 + (uint32_t)(2 * j * kC1PlaneBytes >> 4) + shift16;
+            const uint32_t w = w_lo0 + (uint32_t)((tap * 1536 + 2 * j * 256) >> 4);
+            mma_f16_lohi(tmem_d, a, desc_hi, w, desc_hi, idesc, (tap > 0 || j > 0) ? 1u : 0u);
+            if constexpr (SPLIT) {
+              mma_f16_lohi(tmem_d, a, desc_hi, w + (uint32_t)(kC1WBytes >> 4), desc_hi, idesc, 1u);        // a_hi . w_lo
+              if (has_lo) mma_f16_lohi(tmem_d, a + (uint32_t)(kC1StageBytes >> 4), desc_hi, w, desc_hi, idesc, 1u);  // a_lo . w_hi
+            }
+          }
         }
         mma_commit(empty_bar(stage));
         mma_commit(tfull_bar(acc));
-        if (++stage == kC1Stages) { stage = 0; phase ^= 1u; }
+        if (++stage == kStages) { stage = 0; phase ^= 1u; }
         if (++acc == kC1Acc) { acc = 0; acc_phase ^= 1u; }
       }
     }
@@ -496,16 +569,27 @@ conv1_fwd_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfloa
       __syncwarp();
       if (lane == 0) mbar_arrive(tempty_bar(acc));
       if (valid) {
-        uint32_t pk[8];
+        uint32_t pk[8], pl[SPLIT ? 8 : 1];
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
-          __nv_bfloat162 p = __floats2bfloat162_rn(fmaxf(__uint_as_float(v[2 * j]) + b[2 * j], 0.f),
-                                                   fmaxf(__uint_as_float(v[2 * j + 1]) + b[2 * j + 1], 0.f));
+          const float f0 = fmaxf(__uint_as_float(v[2 * j]) + b[2 * j], 0.f), f1 = fmaxf(__uint_as_float(v[2 * j + 1]) + b[2 * j + 1], 0.f);
+          __nv_bfloat162 p = __floats2bfloat162_rn(f0, f1);
           pk[j] = *reinterpret_cast<uint32_t*>(&p);
+          if constexpr (SPLIT) {          // h1 = hi + lo: the residual of the rounding as a second bf16
+            const float2 h = __bfloat1622float2(p);
+            __nv_bfloat162 l = __floats2bfloat162_rn(f0 - h.x, f1 - h.y);
+            pl[j] = *reinterpret_cast<uint32_t*>(&l);
+          }
         }
-        uint4* dst = reinterpret_cast<uint4*>(out + ((int64_t)it * 100 + oyl * 20 + ox) * 16);
+        const int64_t o = ((int64_t)it * 100 + oyl * 20 + ox) * 16;
+        uint4* dst = reinterpret_cast<uint4*>(out + o);
         dst[0] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
         dst[1] = make_uint4(pk[4], pk[5], pk[6], pk[7]);
+        if constexpr (SPLIT) {
+          uint4* dlo = reinterpret_cast<uint4*>(out_lo + o);
+          dlo[0] = make_uint4(pl[0], pl[1], pl[2], pl[3]);
+          dlo[1] = make_uint4(pl[4], pl[5], pl[6], pl[7]);
+        }
       }
       if (++acc == kC1Acc) { acc = 0; acc_phase ^= 1u; }
     }
@@ -1526,15 +1610,17 @@ pc_planes_wgrad_tcgen05_kernel(const __nv_bfloat16* __restrict__ dyp, const __gr
   }
 }
 
-template <int N, int MODE, bool MASKED = false, int C = 16>
+template <int N, int MODE, bool MASKED = false, int C = 16, bool SPLIT = false>
 static int launch_conv(const CUtensorMap& ta, const CUtensorMap& ta2, const CUtensorMap& tw, const CUtensorMap& tc,
-                       const ConvArgs& g, cudaStream_t st) {
+                       const ConvArgs& g, cudaStream_t st, const CUtensorMap& talo, const CUtensorMap& talo2,
+                       const CUtensorMap& twlo) {
   using Cfg = ConvCfg<MODE, C>;
-  constexpr int kWBytes = (Cfg::kSteps * N * Cfg::kRowBytes + 1023) / 1024 * 1024;
+  constexpr int kWBytes = (SPLIT ? 2 : 1) * ((Cfg::kSteps * N * Cfg::kRowBytes + 1023) / 1024 * 1024);
   // + 5 KB: the last stage's 128-row UMMA read runs 40 rows past its 88-row stage into barriers / epilogue buffers
-  constexpr int kSmem = kWBytes + Cfg::kStages * Cfg::kStageBytes + 1024 + Cfg::kEpiWarps * 2 * 4096 + 1024;
+  constexpr int kSmem = kWBytes + (SPLIT ? 2 * 2 * Cfg::kStageBytes : Cfg::kStages * Cfg::kStageBytes) + 1024 +
+                        Cfg::kEpiWarps * 2 * 4096 + 1024;
   static bool configured = false;
-  auto kern = conv_fwd_tcgen05_kernel<N, MODE, MASKED, C>;
+  auto kern = conv_fwd_tcgen05_kernel<N, MODE, MASKED, C, SPLIT>;
   if (!configured) {
     UNREAL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem));
     configured = true;
@@ -1542,7 +1628,7 @@ static int launch_conv(const CUtensorMap& ta, const CUtensorMap& ta2, const CUte
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   const int grid = g.items < 2 * sms ? g.items : 2 * sms;
-  kern<<<grid, kConvThreads, kSmem, st>>>(ta, ta2, tw, tc, g);
+  kern<<<grid, kConvThreads, kSmem, st>>>(ta, ta2, tw, tc, g, talo, talo2, twlo);
   UNREAL_LAUNCH_CHECK("conv_fwd_tcgen05_kernel");
   return UNREAL_OK;
 }
@@ -1551,7 +1637,7 @@ static int launch_conv(const CUtensorMap& ta, const CUtensorMap& ta2, const CUte
 
 using namespace unreal;
 
-extern "C" int unreal_s2d_frames(const void* frames, int dtype, void* out_bf16, int s, void* stream) {
+static int s2d_frames_impl(const void* frames, int dtype, void* out_bf16, void* out_lo_bf16, int s, void* stream) {
   UNREAL_REQUIRE(frames && out_bf16 && s > 0, "unreal_s2d_frames: null buffer or s <= 0");
   UNREAL_REQUIRE(dtype == UNREAL_F32 || dtype == UNREAL_U8, "unreal_s2d_frames: frames must be f32 or u8");
   UNREAL_REQUIRE(aligned16(frames) && aligned16(out_bf16), "unreal_s2d_frames: buffers must be 16-byte aligned");
@@ -1560,13 +1646,53 @@ extern "C" int unreal_s2d_frames(const void* frames, int dtype, void* out_bf16, 
   if (sms <= 0) return UNREAL_ECUDA;
   int64_t want = (total + 255) / 256;
   const int grid = (int)(want < (int64_t)sms * 16 ? want : (int64_t)sms * 16);
-  if (dtype == UNREAL_F32)
-    s2d_frames_kernel<float><<<grid, 256, 0, as_stream(stream)>>>(reinterpret_cast<const float*>(frames),
-                                                                 reinterpret_cast<__nv_bfloat16*>(out_bf16), total, 0x4B000000u);
+  auto* hi = reinterpret_cast<__nv_bfloat16*>(out_bf16);
+  auto* lo = reinterpret_cast<__nv_bfloat16*>(out_lo_bf16);
+  if (dtype == UNREAL_F32 && lo)
+    s2d_frames_kernel<float, true><<<grid, 256, 0, as_stream(stream)>>>(reinterpret_cast<const float*>(frames), hi, total, 0x4B000000u, lo);
+  else if (dtype == UNREAL_F32)
+    s2d_frames_kernel<float><<<grid, 256, 0, as_stream(stream)>>>(reinterpret_cast<const float*>(frames), hi, total, 0x4B000000u, nullptr);
+  else if (lo)
+    s2d_frames_kernel<uint8_t, true><<<grid, 256, 0, as_stream(stream)>>>(reinterpret_cast<const uint8_t*>(frames), hi, total, 0x4B000000u, lo);
   else
-    s2d_frames_kernel<uint8_t><<<grid, 256, 0, as_stream(stream)>>>(reinterpret_cast<const uint8_t*>(frames),
-                                                                   reinterpret_cast<__nv_bfloat16*>(out_bf16), total, 0x4B000000u);
+    s2d_frames_kernel<uint8_t><<<grid, 256, 0, as_stream(stream)>>>(reinterpret_cast<const uint8_t*>(frames), hi, total, 0x4B000000u, nullptr);
   UNREAL_LAUNCH_CHECK("s2d_frames_kernel");
+  return UNREAL_OK;
+}
+
+extern "C" int unreal_s2d_frames(const void* frames, int dtype, void* out_bf16, int s, void* stream) {
+  return s2d_frames_impl(frames, dtype, out_bf16, nullptr, s, stream);
+}
+
+extern "C" int unreal_s2d_frames_split(const void* frames, int dtype, void* out_hi_bf16, void* out_lo_bf16, int s, void* stream) {
+  UNREAL_REQUIRE(out_lo_bf16 && aligned16(out_lo_bf16), "unreal_s2d_frames_split: null or unaligned lo planes");
+  return s2d_frames_impl(frames, dtype, out_hi_bf16, out_lo_bf16, s, stream);
+}
+
+// conv1 forward over x'' planes (pos == NULL) or render-fused over maze cells; SPLIT: w_lo / out_lo non-null, xpp_lo nullable
+template <bool SPLIT>
+static int conv1_fwd_launch(const void* xpp, const int32_t* pos, const void* w_taps, const float* bias, void* out, int s,
+                            void* stream, const void* xpp_lo = nullptr, const void* w_lo = nullptr, void* out_lo = nullptr) {
+  uint64_t walls = 0;
+  if (pos != nullptr) {
+    int rc = maze_walls49(&walls);
+    if (rc != UNREAL_OK) return rc;
+  }
+  constexpr int kSmem = SPLIT ? kC1SplitSmem : kC1Smem;
+  static bool configured = false;
+  if (!configured) {
+    UNREAL_CUDA(cudaFuncSetAttribute(conv1_fwd_tcgen05_kernel<SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem));
+    configured = true;
+  }
+  const int sms = sm_count();
+  if (sms <= 0) return UNREAL_ECUDA;
+  const int items = s * 4;
+  const int ctas = 2 * sms;
+  using bf = __nv_bfloat16;
+  conv1_fwd_tcgen05_kernel<SPLIT><<<items < ctas ? items : ctas, kConvThreads, kSmem, as_stream(stream)>>>(
+      reinterpret_cast<const bf*>(xpp), reinterpret_cast<const bf*>(w_taps), bias, reinterpret_cast<bf*>(out), items, pos, walls,
+      reinterpret_cast<const bf*>(xpp_lo), reinterpret_cast<const bf*>(w_lo), reinterpret_cast<bf*>(out_lo));
+  UNREAL_LAUNCH_CHECK(pos ? "conv1_fwd_tcgen05_kernel(maze)" : "conv1_fwd_tcgen05_kernel");
   return UNREAL_OK;
 }
 
@@ -1575,28 +1701,33 @@ extern "C" int unreal_conv1_fwd_maze(const int32_t* pos, const void* w_taps_bf16
   UNREAL_REQUIRE(pos && w_taps_bf16 && out_bf16 && s > 0, "unreal_conv1_fwd_maze: null buffer or s <= 0");
   UNREAL_REQUIRE(aligned16(w_taps_bf16) && aligned16(out_bf16) && (reinterpret_cast<uintptr_t>(pos) & 7u) == 0,
                  "unreal_conv1_fwd_maze: alignment (pos 8, buffers 16 bytes)");
-  uint64_t walls = 0;
-  int rc = maze_walls49(&walls);
-  if (rc != UNREAL_OK) return rc;
-  static bool configured = false;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(conv1_fwd_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kC1Smem));
-    configured = true;
-  }
-  const int sms = sm_count();
-  if (sms <= 0) return UNREAL_ECUDA;
-  const int items = s * 4;
-  const int ctas = 2 * sms;
-  conv1_fwd_tcgen05_kernel<<<items < ctas ? items : ctas, kConvThreads, kC1Smem, as_stream(stream)>>>(
-      nullptr, reinterpret_cast<const __nv_bfloat16*>(w_taps_bf16), bias, reinterpret_cast<__nv_bfloat16*>(out_bf16), items,
-      pos, walls);
-  UNREAL_LAUNCH_CHECK("conv1_fwd_tcgen05_kernel(maze)");
-  return UNREAL_OK;
+  return conv1_fwd_launch<false>(nullptr, pos, w_taps_bf16, bias, out_bf16, s, stream);
+}
+
+extern "C" int unreal_conv1_fwd_maze_split(const int32_t* pos, const void* w_hi_bf16, const void* w_lo_bf16, const float* bias,
+                                           void* out_hi_bf16, void* out_lo_bf16, int s, void* stream) {
+  UNREAL_REQUIRE(pos && w_hi_bf16 && w_lo_bf16 && out_hi_bf16 && out_lo_bf16 && s > 0,
+                 "unreal_conv1_fwd_maze_split: null buffer or s <= 0");
+  UNREAL_REQUIRE(aligned16(w_hi_bf16) && aligned16(w_lo_bf16) && aligned16(out_hi_bf16) && aligned16(out_lo_bf16) &&
+                 (reinterpret_cast<uintptr_t>(pos) & 7u) == 0, "unreal_conv1_fwd_maze_split: alignment (pos 8, buffers 16 bytes)");
+  return conv1_fwd_launch<true>(nullptr, pos, w_hi_bf16, bias, out_hi_bf16, s, stream, nullptr, w_lo_bf16, out_lo_bf16);
+}
+
+extern "C" int unreal_conv1_fwd_split(const void* xpp_hi_bf16, const void* xpp_lo_bf16, const void* w_hi_bf16,
+                                      const void* w_lo_bf16, const float* bias, void* out_hi_bf16, void* out_lo_bf16, int s,
+                                      void* stream) {
+  UNREAL_REQUIRE(xpp_hi_bf16 && w_hi_bf16 && w_lo_bf16 && out_hi_bf16 && out_lo_bf16 && s > 0,
+                 "unreal_conv1_fwd_split: null buffer or s <= 0");
+  UNREAL_REQUIRE(aligned16(xpp_hi_bf16) && (xpp_lo_bf16 == nullptr || aligned16(xpp_lo_bf16)) && aligned16(w_hi_bf16) &&
+                 aligned16(w_lo_bf16) && aligned16(out_hi_bf16) && aligned16(out_lo_bf16),
+                 "unreal_conv1_fwd_split: buffers must be 16-byte aligned");
+  return conv1_fwd_launch<true>(xpp_hi_bf16, nullptr, w_hi_bf16, bias, out_hi_bf16, s, stream, xpp_lo_bf16, w_lo_bf16,
+                                out_lo_bf16);
 }
 
 static int conv_fwd_impl(const void* in_bf16, int layer, const void* w_taps_bf16, const float* bias, void* out_bf16, int s,
                          int relu, void* stream, const float* scale = nullptr, const void* mask_y = nullptr,
-                         float* db = nullptr, int c_in = 16) {
+                         float* db = nullptr, int c_in = 16, const void* in_lo_bf16 = nullptr, const void* w_lo_bf16 = nullptr) {
   UNREAL_REQUIRE(in_bf16 && w_taps_bf16 && out_bf16 && s > 0, "unreal_conv_fwd: null buffer or s <= 0");
   UNREAL_REQUIRE(mask_y == nullptr || (layer == 2 && bias == nullptr && !relu && aligned16(mask_y)),
                  "unreal_conv2_fwd_linear_masked: conv2 geometry, no bias / ReLU, 16-byte aligned mask");
@@ -1604,7 +1735,8 @@ static int conv_fwd_impl(const void* in_bf16, int layer, const void* w_taps_bf16
   UNREAL_REQUIRE(layer == 1 || layer == 2, "unreal_conv_fwd: layer must be 1 (conv1 over x') or 2 (conv2 over h1)");
   UNREAL_REQUIRE(aligned16(in_bf16) && aligned16(w_taps_bf16) && aligned16(out_bf16),
                  "unreal_conv_fwd: buffers must be 16-byte aligned");
-  CUtensorMap ta, ta2, tw, tc;
+  const bool split = in_lo_bf16 != nullptr;     // conv2 only (the split conv1 has its own entry point)
+  CUtensorMap ta, ta2, tw, tc, talo, talo2, twlo;
   ConvArgs g;
   g.bias = bias;
   g.mode = layer;
@@ -1616,20 +1748,7 @@ static int conv_fwd_impl(const void* in_bf16, int layer, const void* w_taps_bf16
   const int n = layer == 1 ? 16 : 32;
   if (layer == 1) {
     // x'' [S*6 planes][441 pixels][8 ch] bf16: the kernel bulk-copies 126-pixel plane slices
-    static bool configured = false;
-    if (!configured) {
-      UNREAL_CUDA(cudaFuncSetAttribute(conv1_fwd_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kC1Smem));
-      configured = true;
-    }
-    const int sms = sm_count();
-    if (sms <= 0) return UNREAL_ECUDA;
-    const int items = s * 4;
-    const int ctas = 2 * sms;
-    conv1_fwd_tcgen05_kernel<<<items < ctas ? items : ctas, kConvThreads, kC1Smem, as_stream(stream)>>>(
-        reinterpret_cast<const __nv_bfloat16*>(in_bf16), reinterpret_cast<const __nv_bfloat16*>(w_taps_bf16), bias,
-        reinterpret_cast<__nv_bfloat16*>(out_bf16), items, nullptr, 0ull);
-    UNREAL_LAUNCH_CHECK("conv1_fwd_tcgen05_kernel");
-    return UNREAL_OK;
+    return conv1_fwd_launch<false>(in_bf16, nullptr, w_taps_bf16, bias, out_bf16, s, stream);
   } else {
     // h1 [S][20][20][16]: image rows y = 2Y' + dy as {64 (4 pixels x 16 c), 9 X (stride 2 pixels: rows overlap),
     // 10 Y', S}, one map per dy; the box at Y' = by is filter row ky = 2by+dy for all 81 outputs
@@ -1641,6 +1760,11 @@ static int conv_fwd_impl(const void* in_bf16, int layer, const void* w_taps_bf16
     rc = make_tma_nd_bf16(&ta, in_bf16, 4, dims, strides, box, 2 * (int)c4);
     if (rc != UNREAL_OK) return rc;
     rc = make_tma_nd_bf16(&ta2, reinterpret_cast<const uint8_t*>(in_bf16) + 10 * c4, 4, dims, strides, box, 2 * (int)c4);
+    if (rc == UNREAL_OK && split) {
+      rc = make_tma_nd_bf16(&talo, in_lo_bf16, 4, dims, strides, box, 2 * (int)c4);
+      if (rc == UNREAL_OK)
+        rc = make_tma_nd_bf16(&talo2, reinterpret_cast<const uint8_t*>(in_lo_bf16) + 10 * c4, 4, dims, strides, box, 2 * (int)c4);
+    }
     g.items = s; g.rows = 81; g.box_bytes = (int)c4 * 9 * 9 * 2;
   }
   if (rc != UNREAL_OK) return rc;
@@ -1650,6 +1774,7 @@ static int conv_fwd_impl(const void* in_bf16, int layer, const void* w_taps_bf16
     const uint64_t strides[1] = {8 * k_row};
     const uint32_t box[2] = {(uint32_t)k_row, (uint32_t)n};
     rc = make_tma_nd_bf16(&tw, w_taps_bf16, 2, dims, strides, box, 2 * (int)k_row);
+    if (rc == UNREAL_OK && split) rc = make_tma_nd_bf16(&twlo, w_lo_bf16, 2, dims, strides, box, 2 * (int)k_row);
     if (rc != UNREAL_OK) return rc;
   }
   {
@@ -1660,14 +1785,24 @@ static int conv_fwd_impl(const void* in_bf16, int layer, const void* w_taps_bf16
     rc = make_tma_nd_bf16(&tc, out_bf16, 3, dims, strides, box, 128);
     if (rc != UNREAL_OK) return rc;
   }
-  if (mask_y != nullptr && c_in == 8) return launch_conv<32, 2, true, 8>(ta, ta2, tw, tc, g, as_stream(stream));
-  if (mask_y != nullptr) return launch_conv<32, 2, true>(ta, ta2, tw, tc, g, as_stream(stream));
-  return launch_conv<32, 2>(ta, ta2, tw, tc, g, as_stream(stream));
+  cudaStream_t st = as_stream(stream);
+  if (split) return launch_conv<32, 2, false, 16, true>(ta, ta2, tw, tc, g, st, talo, talo2, twlo);
+  if (mask_y != nullptr && c_in == 8) return launch_conv<32, 2, true, 8>(ta, ta2, tw, tc, g, st, ta, ta2, tw);
+  if (mask_y != nullptr) return launch_conv<32, 2, true>(ta, ta2, tw, tc, g, st, ta, ta2, tw);
+  return launch_conv<32, 2>(ta, ta2, tw, tc, g, st, ta, ta2, tw);
 }
 
 extern "C" int unreal_conv_fwd(const void* in_bf16, int layer, const void* w_taps_bf16, const float* bias,
                                void* out_bf16, int s, void* stream) {
   return conv_fwd_impl(in_bf16, layer, w_taps_bf16, bias, out_bf16, s, 1, stream);
+}
+
+extern "C" int unreal_conv2_fwd_split(const void* h1_hi_bf16, const void* h1_lo_bf16, const void* w_hi_bf16,
+                                      const void* w_lo_bf16, const float* bias, void* out_bf16, int s, void* stream) {
+  UNREAL_REQUIRE(h1_lo_bf16 && w_lo_bf16 && aligned16(h1_lo_bf16) && aligned16(w_lo_bf16),
+                 "unreal_conv2_fwd_split: null or unaligned lo operand");
+  return conv_fwd_impl(h1_hi_bf16, 2, w_hi_bf16, bias, out_bf16, s, 1, stream, nullptr, nullptr, nullptr, 16, h1_lo_bf16,
+                       w_lo_bf16);
 }
 
 extern "C" int unreal_conv2_fwd_linear(const void* in_bf16, const void* w_taps_bf16, void* out_bf16, int s, void* stream) {

@@ -764,6 +764,57 @@ def conv1_fwd_maze(pos, w_taps, bias, out=None):
   return out
 
 
+def split_bf16(w32):
+  """fp32 tensor -> (hi, lo) bf16 with hi = bf16(w), lo = bf16(w - hi): hi + lo holds w to about 16 mantissa bits."""
+  hi = w32.to(torch.bfloat16)
+  return hi, (w32 - hi.float()).to(torch.bfloat16)
+
+
+def s2d_frames_split(frames):
+  """frames [S,84,84,3] f32 / u8 -> (x'' hi, x'' lo) bf16 [S,6,441,8] each, as s2d_frames; lo = bf16(x - hi)."""
+  s = frames.shape[0]
+  if tuple(frames.shape[1:]) != (84, 84, 3):
+    raise _lib.UnrealError("s2d_frames_split expects [S,84,84,3] frames")
+  hi = torch.empty(s, 6, 441, 8, dtype=torch.bfloat16, device=frames.device)
+  lo = torch.empty_like(hi)
+  call("unreal_s2d_frames_split", ptr(frames, None, "frames"), _lib.dtype_tag(frames), ptr(hi, torch.bfloat16, "hi"),
+       ptr(lo, torch.bfloat16, "lo"), s, stream_ptr())
+  return hi, lo
+
+
+def conv1_fwd_split(xpp_hi, xpp_lo, w_hi, w_lo, bias):
+  """Split-bf16 conv1: x'' hi / lo planes [S,6,441,8] (xpp_lo None: the input is exactly bf16), filter planes hi / lo
+  (conv1_w_planes of both halves) -> h1 = relu(conv + bias) as (hi, lo) bf16 [S,20,20,16]."""
+  s = xpp_hi.shape[0]
+  hi = torch.empty(s, 20, 20, 16, dtype=torch.bfloat16, device=xpp_hi.device)
+  lo = torch.empty_like(hi)
+  call("unreal_conv1_fwd_split", ptr(xpp_hi, torch.bfloat16, "xpp_hi"), ptr(xpp_lo, torch.bfloat16, "xpp_lo"),
+       ptr(w_hi, torch.bfloat16, "w_hi"), ptr(w_lo, torch.bfloat16, "w_lo"), ptr(bias, torch.float32, "bias"),
+       ptr(hi, torch.bfloat16, "hi"), ptr(lo, torch.bfloat16, "lo"), s, stream_ptr())
+  return hi, lo
+
+
+def conv1_fwd_maze_split(pos, w_hi, w_lo, bias):
+  """Split-bf16 render-fused conv1: pos [S,2] i32 -> h1 (hi, lo) bf16 [S,20,20,16]."""
+  s = pos.shape[0]
+  hi = torch.empty(s, 20, 20, 16, dtype=torch.bfloat16, device=pos.device)
+  lo = torch.empty_like(hi)
+  call("unreal_conv1_fwd_maze_split", ptr(pos, torch.int32, "pos"), ptr(w_hi, torch.bfloat16, "w_hi"),
+       ptr(w_lo, torch.bfloat16, "w_lo"), ptr(bias, torch.float32, "bias"), ptr(hi, torch.bfloat16, "hi"),
+       ptr(lo, torch.bfloat16, "lo"), s, stream_ptr())
+  return hi, lo
+
+
+def conv2_fwd_split(h1_hi, h1_lo, w_hi, w_lo, bias):
+  """Split-bf16 conv2: h1 hi / lo [S,20,20,16], filters hi / lo (conv_taps of both halves) -> h2 bf16 [S,9,9,32]."""
+  s = h1_hi.shape[0]
+  out = torch.empty(s, 9, 9, 32, dtype=torch.bfloat16, device=h1_hi.device)
+  call("unreal_conv2_fwd_split", ptr(h1_hi, torch.bfloat16, "h1_hi"), ptr(h1_lo, torch.bfloat16, "h1_lo"),
+       ptr(w_hi, torch.bfloat16, "w_hi"), ptr(w_lo, torch.bfloat16, "w_lo"), ptr(bias, torch.float32, "bias"),
+       ptr(out, torch.bfloat16, "out"), s, stream_ptr())
+  return out
+
+
 def conv1_wgrad_maze(pos, dy_planes21):
   """Render-fused conv1 filter gradient: pos [S,2] i32, dy planes [2, S*420, 8] bf16 -> HWIO [8,8,3,16] f32."""
   s = pos.shape[0]

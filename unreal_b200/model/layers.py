@@ -158,20 +158,35 @@ class EncoderFn(torch.autograd.Function):
   and bias gradient directly (`unreal_conv2_dgrad_relu`) -- the dense [S,20,20,16] gradient and the separate
   ReLU-gradient pass over it (38 KB per frame of HBM traffic) do not exist.  Frames: f32 / u8 [S,84,84,3], the
   space-to-depth planes bf16 [S,6,441,8], or maze CELLS int32 [S,2] (the conv1 kernels then synthesise their
-  input tiles in shared memory: unreal_conv1_fwd_maze / unreal_conv1_wgrad_maze)."""
+  input tiles in shared memory: unreal_conv1_fwd_maze / unreal_conv1_wgrad_maze).
+
+  taps_lo = (conv1 planes, conv2 taps) of the filters' rounding residuals bf16(W - bf16(W)): the split-bf16 forward
+  (UnrealModel(encoder_precision='bf16x3')).  Frames, conv1's output and the filters enter conv1 and conv2 as hi + lo
+  bf16 pairs (three tensor-core passes; two where the input is exactly bf16: maze cells, x'' planes), so the forward
+  products are fp32-grade.  Only the hi halves are kept for the backward pass, which is the bf16 one: the gradient
+  rounding it adds is far below the forward rounding the split removes."""
 
   @staticmethod
-  def forward(ctx, x, w1_32, b1_32, w2_32, b2_32, taps1, taps2):
+  def forward(ctx, x, w1_32, b1_32, w2_32, b2_32, taps1, taps2, taps_lo=None):
     pre_s2d = x.dtype == torch.bfloat16 and tuple(x.shape[1:]) == (6, 441, 8)
     s = x.shape[0]
     ctx.cells = x.dtype == torch.int32                          # maze cells [S,2]: render-fused conv1, no frame in HBM
-    if ctx.cells:
-      xpp = x.contiguous()
-      h1 = K.conv1_fwd_maze(xpp, taps1, b1_32)
+    if taps_lo is not None:
+      if ctx.cells:
+        xpp = x.contiguous()
+        h1, h1_lo = K.conv1_fwd_maze_split(xpp, taps1, taps_lo[0], b1_32)
+      else:
+        xpp, xpp_lo = (x, None) if pre_s2d else K.s2d_frames_split(x)
+        h1, h1_lo = K.conv1_fwd_split(xpp, xpp_lo, taps1, taps_lo[0], b1_32)
+      h2 = K.conv2_fwd_split(h1, h1_lo, taps2[0], taps_lo[1], b2_32)
     else:
-      xpp = x if pre_s2d else K.s2d_frames(x)
-      h1 = K.conv_fwd(xpp, 1, taps1, b1_32)                    # bf16 [S,20,20,16]
-    h2 = K.conv_fwd(h1.view(s, 20, 20, 16), 2, taps2[0], b2_32)
+      if ctx.cells:
+        xpp = x.contiguous()
+        h1 = K.conv1_fwd_maze(xpp, taps1, b1_32)
+      else:
+        xpp = x if pre_s2d else K.s2d_frames(x)
+        h1 = K.conv_fwd(xpp, 1, taps1, b1_32)                  # bf16 [S,20,20,16]
+      h2 = K.conv_fwd(h1.view(s, 20, 20, 16), 2, taps2[0], b2_32)
     ctx.dtaps = taps2[1]
     ctx.save_for_backward(xpp, h1, h2)
     return h2.view(s, 9, 9, 32)
@@ -184,7 +199,7 @@ class EncoderFn(torch.autograd.Function):
     dw2 = K.conv2_wgrad(h1.view(s, 20, 20, 16), dy2)
     dy1_planes, db1 = K.conv2_dgrad_relu(dy2, ctx.dtaps, h1, pitch21=True)
     dw1 = K.conv1_wgrad_maze(xpp, dy1_planes) if ctx.cells else K.conv1_wgrad(xpp, dy1_planes)
-    return None, dw1, db1, dw2, db2, None, None
+    return None, dw1, db1, dw2, db2, None, None, None
 
 
 class LstmFn(torch.autograd.Function):

@@ -53,8 +53,13 @@ class UnrealModel(object):
   def __init__(self, action_size, objective_size, thread_index, use_lstm, use_pixel_change, use_value_replay,
                use_reward_prediction, pixel_change_lambda, entropy_beta, device, segnet_param_dict=None,
                image_shape=(84, 84), is_training=True, n_classes=0, segnet_lambda=0.0, dropout=0.0,
-               for_display=False, num_envs=1, seed=0):
+               for_display=False, num_envs=1, seed=0, encoder_precision='bf16'):
     _lib.require_device()
+    if encoder_precision not in ('bf16', 'bf16x3'):
+      raise _lib.UnrealError("encoder_precision must be 'bf16' or 'bf16x3', got %r" % (encoder_precision,))
+    # 'bf16x3': conv1 and conv2 forward on split-bf16 operands (fp32-grade products, the reference's arithmetic); fixed at
+    # construction because the filter shadows it needs are built by refresh_shadow and captured by CUDA graphs
+    self._encoder_precision = encoder_precision
     segnet_param_dict = segnet_param_dict or {'segnet_mode': 0}
     if segnet_param_dict.get('segnet_mode', 0) != 0:
       raise _lib.UnrealError("segnet_mode != 0 (ErfNet encoder/decoder) is outside the B200 hot path")
@@ -144,6 +149,11 @@ class UnrealModel(object):
     self._offsets = offsets
     self.refresh_shadow()
 
+  @property
+  def encoder_precision(self):
+    """'bf16' (bf16 operands, fp32 accumulation) or 'bf16x3' (split-bf16 operands in conv1 and conv2's forward pass)."""
+    return self._encoder_precision
+
   def _views(self, flat):
     if torch.is_grad_enabled() and flat.requires_grad:      # one autograd node for all variables (layers.FlatViewsFn)
       return OrderedDict(zip((name for name, _, _, _ in self._offsets), FlatViewsFn.apply(flat, self._offsets)))
@@ -169,8 +179,18 @@ class UnrealModel(object):
         self.taps1, self.taps2 = t1, (t2, d2)
       else:
         self.taps1.copy_(t1); self.taps2[0].copy_(t2); self.taps2[1].copy_(d2)
+      if self._encoder_precision == 'bf16x3':
+        # the same tap layouts of the rounding residuals bf16(W - bf16(W)) (the hi halves are taps1 / taps2[0])
+        with torch.no_grad():
+          v32 = self._views(self.flat)
+          l1 = K.conv1_w_planes(K.split_bf16(v32["W_base_conv1"])[1])
+          l2 = K.conv_taps(K.split_bf16(v32["W_base_conv2"])[1], 2)
+        if getattr(self, "taps_lo", None) is None:
+          self.taps_lo = (l1, l2)
+        else:
+          self.taps_lo[0].copy_(l1); self.taps_lo[1].copy_(l2)
     else:
-      self.taps1 = self.taps2 = None
+      self.taps1 = self.taps2 = self.taps_lo = None
     if self._use_reward_prediction:
       # W_rp [7776,3] as a bf16 [7776,8] shadow (zero columns 3..7): the B operand of the head's tcgen05 GEMM
       if getattr(self, "rp_w8", None) is None:
@@ -183,8 +203,7 @@ class UnrealModel(object):
       # acting-side table fc1(conv2(conv1(frame of cell))) for all 49 cells, refreshed IN PLACE with the parameters
       with torch.no_grad():
         p32 = self._views(self.flat)
-        h2 = EncoderFn.apply(self._cells49, p32["W_base_conv1"], p32["b_base_conv1"], p32["W_base_conv2"], p32["b_base_conv2"],
-                             self.taps1, self.taps2)
+        h2 = self._encoder_fn(p32, self._cells49)
         K.gemm_bf16(h2.view(49, 2592), self.v16["W_base_fc1"], out=self._fc_tab_act, b_mn_major=True, bias=p32["b_base_fc1"],
                     relu=True)
     if self._use_pixel_change:
@@ -234,12 +253,18 @@ class UnrealModel(object):
     self.refresh_shadow()
 
   # ---- towers -------------------------------------------------------------------------
+  def _encoder_fn(self, p32, images):
+    """The fused encoder node (EncoderFn) in this model's encoder precision."""
+    return EncoderFn.apply(images, p32["W_base_conv1"], p32["b_base_conv1"], p32["W_base_conv2"], p32["b_base_conv2"],
+                           self.taps1, self.taps2, self.taps_lo if self._encoder_precision == 'bf16x3' else None)
+
   def _encoder(self, p32, images):
     """model.py:281-289.  images [S,84,84,3] f32 / u8, x'' planes bf16 [S,6,441,8] or maze cells int32 [S,2]
     -> h2 bf16 [S,9,9,32]."""
     if self.fused_conv and self.fused_encoder:
-      return EncoderFn.apply(images, p32["W_base_conv1"], p32["b_base_conv1"], p32["W_base_conv2"], p32["b_base_conv2"],
-                             self.taps1, self.taps2)
+      return self._encoder_fn(p32, images)
+    if self._encoder_precision != 'bf16':
+      raise _lib.UnrealError("encoder_precision 'bf16x3' needs the fused encoder (fused_conv and fused_encoder)")
     if images.dtype == torch.int32:
       raise _lib.UnrealError("cell observations (int32 [S,2]) need the fused encoder (fused_conv and fused_encoder)")
     h1 = ConvFn.apply(images, self.v16["W_base_conv1"].view(192, 16), p32["W_base_conv1"], p32["b_base_conv1"], 8, 8, 4,
@@ -265,8 +290,7 @@ class UnrealModel(object):
   def _cell_tables(self, p32):
     """(h2 table bf16 [49,2592], fc1 table f32 [49,256]) of the 49 maze cells, inside the autograd graph: every tower of
     the update gathers its rows from them, and their gradients arrive as per-cell sums."""
-    h2t = EncoderFn.apply(self._cells49, p32["W_base_conv1"], p32["b_base_conv1"], p32["W_base_conv2"], p32["b_base_conv2"],
-                          self.taps1, self.taps2).view(49, 2592)
+    h2t = self._encoder_fn(p32, self._cells49).view(49, 2592)
     fct = LinearFn.apply(h2t, self.v16["W_base_fc1"], p32["W_base_fc1"], p32["b_base_fc1"], True, True)
     return h2t, fct.float()
 
@@ -385,8 +409,7 @@ class UnrealModel(object):
     if self._use_tables(images):      # maze cells: fc1's output is a row of the 49-entry table (refresh_shadow)
       K.cell_gather(self._fc_tab_act, images.reshape(n, 2), out=xh[:, :256])
     else:
-      h2 = EncoderFn.apply(images, p32["W_base_conv1"], p32["b_base_conv1"], p32["W_base_conv2"], p32["b_base_conv2"],
-                           self.taps1, self.taps2)
+      h2 = self._encoder_fn(p32, images)
       K.gemm_bf16(h2.view(n, 2592), self.v16["W_base_fc1"], out=xh[:, :256], b_mn_major=True, bias=p32["b_base_fc1"], relu=True)
     xh[:, 256:self.lstm_in].copy_(lar)
     xh[:, self.kx:].copy_(h_prev)
