@@ -46,9 +46,23 @@ def _operands(s, seed):
 def _cells(s):
   from oracle import unreal_oracle as O
   free = [(x, y) for y in range(7) for x in range(7) if not O.WALLS[y, x]]
-  pos = [free[i % len(free)] for i in range(s)]
-  frames = np.stack([O.maze_render(x, y) for x, y in pos]).astype(np.float32)
-  return torch.tensor(pos, dtype=torch.int32, device=DEV), torch.from_numpy(frames).to(DEV)
+  idx = torch.arange(s, device=DEV) % len(free)
+  frames = torch.from_numpy(np.stack([O.maze_render(x, y) for x, y in free]).astype(np.float32)).to(DEV)
+  return torch.tensor(free, dtype=torch.int32, device=DEV)[idx].contiguous(), frames[idx]
+
+
+def _samples(s):
+  """Sample count of a parameter: a number, or one of the multi-item sizes of test_gpu_model (several work items per
+  CTA of the persistent conv kernels, derived from the SM count)."""
+  from test_gpu_model import conv_multi_item_sizes, items_per_cta
+  if isinstance(s, int):
+    return s
+  n = dict(zip(("past-one-wave", "8-items-per-cta"), conv_multi_item_sizes()))[s]
+  assert items_per_cta(n) >= (8 if s == "8-items-per-cta" else 2)
+  return n
+
+
+SIZES = [1, 3, 129, "past-one-wave", "8-items-per-cta", 20480]
 
 
 def _frames(kind, s, g):
@@ -60,10 +74,11 @@ def _frames(kind, s, g):
 
 
 # ---- the kernels ---------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("s", [1, 3, 129])
+@pytest.mark.parametrize("s", SIZES)
 @pytest.mark.parametrize("source", ["f32", "u8", "cells"])
 def test_split_conv1_is_30x_closer_to_fp64_than_bf16(source, s):
   from unreal_b200 import kernels as K
+  s = _samples(s)
   g, w1, b1, _, _ = _operands(s, 11 + s)
   w_hi, w_lo = K.split_bf16(w1)
   t_hi, t_lo = K.conv1_w_planes(w_hi), K.conv1_w_planes(w_lo)
@@ -87,11 +102,12 @@ def test_split_conv1_is_30x_closer_to_fp64_than_bf16(source, s):
   assert bool((lo.float().abs() <= hi.float().abs() * 2 ** -8 + 1e-30).all())
 
 
-@pytest.mark.parametrize("s", [1, 3, 129])
+@pytest.mark.parametrize("s", SIZES)
 def test_split_conv2_is_30x_closer_to_fp64_than_bf16(s):
   """conv2 writes h2 as bf16 in both modes, so both are compared with the correctly rounded fp64 result: the split
   kernel misses it only where the fp32 error crosses a rounding boundary."""
   from unreal_b200 import kernels as K
+  s = _samples(s)
   g, _, _, w2, b2 = _operands(s, 21 + s)
   h1 = torch.relu(torch.randn(s, 20, 20, 16, device=DEV, generator=g))
   h_hi, h_lo = K.split_bf16(h1)
@@ -105,9 +121,10 @@ def test_split_conv2_is_30x_closer_to_fp64_than_bf16(s):
   assert err_split * 30 <= err_bf16, (err_split, err_bf16)
 
 
-@pytest.mark.parametrize("s", [1, 3, 129])
+@pytest.mark.parametrize("s", SIZES)
 def test_split_kernels_with_zero_lo_equal_the_bf16_kernels(s):
   from unreal_b200 import kernels as K
+  s = _samples(s)
   g, w1, b1, w2, b2 = _operands(s, 31 + s)
   t1 = K.conv1_w_planes(w1.to(torch.bfloat16))
   z1 = torch.zeros_like(t1)

@@ -269,15 +269,45 @@ def test_update_applies_rmsprop_like_the_oracle():
   assert torch.equal(m.flat16.float(), m.flat.detach().to(torch.bfloat16).float())
 
 
+def _sms():
+  return torch.cuda.get_device_properties(0).multi_processor_count
+
+
+def conv_multi_item_sizes():
+  """Sample counts that run the persistent conv kernels (grid = min(items, 2 CTAs per SM)) through several work items
+  per CTA, for the kernels with one item per sample (conv2 forward, the transposed convolutions; conv1 has 4 per
+  sample): just past one wave, kStages + 2 = 8 items per CTA (ConvCfg<2,16>::kStages = 6: the stage ring wraps across
+  items), and config 5's batch of 1024 envs x T = 20."""
+  grid = 2 * _sms()
+  sizes = (grid + 1, 8 * grid, 20480)
+  assert items_per_cta(sizes[1]) >= 8 and items_per_cta(sizes[2]) >= 3
+  return sizes
+
+
+def items_per_cta(items):
+  """Most work items one CTA of a persistent conv kernel runs."""
+  grid = min(items, 2 * _sms())
+  return -(-items // grid)
+
+
+def _conv64(x, w_oihw, b=None, stride=1, transpose=False):
+  """conv2d / conv_transpose2d in float64 on NHWC tensors (NCHW-ordered weights) -> NHWC float64."""
+  import torch.nn.functional as F
+  op = F.conv_transpose2d if transpose else F.conv2d
+  y = op(x.double().permute(0, 3, 1, 2), w_oihw.double(), None if b is None else b.double(), stride=stride)
+  return y.permute(0, 2, 3, 1)
+
+
 @pytest.mark.parametrize("dtype", [torch.float32, torch.uint8])
 def test_fused_conv_forward_matches_direct_convolution(dtype):
-  """TMA-im2col convolutions (space-to-depth taps) against torch's conv2d on the same bf16-rounded
-  operands in fp32: only the fp32 summation order differs -> one bf16 ulp (2^-8 relative)."""
+  """TMA-im2col convolutions (space-to-depth taps) against conv2d on the same bf16-rounded operands in float64: the
+  kernels' fp32 sums and their bf16 output -> one bf16 ulp (2^-8 relative).  Every output row is compared, up to
+  S = 20 480 (many items per CTA)."""
   from unreal_b200 import kernels as K
-  import torch.nn.functional as F
   dev = torch.device("cuda", 0)
   g = torch.Generator(device=dev).manual_seed(3)
-  for s in (1, 5, 37):
+  assert items_per_cta(20480) >= 3 and items_per_cta(4 * 20480) >= 3
+  for s in (1, 5, 37) + conv_multi_item_sizes():
     if dtype == torch.uint8:
       x = torch.randint(0, 256, (s, 84, 84, 3), device=dev, dtype=torch.uint8, generator=g)
       xf = (x.float() / 255.0).to(torch.bfloat16).float()
@@ -292,20 +322,22 @@ def test_fused_conv_forward_matches_direct_convolution(dtype):
     want_s2d = xf.view(s, 21, 4, 21, 4, 3).permute(0, 1, 3, 2, 4, 5).reshape(s, 441, 6, 8).permute(0, 2, 1, 3)
     assert torch.equal(xs.float(), want_s2d)
     h1 = K.conv_fwd(xs, 1, K.conv1_w_planes(w1), b1)
-    ref1 = F.relu(F.conv2d(xf.permute(0, 3, 1, 2), w1.float().permute(3, 2, 0, 1), b1, stride=4)).permute(0, 2, 3, 1)
+    ref1 = torch.relu(_conv64(xf, w1.permute(3, 2, 0, 1), b1, stride=4))
+    del xs, xf, x
     assert tuple(h1.shape) == (s, 20, 20, 16)
-    assert torch.allclose(h1.float(), ref1, rtol=2.0 ** -7, atol=1e-3)
+    assert torch.allclose(h1.double(), ref1, rtol=2.0 ** -7, atol=1e-3), s
+    del ref1
     h2 = K.conv_fwd(h1, 2, K.conv_taps(w2, 2), b2)
     # transposed convolution (input gradient of conv2) through the zero-filling TMA boxes
     dy2 = (torch.randn(s * 81, 32, device=dev, generator=g) * 0.1).to(torch.bfloat16)
     dh1 = K.conv2_dgrad(dy2, K.conv2_dgrad_taps(w2))
-    ref_dh1 = F.conv_transpose2d(dy2.float().view(s, 9, 9, 32).permute(0, 3, 1, 2), w2.float().permute(3, 2, 0, 1),
-                                 stride=2).permute(0, 2, 3, 1)
+    ref_dh1 = _conv64(dy2.view(s, 9, 9, 32), w2.permute(3, 2, 0, 1), stride=2, transpose=True)
     assert tuple(dh1.shape) == (s, 20, 20, 16)
-    assert torch.allclose(dh1.float(), ref_dh1, rtol=2.0 ** -7, atol=1e-3)
-    ref2 = F.relu(F.conv2d(h1.float().permute(0, 3, 1, 2), w2.float().permute(3, 2, 0, 1), b2, stride=2)).permute(0, 2, 3, 1)
+    assert torch.allclose(dh1.double(), ref_dh1, rtol=2.0 ** -7, atol=1e-3), s
+    del ref_dh1, dh1
+    ref2 = torch.relu(_conv64(h1, w2.permute(3, 2, 0, 1), b2, stride=2))
     assert tuple(h2.shape) == (s, 9, 9, 32)
-    assert torch.allclose(h2.float(), ref2, rtol=2.0 ** -7, atol=1e-3)
+    assert torch.allclose(h2.double(), ref2, rtol=2.0 ** -7, atol=1e-3), s
 
 
 def test_fused_conv1_wgrad_matches_autograd():
@@ -385,21 +417,20 @@ def test_fused_conv2_wgrad_matches_autograd():
 
 def test_fused_pc_deconv_forward_matches_conv_transpose():
   """The pixel-control head's merged 8-channel deconv forward (conv2's transposed-convolution tcgen05
-  kernel at 8 channels, bias + ReLU epilogue) against torch conv_transpose2d in fp32 on the same
+  kernel at 8 channels, bias + ReLU epilogue) against torch conv_transpose2d in float64 on the same
   bf16-rounded operands, and against the GEMM + col2im path it replaces."""
   from unreal_b200 import kernels as K
-  import torch.nn.functional as F
   dev = torch.device("cuda", 0)
   g = torch.Generator(device=dev).manual_seed(21)
-  for s in (1, 3, 500):
+  for s in (1, 3, 500) + conv_multi_item_sizes():
     h = torch.rand(s, 9, 9, 32, device=dev, generator=g).to(torch.bfloat16)
     w8 = ((torch.rand(4, 4, 8, 32, device=dev, generator=g) - 0.5) * 0.2).to(torch.bfloat16)     # [kh,kw,out,in]
     b8 = (torch.rand(8, device=dev, generator=g) - 0.5) * 0.1
     y = K.pc_deconv_fwd(h, K.pc_deconv_taps(w8), b8)
     assert tuple(y.shape) == (s, 20, 20, 8) and y.dtype == torch.float32
-    ref = F.conv_transpose2d(h.float().permute(0, 3, 1, 2), w8.float().permute(3, 2, 0, 1), bias=b8, stride=2)
-    ref = torch.relu(ref).permute(0, 2, 3, 1)
-    assert torch.allclose(y, ref, rtol=1e-4, atol=1e-5), (s, float((y - ref).abs().max()))
+    ref = torch.relu(_conv64(h, w8.permute(3, 2, 0, 1), b8, stride=2, transpose=True))
+    assert torch.allclose(y.double(), ref, rtol=1e-4, atol=1e-5), (s, float((y - ref).abs().max()))
+    del ref
     cols = K.gemm_bf16(h.view(s * 81, 32), w8.view(128, 32))
     old = K.col2im(cols, s, 20, 20, 8, 4, 4, 2, bias=b8, relu=True)
     assert torch.allclose(y, old, rtol=1e-4, atol=1e-5)
@@ -411,7 +442,7 @@ def test_conv2_dgrad_relu_equals_dgrad_then_relu_grad():
   from unreal_b200 import kernels as K
   dev = torch.device("cuda", 0)
   g = torch.Generator(device=dev).manual_seed(5)
-  for s in (1, 3, 600):
+  for s in (1, 3, 600) + conv_multi_item_sizes():
     dy = (torch.randn(s * 81, 32, device=dev, generator=g) * 0.1).to(torch.bfloat16)
     w = ((torch.rand(4, 4, 16, 32, device=dev, generator=g) - 0.5) * 0.2).to(torch.bfloat16)
     h1 = torch.relu(torch.randn(s, 20, 20, 16, device=dev, generator=g)).to(torch.bfloat16)     # about half zeros
@@ -421,6 +452,13 @@ def test_conv2_dgrad_relu_equals_dgrad_then_relu_grad():
     planes, db = K.conv2_dgrad_relu(dy, taps, h1)
     assert torch.equal(planes, want_planes), s
     assert torch.allclose(db, want_db, rtol=1e-4, atol=1e-4 * float(want_db.abs().max() + 1e-6)), s
+    # independently: conv_transpose2d in float64, masked by h1 > 0; the planes hold it rounded once to bf16, the bias
+    # gradient is the sum of those rounded values over samples and pixels (fp32 partial sums and atomics)
+    ref = (_conv64(dy.view(s, 9, 9, 32), w.permute(3, 2, 0, 1), stride=2, transpose=True) * (h1 > 0)).reshape(s * 400, 16)
+    got = planes.permute(1, 0, 2).reshape(s * 400, 16).double()
+    assert torch.allclose(got, ref, rtol=2.0 ** -8, atol=1e-5), (s, float((got - ref).abs().max()))
+    assert torch.allclose(db.double(), got.sum(0), rtol=0, atol=1e-4 * float(got.abs().sum(0).max()) + 1e-6), s
+    del ref, got, dense
     # the 21-pixel-pitch form conv1's wgrad copies in one piece per plane: same values, zero column 20
     p21, _ = K.conv2_dgrad_relu(dy, taps, h1, pitch21=True)
     p21 = p21.view(2, s, 20, 21, 8)
@@ -461,10 +499,20 @@ def test_render_fused_conv1_equals_conv1_on_rendered_frames():
   want = K.conv_fwd(xpp, 1, taps, b1)
   got = K.conv1_fwd_maze(pos, taps, b1)
   assert torch.equal(got, want)
-  # and against the plain convolution of the oracle's float frame
+  # and every frame against the float64 convolution of the oracle's frame of its cell (0 / 1 pixels: the kernel's
+  # operands are exact, so only its fp32 sums and the bf16 output rounding differ) -- here and at sample counts with
+  # several conv1 items (4 per frame) per CTA, up to 20 480 frames
   frames = torch.from_numpy(np.stack([O.maze_render(x, y) for x, y in cells]).astype(np.float32)).to(dev)
-  ref = torch.relu(torch.nn.functional.conv2d(frames.permute(0, 3, 1, 2), w1.float().permute(3, 2, 0, 1), b1, stride=4))
-  assert torch.allclose(got[:len(cells)].float(), ref.permute(0, 2, 3, 1), rtol=2e-2, atol=2e-2)
+  ref_cell = torch.relu(_conv64(frames, w1.permute(3, 2, 0, 1), b1, stride=4))          # [cells, 20, 20, 16]
+  assert torch.allclose(got.double(), ref_cell.repeat(9, 1, 1, 1), rtol=2.0 ** -7, atol=1e-3)
+  assert items_per_cta(4 * s) >= 3
+  rs = np.random.RandomState(4)
+  for n in conv_multi_item_sizes():
+    idx = rs.randint(0, len(cells), size=n)
+    h = K.conv1_fwd_maze(pos[:len(cells)][torch.from_numpy(idx).to(dev)].contiguous(), taps, b1)
+    ref = ref_cell[torch.from_numpy(idx).to(dev)]
+    assert torch.allclose(h.double(), ref, rtol=2.0 ** -7, atol=1e-3), (n, float((h.double() - ref).abs().max()))
+    del h, ref
   dy = (torch.randn(2, s * 420, 8, device=dev, generator=g) * 0.1).to(torch.bfloat16)
   dy.view(2, s, 20, 21, 8)[:, :, :, 20] = 0
   a = K.conv1_wgrad_maze(pos, dy)
@@ -790,6 +838,26 @@ def test_pc_q_max_epilogue_equals_the_materialised_head():
     out[fused] = m.run_pc_q_max(None, {'image': frames}, lar).clone()
   assert tuple(out[True].shape) == (5, 20, 20)
   assert torch.allclose(out[True], out[False], rtol=1e-5, atol=1e-6)
+
+
+@pytest.mark.parametrize("na", [3, 4, 7])
+def test_pc_deconv_qmax_matches_the_dueling_max_in_float64(na):
+  """unreal_pc_deconv_qmax's epilogue (ReLU head, V + A - mean A, max over the `na` actions) against the same
+  arithmetic on conv_transpose2d in float64, at sample counts with several items per CTA (up to 20 480)."""
+  from unreal_b200 import kernels as K
+  dev = torch.device("cuda", 0)
+  g = torch.Generator(device=dev).manual_seed(40 + na)
+  for s in (5,) + conv_multi_item_sizes():
+    h = torch.rand(s, 9, 9, 32, device=dev, generator=g).to(torch.bfloat16)
+    w8 = ((torch.rand(4, 4, 8, 32, device=dev, generator=g) - 0.5) * 0.2).to(torch.bfloat16)     # [kh,kw,out,in]
+    b8 = (torch.rand(8, device=dev, generator=g) - 0.5) * 0.1
+    q = K.pc_deconv_qmax(h, K.pc_deconv_taps(w8), b8, na)
+    y = torch.relu(_conv64(h, w8.permute(3, 2, 0, 1), b8, stride=2, transpose=True))      # [S,20,20,8]: V, A_1..A_7
+    adv = y[..., 1:1 + na]
+    ref = y[..., 0] + adv.max(dim=3).values - adv.mean(dim=3)
+    assert tuple(q.shape) == (s, 20, 20)
+    assert torch.allclose(q.double(), ref, rtol=1e-4, atol=1e-5), (s, float((q.double() - ref).abs().max()))
+    del y, adv, ref
 
 
 def _bf16_close(got, want, ulps=1.0):

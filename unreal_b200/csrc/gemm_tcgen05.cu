@@ -614,7 +614,9 @@ extern "C" int unreal_gemm_bf16(const void* a, int64_t lda, int a_mn_major, cons
                                 void* stream) {
   UNREAL_REQUIRE(a && b && c, "unreal_gemm_bf16: null operand");
   UNREAL_REQUIRE(m > 0 && n > 0 && k > 0, "unreal_gemm_bf16: empty problem %d x %d x %d", m, n, k);
-  UNREAL_REQUIRE(aligned16(a) && aligned16(b) && aligned16(c), "unreal_gemm_bf16: operands must be 16-byte aligned");
+  // the TMA-store epilogue reads the bias as float4
+  UNREAL_REQUIRE(aligned16(a) && aligned16(b) && aligned16(c) && (bias == nullptr || aligned16(bias)),
+                 "unreal_gemm_bf16: operands and bias must be 16-byte aligned");
   UNREAL_REQUIRE((lda & 7) == 0 && (ldb & 7) == 0, "unreal_gemm_bf16: lda/ldb must be multiples of 8 elements (TMA)");
   UNREAL_REQUIRE(lda >= (a_mn_major ? m : k) && ldb >= (b_mn_major ? n : k) && ldc >= n,
                  "unreal_gemm_bf16: leading dimension smaller than the row length");
@@ -642,6 +644,9 @@ extern "C" int unreal_gemm_bf16(const void* a, int64_t lda, int a_mn_major, cons
   }
   { int forced = get_tunable("gemm_bn", 0); if (forced == 32 || forced == 64 || forced == 128 || forced == 256) bn = forced; }
   if (b_mn_major && bn < 64) bn = 64;
+  // a bf16 output row of the TMA-store epilogue is staged and stored 64 columns at a time: a 32-column tile would read
+  // the other accumulator's TMEM columns and store them over the next tile
+  if (c_dtype == UNREAL_GEMM_OUT_BF16 && bn < 64) bn = 64;
   // CTA-pair kernel (256 x 256 tiles) once there is at least one full wave of pairs
   const int64_t work2 = (int64_t)((m + 255) / 256) * ((n + 255) / 256) * split_k;
   // ... and the problem is compute-bound (long K): short-K, output-dominated shapes are paced by the
@@ -677,8 +682,10 @@ extern "C" int unreal_gemm_bf16(const void* a, int64_t lda, int a_mn_major, cons
   else rc = make_tma_2d(&tb, b, n, k, ldb, use_2sm ? bn / 2 : bn, false);   // a CTA of a pair loads half the B rows
   if (rc != UNREAL_OK) return rc;
   const bool c_bf16 = c_dtype == UNREAL_GEMM_OUT_BF16;
-  // TMA epilogue needs a 16-byte row pitch; odd leading dimensions fall back to element stores
-  int tma_store = ((ldc * (c_bf16 ? 2 : 4)) % 16 == 0) && get_tunable("gemm_tma_store", 1) != 0;
+  // TMA epilogue needs a 16-byte row pitch and rows of whole 16-byte chunks: a bf16 C of n = 52 (104-byte rows) inside
+  // a wider buffer had the columns past n written by the TMA store.  Other shapes fall back to element stores.
+  const int c_esize = c_bf16 ? 2 : 4;
+  int tma_store = ((ldc * c_esize) % 16 == 0) && (((int64_t)n * c_esize) % 16 == 0) && get_tunable("gemm_tma_store", 1) != 0;
   if (tma_store) {
     rc = make_tma_2d(&tc, c, m, n, ldc, 32, !c_bf16);
     if (rc != UNREAL_OK) return rc;
