@@ -441,7 +441,8 @@ int unreal_pc_deconv_fwd(const void* h_bf16, const void* w_dtaps_bf16, const flo
  *   sums [3] f64 += (policy loss, value loss, entropy) with act [M] i32, adv, r, mask [M] f32 (mask NULL: all ones):
  *     policy = -sum mask (log pi[a] adv + entropy_beta H), value = value_coef sum mask (r - v)^2, pi clamped to [1e-20,1]
  *   dz [M,A] = d policy / d logits, dv [M] = d value / d v   (consumed by unreal_a3c_head_bwd)
- * act NULL: no policy loss (value replay); r NULL: no value loss; a = 0 / wp NULL: value head only. */
+ * act NULL: no policy loss (value replay); r NULL: no value loss; a = 0 / wp NULL: value head only.
+ * a <= 15 (a <= 7 runs the 8-output build, a = 8..15 the 16-output one; unreal_a3c_head_bwd alike). */
 int unreal_a3c_head_loss(const float* h, const float* wp, const float* bp, const float* wv, const float* bv,
                          const int32_t* act, const float* adv, const float* r, const float* mask, int64_t m, int a,
                          float entropy_beta, float value_coef, float* pi_out, float* v_out, double* sums, float* dz,
@@ -502,6 +503,20 @@ int unreal_pc_planes_wgrad(const void* dy_planes_bf16, const void* hp_bf16, floa
  * and the max over actions in its epilogue -> qmax f32 [S,20,20]; the head output itself is not written. */
 int unreal_pc_deconv_qmax(const void* h_bf16, const void* w_dtaps_bf16, const float* bias8, int a, int s, float* qmax,
                           void* stream);
+/* The 16-channel pixel-control head for 8..15 actions (model.py:411-441 head and dueling combine, :531-546 loss, :707-712
+ * run_pc_q_max): the merged deconv filter [4,4,16,32] holds the value in channel 0 and the advantages in channels 1..a
+ * (the rest zero); w_dtaps bf16 [4 taps, 64 (dy,dx,c), 32] (conv2's transposed-convolution tap layout), bias16 f32 [16].
+ *   unreal_pc_deconv_loss16: h bf16 [S,9,9,32] -> loss (double, accumulated) += lam 0.5 sum mask (R - Q_act)^2,
+ *     dy16 bf16 [S,400,16] = d loss / d (pre-ReLU deconv output), every channel real and not yet multiplied by the upstream
+ *     gradient (unreal_conv2_fwd_linear_masked with c_in 16 and unreal_conv2_wgrad take it), db16 f32 [16] += the
+ *     bias gradient (caller-zeroed, nullable); act [S] i32, target [S,20,20] f32, mask [S] f32.
+ *   unreal_pc_deconv_qmax16: qmax f32 [S,20,20] = max over actions of the dueling combine.
+ * a outside 8..15 is an argument error (a <= 7 is the 8-channel head above). */
+int unreal_pc_deconv_loss16(const void* h_bf16, const void* w_dtaps_bf16, const float* bias16, const int32_t* act,
+                            const float* target, const float* mask, int a, float lam, int s, double* loss, void* dy16_bf16,
+                            float* db16, void* stream);
+int unreal_pc_deconv_qmax16(const void* h_bf16, const void* w_dtaps_bf16, const float* bias16, int a, int s, float* qmax,
+                            void* stream);
 /* Reward-prediction head after its fc GEMM (model.py:482-488 softmax, :571-575 loss).  logits8 [N,8] f32: columns 0..2 =
  * features . W_rp (the bf16 tcgen05 GEMM on the weight shadow padded to 8 columns), bias [3] added here.
  *   p_out (nullable) [N,3] = softmax(logits + bias)                                  (run_rp_c, model.py:723-728)

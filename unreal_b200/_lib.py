@@ -122,6 +122,8 @@ SIGNATURES = {
     "unreal_pc_planes_conv": (c_int, [P, P, P, P, P, P, c_int, P]),
     "unreal_pc_planes_wgrad": (c_int, [P, P, P, c_int, P]),
     "unreal_pc_deconv_qmax": (c_int, [P, P, P, c_int, c_int, P, P]),
+    "unreal_pc_deconv_loss16": (c_int, [P, P, P, P, P, P, c_int, c_float, c_int, P, P, P, P]),
+    "unreal_pc_deconv_qmax16": (c_int, [P, P, P, c_int, c_int, P, P]),
     "unreal_conv2_fwd_linear_scaled": (c_int, [P, P, P, P, c_int, P]),
     "unreal_conv2_fwd_linear_masked": (c_int, [P, c_int, P, P, P, P, P, c_int, P]),
     "unreal_rp_loss": (c_int, [P, P, P, c_int64, P, P, P, P, P, P]),

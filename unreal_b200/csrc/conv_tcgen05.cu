@@ -962,11 +962,14 @@ struct PcLossArgs {
                           // 2: as four parity planes [S][4 (dy,dx)][100 (Y,X)][8] (pc_planes_*_tcgen05_kernel's tile)
 };
 
-// EPI = 8 (CO = 8 only): two epilogue warps per TMEM lane quarter, one per output-row parity dy (16 accumulator columns
-// each).  The loss epilogue is a chain of dependent instructions per pixel on ONE warp per scheduler (ncu of the 4-warp
+// PC (CO = 16 only): the same loss (or the q-max map) for the 16-channel head of 8..15 actions -- channel 0 the value,
+// 1..A the advantages.  The thread holds all 16 channels of its pixels and writes the loss gradient as [S,400,16] with
+// every channel real; the bias gradient is db [16].
+// EPI = 8 (CO = 8, or PC): two epilogue warps per TMEM lane quarter, one per output-row parity dy (16 accumulator columns
+// each; 32 with PC).  The loss epilogue is a chain of dependent instructions per pixel on ONE warp per scheduler (ncu of the 4-warp
 // build, profiles/r2_conv2_bwd_20480samples_ncu_summary.txt: issue slots 39 % active, DRAM 29 %, tensor pipe 7 %, nothing
 // saturated); twice the warps hide twice the latency.
-template <int CO, int EPI = 4, int NA = 0>       // NA: the pixel-control loss's action count when known at compile time (0: run time)
+template <int CO, int EPI = 4, int NA = 0, bool PC = false>   // NA: the pixel-control loss's action count when known at compile time (0: run time)
 __global__ void __launch_bounds__(64 + 32 * EPI, 2)
 conv2_dgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_w,
                            void* __restrict__ out_raw, const float* __restrict__ bias, int samples,
@@ -985,6 +988,8 @@ conv2_dgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __gr
   auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * kDgStages + kDgAcc + a); };
   const uint32_t w_bar = bar_base + 8u * (2 * kDgStages + 2 * kDgAcc);
   const uint32_t tmem_slot = w_bar + 8u;
+  // PC: the 16 bias values in the barrier block's spare bytes (in registers they push the EPI = 8 epilogue into spills)
+  float* s_bias = reinterpret_cast<float*>(smem_raw + (bar_base + 512u - smem_u32(smem_raw)));
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (warp == 0 && lane == 0) {
     prefetch_tensormap(&tma_a); prefetch_tensormap(&tma_w);
@@ -994,6 +999,8 @@ conv2_dgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __gr
     fence_mbar_init();
   } else if (warp == 2) {
     tmem_alloc<kDgAcc * 64>(tmem_slot);
+  } else if (PC && warp == 3 && lane < 16) {
+    s_bias[lane] = __ldg(bias + lane);
   }
   fence_before_sync();
   __syncthreads();
@@ -1058,14 +1065,15 @@ conv2_dgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __gr
     float dbacc[16];
 #pragma unroll
     for (int c = 0; c < 16; ++c) dbacc[c] = 0.f;
+    const float* b16 = s_bias;
     float loss_part = 0.f;
-    constexpr int kDyPre = (CO == 8 && EPI == 8) ? 1 : 2;
+    constexpr int kDyPre = ((CO == 8 || PC) && EPI == 8) ? 1 : 2;
     float2 tg_next[kDyPre];
     float m_next = 0.f;
     int a_next = 0;
 #pragma unroll
     for (int d = 0; d < kDyPre; ++d) tg_next[d] = make_float2(0.f, 0.f);
-    if (CO == 8 && pl.target != nullptr && r < 100 && (int)blockIdx.x < samples) {
+    if ((CO == 8 || PC) && pl.target != nullptr && r < 100 && (int)blockIdx.x < samples) {
       const int dyb = EPI == 8 ? ((warp - 2) >> 2) : 0;
       m_next = __ldg(pl.mask + blockIdx.x);
       a_next = __ldg(pl.act + blockIdx.x);
@@ -1209,6 +1217,98 @@ conv2_dgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __gr
         if (++acc == kDgAcc) { acc = 0; acc_phase ^= 1u; }
         continue;
       }
+      if constexpr (PC) {
+        // column (dy, dx, c) = dy*32 + dx*16 + c.  EPI = 4: both parities; EPI = 8: this warp's parity only
+        constexpr int kDy = EPI == 8 ? 1 : 2;
+        const int dy_base = EPI == 8 ? ((warp - 2) >> 2) : 0;
+        uint32_t v[kDy][32];
+#pragma unroll
+        for (int d = 0; d < kDy; ++d) tmem_ld32(taddr + (uint32_t)(32 * (dy_base + d)), v[d]);
+        tmem_ld_wait();
+        fence_before_sync();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(tempty_bar(acc));
+        const float inv_a = 1.0f / (float)pl.a;
+        if (pl.qmax != nullptr) {
+          if (r < 100) {
+#pragma unroll
+            for (int d = 0; d < kDy; ++d) {
+              float q2[2];
+#pragma unroll
+              for (int dx = 0; dx < 2; ++dx) {
+                const uint32_t* vv = v[d] + dx * 16;
+                float sum = 0.f, best = -3.4e38f;
+#pragma unroll
+                for (int k = 0; k < 15; ++k) {
+                  if (k < pl.a) {
+                    const float y = fmaxf(__uint_as_float(vv[1 + k]) + b16[1 + k], 0.f);
+                    sum += y; best = fmaxf(best, y);
+                  }
+                }
+                q2[dx] = fmaxf(__uint_as_float(vv[0]) + b16[0], 0.f) + best - sum * inv_a;
+              }
+              *reinterpret_cast<float2*>(pl.qmax + ((int64_t)it * 20 + 2 * Y + dy_base + d) * 20 + 2 * X) = make_float2(q2[0], q2[1]);
+            }
+          }
+          if (++acc == kDgAcc) { acc = 0; acc_phase ^= 1u; }
+          continue;
+        }
+        float2 tgs[kDy];
+#pragma unroll
+        for (int d = 0; d < kDy; ++d) tgs[d] = tg_next[d];
+        const float m = m_next;
+        const int a = a_next;
+        if (r < 100 && it + (int)gridDim.x < samples) {
+          const int nx = it + (int)gridDim.x;
+          m_next = __ldg(pl.mask + nx);
+          a_next = __ldg(pl.act + nx);
+#pragma unroll
+          for (int d = 0; d < kDy; ++d)
+            tg_next[d] = __ldcs(reinterpret_cast<const float2*>(pl.target + ((int64_t)nx * 20 + 2 * Y + dy_base + d) * 20 + 2 * X));
+        }
+        if (r < 100) {
+          uint4* out16 = reinterpret_cast<uint4*>(out_raw);
+#pragma unroll
+          for (int d = 0; d < kDy; ++d) {
+            const int64_t pix = ((int64_t)it * 20 + 2 * Y + dy_base + d) * 20 + 2 * X;
+#pragma unroll
+            for (int dx = 0; dx < 2; ++dx) {
+              const uint32_t* vv = v[d] + dx * 16;
+              float y[16];
+#pragma unroll
+              for (int c = 0; c < 16; ++c) y[c] = fmaxf(__uint_as_float(vv[c]) + b16[c], 0.f);
+              float sum = 0.f, qa = 0.f;
+#pragma unroll
+              for (int k = 0; k < 15; ++k) {
+                if (k < pl.a) { sum += y[1 + k]; if (k == a) qa = y[1 + k]; }
+              }
+              qa = y[0] + qa - sum * inv_a;
+              const float diff = qa - (dx ? tgs[d].y : tgs[d].x);
+              loss_part += m * diff * diff;
+              const float g = pl.lam * m * diff;
+              uint32_t pk[8];
+#pragma unroll
+              for (int j = 0; j < 8; ++j) {
+                float dd[2];
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                  const int c = 2 * j + e, k = c - 1;
+                  dd[e] = c == 0 ? (y[0] > 0.f ? g : 0.f)
+                                 : ((k < pl.a && y[c] > 0.f) ? g * ((k == a ? 1.f : 0.f) - inv_a) : 0.f);
+                }
+                __nv_bfloat162 p = __floats2bfloat162_rn(dd[0], dd[1]);
+                pk[j] = *reinterpret_cast<uint32_t*>(&p);
+                const float2 f = __bfloat1622float2(p);      // the bias gradient sums the ROUNDED values
+                dbacc[2 * j] += f.x; dbacc[2 * j + 1] += f.y;
+              }
+              __stcs(out16 + pix * 2 + 2 * dx, make_uint4(pk[0], pk[1], pk[2], pk[3]));
+              __stcs(out16 + pix * 2 + 2 * dx + 1, make_uint4(pk[4], pk[5], pk[6], pk[7]));
+            }
+          }
+        }
+        if (++acc == kDgAcc) { acc = 0; acc_phase ^= 1u; }
+        continue;
+      }
       __nv_bfloat16* out = reinterpret_cast<__nv_bfloat16*>(out_raw);
       uint32_t v0[32], v1[32];
       tmem_ld32(taddr, v0);            // dy = 0: (dx, c) = 32 values = pixels (2Y, 2X) and (2Y, 2X+1)
@@ -1287,10 +1387,10 @@ conv2_dgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __gr
         if (lane == 0) atomicAdd(db + c, x);
       }
     }
-    if (CO == 8 && pl.target != nullptr) {
+    if ((CO == 8 || PC) && pl.target != nullptr) {
       if (db != nullptr) {
 #pragma unroll
-        for (int c = 0; c < 8; ++c) {
+        for (int c = 0; c < (PC ? 16 : 8); ++c) {
           float x = dbacc[c];
 #pragma unroll
           for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
@@ -1903,7 +2003,7 @@ extern "C" int unreal_conv2_wgrad_c8(const void* x8_bf16, const void* dy_bf16, f
   return conv2_wgrad_launch<8>(x8_bf16, dy_bf16, dw_taps, s, stream);
 }
 
-template <int CO, int EPI = 4, int NA = 0>
+template <int CO, int EPI = 4, int NA = 0, bool PC = false>
 static int launch_deconv(const void* dy_bf16, const void* w_dtaps_bf16, void* out, const float* bias, int s, void* stream,
                          const void* mask_y = nullptr, float* db = nullptr, int pitch21 = 0,
                          PcLossArgs pl = PcLossArgs{nullptr, nullptr, nullptr, nullptr, 0, 0.f, nullptr, 0}) {
@@ -1924,12 +2024,12 @@ static int launch_deconv(const void* dy_bf16, const void* w_dtaps_bf16, void* ou
   }
   static bool configured = false;
   if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(conv2_dgrad_tcgen05_kernel<CO, EPI, NA>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDgSmem));
+    UNREAL_CUDA(cudaFuncSetAttribute(conv2_dgrad_tcgen05_kernel<CO, EPI, NA, PC>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDgSmem));
     configured = true;
   }
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
-  conv2_dgrad_tcgen05_kernel<CO, EPI, NA><<<s < 2 * sms ? s : 2 * sms, 64 + 32 * EPI, kDgSmem, as_stream(stream)>>>(
+  conv2_dgrad_tcgen05_kernel<CO, EPI, NA, PC><<<s < 2 * sms ? s : 2 * sms, 64 + 32 * EPI, kDgSmem, as_stream(stream)>>>(
       ta, tw, out, bias, s, reinterpret_cast<const __nv_bfloat16*>(mask_y), db, pitch21, pl);
   UNREAL_LAUNCH_CHECK("conv2_dgrad_tcgen05_kernel");
   return UNREAL_OK;
@@ -2042,4 +2142,29 @@ extern "C" int unreal_pc_deconv_qmax(const void* h_bf16, const void* w_dtaps_bf1
   UNREAL_REQUIRE(aligned16(h_bf16) && aligned16(w_dtaps_bf16) && aligned16(qmax), "unreal_pc_deconv_qmax: 16-byte alignment");
   return launch_deconv<8>(h_bf16, w_dtaps_bf16, qmax, bias8, s, stream, nullptr, nullptr, 0,
                           PcLossArgs{nullptr, nullptr, nullptr, nullptr, a, 0.f, qmax, 0});
+}
+
+// The 16-channel pixel-control head (8..15 actions): channel 0 the value, 1..A the advantages, no padding channel in the
+// loss gradient, which goes to conv2's own backward kernels (unreal_conv2_fwd_linear_masked with c_in 16, unreal_conv2_wgrad).
+constexpr int kPc16Epi = 8;
+
+extern "C" int unreal_pc_deconv_loss16(const void* h_bf16, const void* w_dtaps_bf16, const float* bias16, const int32_t* act,
+                                       const float* target, const float* mask, int a, float lam, int s, double* loss,
+                                       void* dy16_bf16, float* db16, void* stream) {
+  UNREAL_REQUIRE(h_bf16 && w_dtaps_bf16 && bias16 && act && target && mask && dy16_bf16 && s > 0,
+                 "unreal_pc_deconv_loss16: null buffer or s <= 0");
+  UNREAL_REQUIRE(a >= 8 && a <= 15, "unreal_pc_deconv_loss16: action count %d not in 8..15 (16-channel head)", a);
+  UNREAL_REQUIRE(aligned16(h_bf16) && aligned16(w_dtaps_bf16) && aligned16(dy16_bf16) && aligned16(target),
+                 "unreal_pc_deconv_loss16: 16-byte alignment");
+  return launch_deconv<16, kPc16Epi, 0, true>(h_bf16, w_dtaps_bf16, dy16_bf16, bias16, s, stream, nullptr, db16, 0,
+                                              PcLossArgs{act, target, mask, loss, a, lam, nullptr, 0});
+}
+
+extern "C" int unreal_pc_deconv_qmax16(const void* h_bf16, const void* w_dtaps_bf16, const float* bias16, int a, int s,
+                                       float* qmax, void* stream) {
+  UNREAL_REQUIRE(h_bf16 && w_dtaps_bf16 && bias16 && qmax && s > 0, "unreal_pc_deconv_qmax16: null buffer or s <= 0");
+  UNREAL_REQUIRE(a >= 8 && a <= 15, "unreal_pc_deconv_qmax16: action count %d not in 8..15 (16-channel head)", a);
+  UNREAL_REQUIRE(aligned16(h_bf16) && aligned16(w_dtaps_bf16) && aligned16(qmax), "unreal_pc_deconv_qmax16: 16-byte alignment");
+  return launch_deconv<16, kPc16Epi, 0, true>(h_bf16, w_dtaps_bf16, qmax, bias16, s, stream, nullptr, nullptr, 0,
+                                              PcLossArgs{nullptr, nullptr, nullptr, nullptr, a, 0.f, qmax, 0});
 }

@@ -477,10 +477,14 @@ __global__ void __launch_bounds__(256) pc_loss_kernel(const float* __restrict__ 
 //   value  = coef * sum mask * (R - v)^2        (coef 0.25 base :527, 0.5 value replay :565)
 // The same pass writes d policy / d logits (dz) and d value / d v (dv) for the backward kernel:
 //   dz_j = mask * (-adv * ([j == a] - pi_j) + beta * pi_j * (log pi_j + H)),   dv = -2 coef mask (R - v).
+// The loss and backward kernels are built for up to MAXA = 7 actions (8 outputs, four lanes each) and 15 (16 outputs, two
+// lanes each); a launch takes the narrowest build that holds A.
 constexpr int kHeadMaxA = 7;
+constexpr int kHeadMaxAWide = 15;
 
+template <int MAXA>
 struct HeadW {
-  float wp[8][kHeadMaxA];
+  float wp[8][MAXA];
   float wv[8];
 };
 
@@ -488,20 +492,21 @@ struct HeadW {
 // eight rows k = lane + 32 i into registers.  (Every warp used to fetch its 64 weights with scalar global loads of
 // stride A: at acting batch sizes -- one or two rows of work per warp -- that set-up WAS the kernel, 21 us for an
 // 8 MB read.)  Block size 256.
-__device__ __forceinline__ void head_load_w(HeadW& w, const float* __restrict__ Wp, const float* __restrict__ Wv, int A,
+template <int MAXA>
+__device__ __forceinline__ void head_load_w(HeadW<MAXA>& w, const float* __restrict__ Wp, const float* __restrict__ Wv, int A,
                                             int lane, float* s_w) {
   for (int i = threadIdx.x; i < 256 * A; i += blockDim.x) {
     const int k = i / A, j = i - k * A;
     s_w[j * 256 + k] = Wp[i];
   }
-  for (int k = threadIdx.x; k < 256; k += blockDim.x) s_w[kHeadMaxA * 256 + k] = Wv ? Wv[k] : 0.f;
+  for (int k = threadIdx.x; k < 256; k += blockDim.x) s_w[MAXA * 256 + k] = Wv ? Wv[k] : 0.f;
   __syncthreads();
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     const int k = lane + 32 * i;
 #pragma unroll
-    for (int j = 0; j < kHeadMaxA; ++j) w.wp[i][j] = (j < A) ? s_w[j * 256 + k] : 0.f;
-    w.wv[i] = s_w[kHeadMaxA * 256 + k];
+    for (int j = 0; j < MAXA; ++j) w.wp[i][j] = (j < A) ? s_w[j * 256 + k] : 0.f;
+    w.wv[i] = s_w[MAXA * 256 + k];
   }
 }
 
@@ -511,49 +516,58 @@ __device__ __forceinline__ float warp_sum(float x) {
   return x;
 }
 
-// One row of the heads on one warp.  x[i] = h[r, lane + 32 i].  The eight dot products (7 policy logits + the value) are
-// reduced with a TRANSPOSING butterfly: at distance 16 a lane keeps four of its eight partial sums and trades the other
-// four, at distance 8 two of four, at distance 4 one of two, then two plain steps -- 9 shuffles instead of 40, and
-// lane L ends up holding output j = L >> 2.  Softmax, entropy and log-likelihood then run ACROSS the lanes (three
-// shuffles each at distances 4, 8, 16), each output's exp / log computed once.
-struct HeadRow {
-  float p, lp, H, v, z;      // this lane's (j = lane >> 2) probability and clamped log; entropy and value in every lane
+// One row of the heads on one warp.  x[i] = h[r, lane + 32 i].  The MAXA + 1 dot products (policy logits + the value) are
+// reduced with a TRANSPOSING butterfly.  MAXA = 7: at distance 16 a lane keeps four of its eight partial sums and trades
+// the other four, at distance 8 two of four, at distance 4 one of two, then two plain steps -- 9 shuffles instead of 40,
+// and lane L ends up holding output j = L >> 2.  MAXA = 15: 16 partial sums halve at distances 16, 8, 4 and 2, then one
+// plain step, and lane L holds output j = L >> 1.  Softmax, entropy and log-likelihood then run ACROSS the lanes (one
+// shuffle per remaining distance), each output's exp / log computed once.
+template <int MAXA> struct HeadLanes {
+  static constexpr int kOut = MAXA + 1;                 // outputs per warp
+  static constexpr int kPer = 32 / kOut;                // lanes per output (4 or 2)
+  static constexpr int kShift = kPer == 4 ? 2 : 1;
+  static_assert(kOut * kPer == 32 && (kPer == 4 || kPer == 2), "head builds: 8 or 16 outputs per warp");
 };
-__device__ __forceinline__ HeadRow head_row(const HeadW& w, const float (&x)[8], int lane, int A, float bias_j) {
-  float z[kHeadMaxA + 1];
+struct HeadRow {
+  float p, lp, H, v, z;      // this lane's (j = lane / lanes per output) probability and clamped log; entropy and value in every lane
+};
+template <int MAXA>
+__device__ __forceinline__ HeadRow head_row(const HeadW<MAXA>& w, const float (&x)[8], int lane, int A, float bias_j) {
+  using L = HeadLanes<MAXA>;
+  float z[L::kOut];
 #pragma unroll
-  for (int j = 0; j <= kHeadMaxA; ++j) z[j] = 0.f;
+  for (int j = 0; j < L::kOut; ++j) z[j] = 0.f;
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
 #pragma unroll
-    for (int j = 0; j < kHeadMaxA; ++j) z[j] = fmaf(x[i], w.wp[i][j], z[j]);
-    z[kHeadMaxA] = fmaf(x[i], w.wv[i], z[kHeadMaxA]);
+    for (int j = 0; j < MAXA; ++j) z[j] = fmaf(x[i], w.wp[i][j], z[j]);
+    z[MAXA] = fmaf(x[i], w.wv[i], z[MAXA]);
   }
-  const bool b4 = lane & 16, b3 = lane & 8, b2 = lane & 4;
-  float u[4], t2[2];
 #pragma unroll
-  for (int t = 0; t < 4; ++t) u[t] = (b4 ? z[4 + t] : z[t]) + __shfl_xor_sync(0xffffffffu, b4 ? z[t] : z[4 + t], 16);
+  for (int n = L::kOut / 2, d = 16; d >= L::kPer; n >>= 1, d >>= 1) {
+    const bool hi = lane & d;
 #pragma unroll
-  for (int t = 0; t < 2; ++t) t2[t] = (b3 ? u[2 + t] : u[t]) + __shfl_xor_sync(0xffffffffu, b3 ? u[t] : u[2 + t], 8);
-  float s = (b2 ? t2[1] : t2[0]) + __shfl_xor_sync(0xffffffffu, b2 ? t2[0] : t2[1], 4);
-  s += __shfl_xor_sync(0xffffffffu, s, 2);
-  s += __shfl_xor_sync(0xffffffffu, s, 1);
-  const int j = lane >> 2;
+    for (int t = 0; t < n; ++t) z[t] = (hi ? z[n + t] : z[t]) + __shfl_xor_sync(0xffffffffu, hi ? z[t] : z[n + t], d);
+  }
+  float s = z[0];
+#pragma unroll
+  for (int d = L::kPer / 2; d >= 1; d >>= 1) s += __shfl_xor_sync(0xffffffffu, s, d);
+  const int j = lane >> L::kShift;
   HeadRow o;
   o.z = s + bias_j;
-  o.v = __shfl_sync(0xffffffffu, o.z, 4 * kHeadMaxA);
+  o.v = __shfl_sync(0xffffffffu, o.z, L::kPer * MAXA);
   float mx = (j < A) ? o.z : -3.0e38f;
 #pragma unroll
-  for (int d = 4; d <= 16; d <<= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, d));
+  for (int d = L::kPer; d <= 16; d <<= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, d));
   const float e = (j < A) ? __expf(o.z - mx) : 0.f;
   float den = e;
 #pragma unroll
-  for (int d = 4; d <= 16; d <<= 1) den += __shfl_xor_sync(0xffffffffu, den, d);
+  for (int d = L::kPer; d <= 16; d <<= 1) den += __shfl_xor_sync(0xffffffffu, den, d);
   o.p = e * (1.0f / den);
   o.lp = __logf(fminf(fmaxf(o.p, 1e-20f), 1.0f));
   float H = (j < A) ? -o.p * o.lp : 0.f;
 #pragma unroll
-  for (int d = 4; d <= 16; d <<= 1) H += __shfl_xor_sync(0xffffffffu, H, d);
+  for (int d = L::kPer; d <= 16; d <<= 1) H += __shfl_xor_sync(0xffffffffu, H, d);
   o.H = H;
   return o;
 }
@@ -621,6 +635,7 @@ __global__ void __launch_bounds__(256) lstm_cell_act_heads8_kernel(const __nv_bf
   }
 }
 
+template <int MAXA>
 __global__ void __launch_bounds__(256) a3c_head_loss_kernel(const float* __restrict__ h, const float* __restrict__ Wp,
                                                             const float* __restrict__ bp, const float* __restrict__ Wv,
                                                             const float* __restrict__ bv, const int32_t* __restrict__ act,
@@ -632,13 +647,15 @@ __global__ void __launch_bounds__(256) a3c_head_loss_kernel(const float* __restr
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-  __shared__ float s_w[(kHeadMaxA + 1) * 256];
-  HeadW w;
+  using L = HeadLanes<MAXA>;
+  constexpr int kVLane = L::kPer * MAXA;               // the lane that holds the value
+  __shared__ float s_w[(MAXA + 1) * 256];
+  HeadW<MAXA> w;
   head_load_w(w, Wp, Wv, A, lane, s_w);
-  const int j = lane >> 2;
-  const bool writer = (lane & 3) == 0;                 // one lane per output
-  const float bias_j = (j < A) ? bp[j] : ((j == kHeadMaxA && bv) ? bv[0] : 0.f);
-  float s_pol = 0.f, s_val = 0.f, s_ent = 0.f;         // lane 0 (policy, entropy) and lane 28 (value) accumulate
+  const int j = lane >> L::kShift;
+  const bool writer = (lane & (L::kPer - 1)) == 0;     // one lane per output
+  const float bias_j = (j < A) ? bp[j] : ((j == MAXA && bv) ? bv[0] : 0.f);
+  float s_pol = 0.f, s_val = 0.f, s_ent = 0.f;         // lane 0 (policy, entropy) and lane kVLane (value) accumulate
   // two rows per iteration: both rows' loads are in flight before either row's arithmetic starts
   for (int64_t r0 = 2 * warp0; r0 < M; r0 += 2 * nwarps) {
     const int nrow = (r0 + 1 < M) ? 2 : 1;
@@ -651,19 +668,19 @@ __global__ void __launch_bounds__(256) a3c_head_loss_kernel(const float* __restr
     for (int q = 0; q < 2; ++q) {
       if (q >= nrow) break;
       const int64_t r = r0 + q;
-      const HeadRow o = head_row(w, x[q], lane, A, bias_j);
+      const HeadRow o = head_row<MAXA>(w, x[q], lane, A, bias_j);
       const float m = mask ? mask[r] : 1.f;
       if (writer && j < A && pi_out) pi_out[r * A + j] = o.p;
-      if (lane == 4 * kHeadMaxA && v_out) v_out[r] = o.v;
+      if (lane == kVLane && v_out) v_out[r] = o.v;
       if (act != nullptr) {
         const int a = act[r];
         const float ad = adv[r];
-        const float lpa_any = __shfl_sync(0xffffffffu, o.lp, (4 * a) & 31);
+        const float lpa_any = __shfl_sync(0xffffffffu, o.lp, (L::kPer * a) & 31);
         const float lpa = (a >= 0 && a < A) ? lpa_any : 0.f;
         if (lane == 0) { s_pol -= m * (lpa * ad + beta * o.H); s_ent += m * o.H; }
         if (writer && j < A && dz) dz[r * A + j] = m * (-ad * ((j == a ? 1.f : 0.f) - o.p) + beta * o.p * (o.lp + o.H));
       }
-      if (R != nullptr && lane == 4 * kHeadMaxA) {
+      if (R != nullptr && lane == kVLane) {
         const float d = R[r] - o.v;
         s_val += coef * m * d * d;
         if (dv) dv[r] = -2.f * coef * m * d;
@@ -673,7 +690,7 @@ __global__ void __launch_bounds__(256) a3c_head_loss_kernel(const float* __restr
   if (sums == nullptr) return;
   __shared__ float sp[8][3];
   if (lane == 0) { sp[threadIdx.x >> 5][0] = s_pol; sp[threadIdx.x >> 5][2] = s_ent; }
-  if (lane == 4 * kHeadMaxA) sp[threadIdx.x >> 5][1] = s_val;
+  if (lane == kVLane) sp[threadIdx.x >> 5][1] = s_val;
   __syncthreads();
   if (threadIdx.x < 3) {
     double t = 0.0;
@@ -684,42 +701,46 @@ __global__ void __launch_bounds__(256) a3c_head_loss_kernel(const float* __restr
 
 // dh = go_p * dz Wp^T + go_v * dv Wv^T;  dWp += go_p * h^T dz;  dbp += go_p * sum dz;  dWv += go_v * h^T dv;  dbv += ...
 // One thread per COLUMN k of h (256 per CTA), CTAs stride over chunks of 32 rows whose upstream gradients
-// g[row][0..A) = go_p dz, g[row][7] = go_v dv are staged in shared memory: per row a thread reads h[r,k], writes dh[r,k]
-// (both coalesced) and does 16 FMAs against 8 broadcast values -- ~40 registers, so the SM holds 32+ warps and the
+// g[row][0..A) = go_p dz, g[row][MAXA] = go_v dv are staged in shared memory: per row a thread reads h[r,k], writes dh[r,k]
+// (both coalesced) and does 16 FMAs against 8 broadcast values (32 against 16 in the 15-action build) -- ~40 registers, so the SM holds 32+ warps and the
 // row-to-row load latency is hidden by other warps.  (The first form -- one warp per row, 64 weight + 64 accumulator
 // registers per lane, 16 warps per SM, each row's loads waited for in turn -- ran at 244 us for 163 840 rows: 1.4 TB/s.)
 constexpr int kHeadBwdRows = 32;
+template <int MAXA>
 __global__ void __launch_bounds__(256) a3c_head_bwd_kernel(const float* __restrict__ h, const float* __restrict__ Wp,
                                                            const float* __restrict__ Wv, const float* __restrict__ dz,
                                                            const float* __restrict__ dv, const float* __restrict__ go,
                                                            int64_t M, int A, float* __restrict__ dh, float* __restrict__ dWp,
                                                            float* __restrict__ dbp, float* __restrict__ dWv,
                                                            float* __restrict__ dbv) {
-  __shared__ __align__(16) float s_g[2][kHeadBwdRows][kHeadMaxA + 1];
-  __shared__ float s_b[kHeadMaxA + 1];
+  constexpr int kOut = MAXA + 1;
+  constexpr int kStageRows = 256 / kOut;               // chunk rows one pass of the 256 threads stages
+  __shared__ __align__(16) float s_g[2][kHeadBwdRows][kOut];
+  __shared__ float s_b[kOut];
   const int k = threadIdx.x;
   const float gp = dz ? go[0] : 0.f, gv = dv ? go[1] : 0.f;
-  float w[kHeadMaxA + 1], acc[kHeadMaxA + 1];
+  float w[kOut], acc[kOut];
 #pragma unroll
-  for (int j = 0; j < kHeadMaxA; ++j) { w[j] = (dz && j < A) ? Wp[k * A + j] : 0.f; acc[j] = 0.f; }
-  w[kHeadMaxA] = (dv && Wv) ? Wv[k] : 0.f;
-  acc[kHeadMaxA] = 0.f;
-  if (k <= kHeadMaxA) s_b[k] = 0.f;
-  // staging role of this thread: row k / 8 of a chunk, component k % 8
-  const int srow = k >> 3, sj = k & 7;
+  for (int j = 0; j < MAXA; ++j) { w[j] = (dz && j < A) ? Wp[k * A + j] : 0.f; acc[j] = 0.f; }
+  w[MAXA] = (dv && Wv) ? Wv[k] : 0.f;
+  acc[MAXA] = 0.f;
+  if (k <= MAXA) s_b[k] = 0.f;
+  // staging role of this thread: rows k / kOut (+ kStageRows) of a chunk, component k % kOut
+  const int srow = k / kOut, sj = k % kOut;
   float bsum = 0.f;
   const int64_t chunks = (M + kHeadBwdRows - 1) / kHeadBwdRows;
   int buf = 0;
   for (int64_t c = blockIdx.x; c < chunks; c += gridDim.x, buf ^= 1) {
     const int64_t r0 = c * kHeadBwdRows;
-    {
-      const int64_t r = r0 + srow;
+#pragma unroll
+    for (int p = 0; p < kHeadBwdRows / kStageRows; ++p) {
+      const int64_t r = r0 + srow + p * kStageRows;
       float g = 0.f;
       if (r < M) {
-        if (sj < kHeadMaxA) { if (dz && sj < A) g = gp * dz[r * A + sj]; }
+        if (sj < MAXA) { if (dz && sj < A) g = gp * dz[r * A + sj]; }
         else if (dv) g = gv * dv[r];
       }
-      s_g[buf][srow][sj] = g;
+      s_g[buf][srow + p * kStageRows][sj] = g;
       bsum += g;
     }
     __syncthreads();            // one barrier per chunk: the other buffer is rewritten only after the next one
@@ -729,22 +750,25 @@ __global__ void __launch_bounds__(256) a3c_head_bwd_kernel(const float* __restri
 #pragma unroll 8
     for (int i = 0; i < rows; ++i) {
       const float x = hp[(int64_t)i * 256];
-      const float4 g0 = *reinterpret_cast<const float4*>(&s_g[buf][i][0]);
-      const float4 g1 = *reinterpret_cast<const float4*>(&s_g[buf][i][4]);
-      const float g[8] = {g0.x, g0.y, g0.z, g0.w, g1.x, g1.y, g1.z, g1.w};
+      float g[kOut];
+#pragma unroll
+      for (int q = 0; q < kOut / 4; ++q) {
+        const float4 g4 = *reinterpret_cast<const float4*>(&s_g[buf][i][4 * q]);
+        g[4 * q] = g4.x; g[4 * q + 1] = g4.y; g[4 * q + 2] = g4.z; g[4 * q + 3] = g4.w;
+      }
       float d = 0.f;
 #pragma unroll
-      for (int j = 0; j <= kHeadMaxA; ++j) { d = fmaf(g[j], w[j], d); acc[j] = fmaf(x, g[j], acc[j]); }
+      for (int j = 0; j < kOut; ++j) { d = fmaf(g[j], w[j], d); acc[j] = fmaf(x, g[j], acc[j]); }
       dp[(int64_t)i * 256] = d;
     }
   }
   atomicAdd(&s_b[sj], bsum);
   __syncthreads();
 #pragma unroll
-  for (int j = 0; j < kHeadMaxA; ++j) if (j < A && dWp) atomicAdd(dWp + k * A + j, acc[j]);
-  if (dWv) atomicAdd(dWv + k, acc[kHeadMaxA]);
+  for (int j = 0; j < MAXA; ++j) if (j < A && dWp) atomicAdd(dWp + k * A + j, acc[j]);
+  if (dWv) atomicAdd(dWv + k, acc[MAXA]);
   if (k < A && dbp) atomicAdd(dbp + k, s_b[k]);
-  if (k == kHeadMaxA && dbv) atomicAdd(dbv, s_b[kHeadMaxA]);
+  if (k == MAXA && dbv) atomicAdd(dbv, s_b[MAXA]);
 }
 
 // col2im for f32 columns with C a multiple of 4 (the merged, padded deconv: C = 8): float4 per tap
@@ -1101,16 +1125,20 @@ extern "C" int unreal_a3c_head_loss(const float* h, const float* wp, const float
                                     int a, float entropy_beta, float value_coef, float* pi_out, float* v_out,
                                     double* sums, float* dz, float* dv, void* stream) {
   UNREAL_REQUIRE(h && m > 0, "unreal_a3c_head_loss: null h or m <= 0");
-  UNREAL_REQUIRE(a >= 0 && a <= kHeadMaxA, "unreal_a3c_head_loss: action count %d not in 0..7", a);
-  UNREAL_REQUIRE(a == 0 || (wp && bp), "unreal_a3c_head_loss: policy weights missing");
+  UNREAL_REQUIRE(a >= 0 && a <= kHeadMaxAWide, "unreal_a3c_head_loss: action count %d not in 0..15", a);
+  UNREAL_REQUIRE(a == 0 || (wp && bp), "unreal_a3c_head_loss: policy weights missing for action count %d", a);
   UNREAL_REQUIRE(act == nullptr || (adv != nullptr && a > 0), "unreal_a3c_head_loss: act needs adv and the policy head");
   UNREAL_REQUIRE(r == nullptr || wv != nullptr, "unreal_a3c_head_loss: returns need the value head");
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   int64_t want = (m + 15) / 16;       // a warp takes two rows per iteration
   const int grid = (int)(want < (int64_t)sms * 4 ? want : (int64_t)sms * 4);
-  a3c_head_loss_kernel<<<grid, 256, 0, as_stream(stream)>>>(h, wp, bp, wv, bv, act, adv, r, mask, m, a, entropy_beta, value_coef,
-                                                           pi_out, v_out, sums, dz, dv);
+  if (a <= kHeadMaxA)
+    a3c_head_loss_kernel<kHeadMaxA><<<grid, 256, 0, as_stream(stream)>>>(h, wp, bp, wv, bv, act, adv, r, mask, m, a, entropy_beta,
+                                                                         value_coef, pi_out, v_out, sums, dz, dv);
+  else
+    a3c_head_loss_kernel<kHeadMaxAWide><<<grid, 256, 0, as_stream(stream)>>>(h, wp, bp, wv, bv, act, adv, r, mask, m, a,
+                                                                             entropy_beta, value_coef, pi_out, v_out, sums, dz, dv);
   UNREAL_LAUNCH_CHECK("a3c_head_loss_kernel");
   return UNREAL_OK;
 }
@@ -1119,14 +1147,17 @@ extern "C" int unreal_a3c_head_bwd(const float* h, const float* wp, const float*
                                    const float* go2, int64_t m, int a, float* dh, float* dwp, float* dbp, float* dwv,
                                    float* dbv, void* stream) {
   UNREAL_REQUIRE(h && go2 && dh && m > 0, "unreal_a3c_head_bwd: null buffer or m <= 0");
-  UNREAL_REQUIRE(a >= 0 && a <= kHeadMaxA, "unreal_a3c_head_bwd: action count %d not in 0..7", a);
+  UNREAL_REQUIRE(a >= 0 && a <= kHeadMaxAWide, "unreal_a3c_head_bwd: action count %d not in 0..15", a);
   UNREAL_REQUIRE(dz == nullptr || (wp && a > 0), "unreal_a3c_head_bwd: dz needs the policy weights");
   UNREAL_REQUIRE(dv == nullptr || wv, "unreal_a3c_head_bwd: dv needs the value weights");
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   int64_t want = (m + kHeadBwdRows - 1) / kHeadBwdRows;
   const int grid = (int)(want < (int64_t)sms * 4 ? want : (int64_t)sms * 4);
-  a3c_head_bwd_kernel<<<grid, 256, 0, as_stream(stream)>>>(h, wp, wv, dz, dv, go2, m, a, dh, dwp, dbp, dwv, dbv);
+  if (a <= kHeadMaxA)
+    a3c_head_bwd_kernel<kHeadMaxA><<<grid, 256, 0, as_stream(stream)>>>(h, wp, wv, dz, dv, go2, m, a, dh, dwp, dbp, dwv, dbv);
+  else
+    a3c_head_bwd_kernel<kHeadMaxAWide><<<grid, 256, 0, as_stream(stream)>>>(h, wp, wv, dz, dv, go2, m, a, dh, dwp, dbp, dwv, dbv);
   UNREAL_LAUNCH_CHECK("a3c_head_bwd_kernel");
   return UNREAL_OK;
 }

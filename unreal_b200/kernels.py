@@ -865,12 +865,22 @@ def conv2_fwd_linear(x, w_taps, out=None, scale=None, mask_y=None, want_db=True)
   return out
 
 
+def _pc16(w_dtaps, bias):
+  """True for the 16-channel head (8..15 actions): a [16] bias or [4,64,32] deconv taps (conv2_dgrad_taps of [4,4,16,32])."""
+  wide = bias.numel() == 16 or tuple(w_dtaps.shape) == (4, 64, 32)
+  if wide and not (bias.numel() == 16 and w_dtaps.numel() == 4 * 64 * 32):
+    raise _lib.UnrealError("the 16-channel pixel-control head needs a [16] bias and [4,64,32] deconv taps")
+  return wide
+
+
 def pc_deconv_qmax(h16, w_dtaps, bias8, num_actions, out=None):
-  """max over actions of the pixel-control Q map, straight from the deconv's epilogue: h16 bf16 [S,9,9,32] -> f32 [S,20,20]."""
+  """max over actions of the pixel-control Q map, straight from the deconv's epilogue: h16 bf16 [S,9,9,32] -> f32 [S,20,20].
+  A [16] bias with [4,64,32] taps selects the 16-channel head (8..15 actions)."""
   s = h16.numel() // 2592
   if out is None:
     out = torch.empty(s, 20, 20, dtype=torch.float32, device=h16.device)
-  call("unreal_pc_deconv_qmax", ptr(h16, torch.bfloat16, "h16"), ptr(w_dtaps, torch.bfloat16, "w_dtaps"),
+  call("unreal_pc_deconv_qmax16" if _pc16(w_dtaps, bias8) else "unreal_pc_deconv_qmax", ptr(h16, torch.bfloat16, "h16"),
+       ptr(w_dtaps, torch.bfloat16, "w_dtaps"),
        ptr(bias8, torch.float32, "bias8"), int(num_actions), s, ptr(out, torch.float32, "qmax"), stream_ptr())
   return out
 
@@ -879,9 +889,19 @@ def pc_deconv_loss(h16, w_dtaps, bias8, act, target, mask, num_actions, lam, c8=
   """Pixel-control head + loss in one kernel: h16 bf16 [S,9,9,32] (any view of S*2592) -> (loss f64 [1],
   dy16 bf16 [S,400,16] = d loss / d pre-ReLU output, un-scaled by the upstream gradient, db8 [8]).  `c8`: the gradient
   without its 8 zero padding channels, [S,400,8]; `planes`: as four parity planes of the 10 x 10 space-to-depth grid,
-  [S,4,100,8] (pc_planes_conv / pc_planes_wgrad)."""
+  [S,4,100,8] (pc_planes_conv / pc_planes_wgrad).  A [16] bias with [4,64,32] taps selects the 16-channel head (8..15
+  actions): dy16 [S,400,16] with every channel real and db [16]; it has no c8 or planes layout."""
   s = h16.numel() // 2592
   loss = torch.zeros(1, dtype=torch.float64, device=h16.device)
+  if _pc16(w_dtaps, bias8):
+    if c8 or planes:
+      raise _lib.UnrealError("the 16-channel pixel-control head writes its loss gradient in conv2's [S,400,16] layout only")
+    dy16 = torch.empty(s, 400, 16, dtype=torch.bfloat16, device=h16.device)
+    db16 = torch.zeros(16, dtype=torch.float32, device=h16.device)
+    call("unreal_pc_deconv_loss16", ptr(h16, torch.bfloat16, "h16"), ptr(w_dtaps, torch.bfloat16, "w_dtaps"),
+         ptr(bias8, torch.float32, "bias16"), ptr(act, torch.int32, "act"), ptr(target, torch.float32, "target"),
+         ptr(mask, torch.float32, "mask"), int(num_actions), float(lam), s, ptr(loss), ptr(dy16), ptr(db16), stream_ptr())
+    return loss, dy16, db16
   if planes:
     dy16 = torch.empty(s, 4, 100, 8, dtype=torch.bfloat16, device=h16.device)
   else:

@@ -73,6 +73,9 @@ class UnrealModel(object):
     self._thread_index = thread_index
     self._use_lstm = use_lstm
     self._use_pixel_change = use_pixel_change
+    if use_pixel_change and A > 15:
+      raise _lib.UnrealError("pixel control supports up to 15 actions (a 16-channel head: the value and 15 advantages), "
+                             "got %d" % A)
     self._use_value_replay = use_value_replay
     self._use_reward_prediction = use_reward_prediction
     self._pixel_change_lambda = float(pixel_change_lambda)
@@ -113,8 +116,9 @@ class UnrealModel(object):
     # the captured data phase -- no gain (scripts/act_heads_bench.py); kept as a tested option
     self.fused_act_heads = False
     # ... and the layout of the loss gradient between the fused deconv + loss kernel and the two backward kernels: "planes"
-    # (four parity planes of 8 channels, one bulk copy per sample), "c8" ([S,400,8]) or "c16" (conv2's geometry, zero padded)
-    self.pc_grad_layout = "planes"
+    # (four parity planes of 8 channels, one bulk copy per sample), "c8" ([S,400,8]) or "c16" (conv2's geometry, zero padded).
+    # 8..15 actions: the 16-channel head, whose only layout is "c16" (all 16 channels real)
+    self.pc_grad_layout = "planes" if A <= 7 else "c16"
     self._cells49 = torch.tensor([[x, y] for y in range(7) for x in range(7)], dtype=torch.int32, device=self._device)
     self._fc_tab_act = torch.zeros(49, 256, dtype=torch.bfloat16, device=self._device)
     self._act_xh = {}         # acting-step [x, h] GEMM operands by batch size (persistent: padding columns stay zero)
@@ -206,7 +210,23 @@ class UnrealModel(object):
         h2 = self._encoder_fn(p32, self._cells49)
         K.gemm_bf16(h2.view(49, 2592), self.v16["W_base_fc1"], out=self._fc_tab_act, b_mn_major=True, bias=p32["b_base_fc1"],
                     relu=True)
-    if self._use_pixel_change:
+    if self._use_pixel_change and self._action_size > 7:
+      # 8..15 actions: merged 16-channel shadow (channel 0 = value, 1..A = advantages, the rest zero) in conv2's geometry --
+      # the deconv is conv2's transposed-convolution kernel, its backward pass conv2's forward and filter-gradient kernels
+      A = self._action_size
+      w16 = torch.zeros(4, 4, 16, 32, dtype=torch.bfloat16, device=self._device)
+      w16[:, :, 0:1] = self.v16["W_pc_deconv_v"]; w16[:, :, 1:1 + A] = self.v16["W_pc_deconv_a"]
+      b16 = torch.zeros(16, dtype=torch.float32, device=self._device)
+      with torch.no_grad():
+        v32 = self._views(self.flat)
+        b16[0:1] = v32["b_pc_deconv_v"]; b16[1:1 + A] = v32["b_pc_deconv_a"]
+      t16 = K.conv2_dgrad_taps(w16)
+      l16 = K.conv_taps(w16, 2)
+      if getattr(self, "pc_taps16", None) is None:
+        self.pc_taps16, self.pc_b16, self.pc_lin_taps = t16, b16, l16
+      else:
+        self.pc_taps16.copy_(t16); self.pc_b16.copy_(b16); self.pc_lin_taps.copy_(l16)
+    elif self._use_pixel_change:
       # merged 8-channel shadow of the two pixel-control deconv filters: channel 0 = value, 1..A = advantages
       A = self._action_size
       w8 = torch.zeros(4, 4, 8, 32, dtype=torch.bfloat16, device=self._device)
@@ -309,7 +329,7 @@ class UnrealModel(object):
   def _policy_value(self, p32, h, v_out=None):
     """model.py:358-377 (tiny [.,256]x[256,A+1] products, fp32).  Without autograd (acting, bootstraps): one fused
     head kernel (logits + softmax + value); with autograd: plain torch ops (the losses use A3CHeadLossFn instead)."""
-    if self.fused_heads and not torch.is_grad_enabled() and self._action_size <= 7:
+    if self.fused_heads and not torch.is_grad_enabled() and self._action_size <= 15:
       lead = h.shape[:-1]
       out = K.a3c_head(h.reshape(-1, 256).contiguous(), p32["W_base_fc_p"].contiguous(), p32["b_base_fc_p"],
                        p32["W_base_fc_v"].reshape(256).contiguous(), p32["b_base_fc_v"], want_pi=True, want_v=True,
@@ -326,10 +346,15 @@ class UnrealModel(object):
     (channel 0 = value stream, 1..A = advantage stream)."""
     A = self._action_size
     if A > 7:
-      raise _lib.UnrealError("the merged pixel-control head supports up to 7 actions")
+      raise _lib.UnrealError(self._pc16_requirement())
     hp = LinearFn.apply(h, self.v16["W_pc_fc1"], p32["W_pc_fc1"], p32["b_pc_fc1"], True, True)
     return Deconv8Fn.apply(hp, self.pc_w8, self.pc_b8, p32["W_pc_deconv_v"], p32["b_pc_deconv_v"],
                            p32["W_pc_deconv_a"], p32["b_pc_deconv_a"], A, self.pc_taps if self.fused_conv else None)
+
+  def _pc16_requirement(self):
+    return ("with %d actions pixel control runs on the 16-channel fused tower only: it needs fused_conv, fused_encoder, "
+            "fused_pc_loss and fused_pc_relu on and pc_grad_layout 'c16' (bootstraps: fused_conv and fused_pc_loss)"
+            % self._action_size)
 
   def _pc_q(self, p32, h):
     """model.py:431-441: dueling combine.  h [S,256] f32 -> q [S,20,20,A], q_max [S,20,20]."""
@@ -471,10 +496,12 @@ class UnrealModel(object):
     img = self._images(s_t)
     p32, h, _ = self._step(s_t, last_action_reward, self._zeros_state(img.shape[1]))
     with torch.no_grad():
-      if self.fused_conv and self.fused_pc_loss and self._action_size <= 7:
+      if self.fused_conv and self.fused_pc_loss:
         # pc_fc1 GEMM, then the deconv with the dueling combine + max over actions in its epilogue (no [N,20,20,8] output)
         hp = K.gemm_bf16(h.to(torch.bfloat16), self.v16["W_pc_fc1"], b_mn_major=True, bias=p32["b_pc_fc1"], relu=True,
                          out_dtype=torch.bfloat16)
+        if self._action_size > 7:
+          return K.pc_deconv_qmax(hp, self.pc_taps16, self.pc_b16, self._action_size)
         return K.pc_deconv_qmax(hp, self.pc_taps, self.pc_b8, self._action_size)
       return self._pc_q(p32, h)[1]
 
@@ -515,7 +542,7 @@ class UnrealModel(object):
     tables = self._cell_tables(p32) if self._use_tables(b["images"]) else None
     (h, _, _), _ = self._tower(p32, b["images"], b["lar"], b["c0"], b["h0"], tables)
     mask = b["mask"].to(torch.float32)
-    if self.fused_heads and self._action_size <= 7:
+    if self.fused_heads and self._action_size <= 15:
       t_, n_ = h.shape[:2]
       pol, val, ent = A3CHeadLossFn.apply(
           h.reshape(t_ * n_, 256), p32["W_base_fc_p"], p32["b_base_fc_p"], p32["W_base_fc_v"], p32["b_base_fc_v"],
@@ -537,7 +564,15 @@ class UnrealModel(object):
       act = f["a"].reshape(L * n, -1).argmax(-1).to(torch.int32)
       tgt = f["R"].reshape(L * n, 400).contiguous()
       msk = f["mask"].reshape(L * n).to(torch.float32).contiguous()
-      if self.fused_conv and self.fused_encoder and self.fused_pc_loss and self.fused_pc_relu:
+      fused_tower = self.fused_conv and self.fused_encoder and self.fused_pc_loss and self.fused_pc_relu
+      if self._action_size > 7:
+        if not (fused_tower and self.pc_grad_layout == "c16"):
+          raise _lib.UnrealError(self._pc16_requirement())
+        parts["pc"] = PcTowerFusedFn.apply(h.reshape(L * n, 256), self.v16["W_pc_fc1"], p32["W_pc_fc1"], p32["b_pc_fc1"],
+                                           self.pc_taps16, self.pc_b16, self.pc_lin_taps, p32["W_pc_deconv_v"],
+                                           p32["b_pc_deconv_v"], p32["W_pc_deconv_a"], p32["b_pc_deconv_a"], act, tgt, msk,
+                                           self._action_size, self._pixel_change_lambda)
+      elif fused_tower:
         # pc_fc1 + deconv + loss as one node: the ReLU / bias gradient of pc_fc1 leaves the backward convolution's epilogue
         parts["pc"] = PcTowerFusedFn.apply(h.reshape(L * n, 256), self.v16["W_pc_fc1"], p32["W_pc_fc1"], p32["b_pc_fc1"],
                                            self.pc_taps, self.pc_b8,
