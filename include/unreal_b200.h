@@ -106,6 +106,15 @@ int unreal_maze_pixel_change(const int32_t* pos0, const int32_t* pos1, float* pc
  * len int32 [n] nullable (valid steps per env; later rows of tgt are zero), boot f32 [n,20,20], tgt f32 [t,n,20,20]. */
 int unreal_maze_pc_targets(const int32_t* pos0, const int32_t* pos1, const int32_t* len, const float* boot, float gamma_pc,
                            float* tgt, int t, int n, void* stream);
+/* The targets of a maze rollout pass in one launch, from the frame records K1 wrote: the reverse loops of
+ * Trainer._process_base (trainer.py:298-324) and Trainer._process_pc (:352-372).  Equal, bit for bit, to
+ * unreal_nstep_returns on the pass's rewards / terminals + unreal_pc_targets on its pixel-change maps, which it never
+ * reads: the maps are evaluated from the two cells of each record.  A record whose valid bit is 0 counts as reward 0,
+ * not terminal and map 0.  rec u64 [t,n], values [t,n] f32, boot_value [n], boot_q [n,20,20] -> out_R, out_adv [t,n]
+ * and pc_tgt [t,n,20,20] f32; all time-major. */
+int unreal_maze_rollout_targets(const uint64_t* rec, const float* values, const float* boot_value, const float* boot_q,
+                                float gamma, float gamma_pc, float* out_R, float* out_adv, float* pc_tgt, int t, int n,
+                                void* stream);
 
 /* ---- K2: Environment._calc_pixel_change + _subsample (environment.py:88-99) ------------
  * literal |cur-prev| over the 2-pixel-cropped frame, mean over channels, 4x4 mean.

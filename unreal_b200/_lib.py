@@ -46,6 +46,7 @@ SIGNATURES = {
     "unreal_maze_render": (c_int, [P, P, c_int, c_int, P]),
     "unreal_maze_pixel_change": (c_int, [P, P, P, c_int, P]),
     "unreal_maze_pc_targets": (c_int, [P, P, P, P, c_float, P, c_int, c_int, P]),
+    "unreal_maze_rollout_targets": (c_int, [P, P, P, P, c_float, c_float, P, P, P, c_int, c_int, P]),
     "unreal_pixel_change": (c_int, [P, P, c_int, P, c_int, c_int, c_int, c_int, P]),
     "unreal_pixel_change_stream": (c_int, [P, c_int, P, c_int, c_int, c_int, c_int, c_int, P]),
     "unreal_selfcheck_arith": (c_int, [P, P]),

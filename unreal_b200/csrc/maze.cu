@@ -93,17 +93,26 @@ __device__ __forceinline__ EnvInfo env_logic(const StepArgs& a, int e) {
   return o;
 }
 
+// The 4 pool-column weights pc_overlap(j0 + u, c), u = 0..3, as the bytes of one word: along the pool index a cell's
+// weights are the run [2, 4, 4, 2] starting at 3c - 1, so the word is that run shifted to byte offset 3c - 1 - j0.
+__device__ __forceinline__ uint32_t pc_overlap4(int j0, int c) {
+  const int s = 8 * (3 * c - 1 - j0);
+  const uint32_t run = 0x02040402u;
+  return s >= 0 ? (s < 32 ? run << s : 0u) : (s > -32 ? run >> -s : 0u);
+}
+
 // 100 threads write the 20x20 map of one env as float4: k/48 with
 // k = ov(i,y0)*ov(j,x0) + ov(i,y1)*ov(j,x1), 0 when the agent did not move.
 __device__ __forceinline__ float4 pc_value4(int x0, int y0, int x1, int y1, int q) {
-  int i = q / 5, j0 = (q - i * 5) * 4;
-  bool moved = (x0 != x1) || (y0 != y1);
-  int wy0 = pc_overlap(i, y0), wy1 = pc_overlap(i, y1);
-  if (!moved || (wy0 | wy1) == 0) return make_float4(0.f, 0.f, 0.f, 0.f);    // most rows of the map touch neither square
+  const int i = q / 5, j0 = (q - i * 5) * 4;
+  const bool moved = (x0 != x1) || (y0 != y1);
+  // the four k of the float4 as bytes (each an integer <= 32), two multiply-adds for all four
+  const uint32_t k4 = moved ? (uint32_t)pc_overlap(i, y0) * pc_overlap4(j0, x0) + (uint32_t)pc_overlap(i, y1) * pc_overlap4(j0, x1)
+                            : 0u;
   float v[4];
 #pragma unroll
   for (int u = 0; u < 4; ++u) {
-    const float k = (float)(wy0 * pc_overlap(j0 + u, x0) + wy1 * pc_overlap(j0 + u, x1));      // an integer <= 32
+    const float k = (float)((k4 >> (8 * u)) & 0xffu);
     // k / 48 correctly rounded (= float32 of the reference's float64 means) without the IEEE-division sequence: one
     // Newton correction of k * RN(1/48) with exact FMA residuals; equal to k / 48.0f for every integer k < 200
     // (checked exhaustively; tests/test_gpu_maze.py compares every cell pair with the literal reference computation)
@@ -112,8 +121,9 @@ __device__ __forceinline__ float4 pc_value4(int x0, int y0, int x1, int y1, int 
   }
   return make_float4(v[0], v[1], v[2], v[3]);
 }
+// the maps are write-once outputs nothing in the pass reads back: streamed, so they do not hold L2 against the frames
 __device__ __forceinline__ void write_pc(float* pc, const EnvInfo& f, int q) {
-  reinterpret_cast<float4*>(pc)[q] = pc_value4(f.x0, f.y0, f.x1, f.y1, q);
+  __stcs(reinterpret_cast<float4*>(pc) + q, pc_value4(f.x0, f.y0, f.x1, f.y1, q));
 }
 
 template <typename T> struct One;
@@ -389,15 +399,18 @@ __device__ __forceinline__ EnvInfo window_logic(const WindowArgs& a, int e, int 
   return o;
 }
 
+// t <= 32: the actions are all loaded before the recurrence (unrolled, predicated), one memory round trip instead of t
 __global__ void maze_window_state_kernel(int32_t* pos, int32_t* last_action, float* last_reward,
                                          const int32_t* __restrict__ action, int n, int t, int auto_reset) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= n) return;
+  int acts[32];
+#pragma unroll
+  for (int s = 0; s < 32; ++s) acts[s] = (s < t) ? __ldg(action + (size_t)s * n + e) : 0;
   MazeCursor c{pos[2 * e], pos[2 * e + 1], last_action[e], last_reward[e]};
-  for (int s = 0; s < t; ++s) {
-    const int act = action[(size_t)s * n + e];
-    cursor_advance(c, maze_step_core(c_maze, c.x, c.y, act), act, auto_reset);
-  }
+#pragma unroll
+  for (int s = 0; s < 32; ++s)
+    if (s < t) cursor_advance(c, maze_step_core(c_maze, c.x, c.y, acts[s]), acts[s], auto_reset);
   pos[2 * e] = c.x; pos[2 * e + 1] = c.y; last_action[e] = c.la; last_reward[e] = c.lr;
 }
 
@@ -622,6 +635,95 @@ __global__ void __launch_bounds__(128) maze_pc_targets_kernel(const int2* __rest
   }
 }
 
+// The targets of a rollout pass (trainer.py:298-324 and :352-372) from the [T,N] frame records K1 wrote: rewards,
+// terminals and both cells of every step are in the record, so the [T,N,20,20] pixel-change maps are evaluated in
+// registers (pc_value4, bit-identical to K1's maps) instead of being read back.  A record whose valid bit is 0 counts
+// as reward 0, not terminal, map 0 (what the per-step K1 writes for an inactive env).  Blocks [0, ret_blocks) hold
+// one thread per env for R / adv (coalesced [T,N] loads); the rest one thread per (env, float4 q and q + 50 of the
+// map) for the PC targets: half the threads of one per float4, so the grid fits in one wave of the SMs at 4096 envs
+// (measured on B200 at 4096 x 20: 31 us instead of 37 with one float4 per thread).  Both recurrences run in the order
+// and with the roundings of nstep_returns_kernel / pc_targets_kernel, so the results are bit-equal to those two kernels
+// on the same pass.  Each chunk's loads are issued before its scan.
+constexpr int kTgtThreads = 128;
+constexpr int kTgtChunk = 10;     // R / adv steps loaded ahead of their scan
+constexpr int kTgtPcChunk = 5;    // PC-target steps loaded ahead of theirs
+constexpr int kTgtPcPer = 2;      // float4 of the map per thread
+constexpr int kTgtPcCols = kPcElems / 4 / kTgtPcPer;
+
+__device__ __forceinline__ uint64_t valid_record(uint64_t r) { return frame_valid(r) ? r : 0ull; }
+
+__global__ void __launch_bounds__(kTgtThreads, 8) maze_rollout_targets_kernel(
+    const uint64_t* __restrict__ rec, const float* __restrict__ values, const float* __restrict__ boot_value,
+    const float4* __restrict__ boot_q, float gamma, float gamma_pc, float* __restrict__ out_R,
+    float* __restrict__ out_adv, float4* __restrict__ tgt, int T, int N, int ret_blocks) {
+  if ((int)blockIdx.x < ret_blocks) {
+    const int n = blockIdx.x * kTgtThreads + threadIdx.x;
+    if (n >= N) return;
+    float R = boot_value[n];
+    for (int hi = T; hi > 0; hi -= kTgtChunk) {
+      const int lo = hi - kTgtChunk;
+      int rr[kTgtChunk];        // the reward byte | terminal << 8
+      float vv[kTgtChunk];
+#pragma unroll
+      for (int k = 0; k < kTgtChunk; ++k) {
+        if (lo + k >= 0) {
+          const size_t o = (size_t)(lo + k) * N + n;
+          const uint64_t r = valid_record(__ldg(rec + o));
+          rr[k] = (frame_reward(r) & 0xff) | (frame_terminal(r) << 8);
+          vv[k] = __ldcs(values + o);
+        }
+      }
+#pragma unroll
+      for (int k = kTgtChunk - 1; k >= 0; --k) {
+        if (lo + k >= 0) {
+          const size_t o = (size_t)(lo + k) * N + n;
+          R = (rr[k] & 0x100) ? 0.f : R;                                   // (:298-300)
+          R = __fadd_rn((float)(int8_t)rr[k], __fmul_rn(gamma, R));       // R = ri + gamma * R   (:314)
+          __stcs(out_R + o, R);
+          __stcs(out_adv + o, __fsub_rn(R, vv[k]));                        // adv = R - Vi   (:315)
+        }
+      }
+    }
+    return;
+  }
+  const size_t per_t = (size_t)N * (kPcElems / 4);
+  const size_t col = (size_t)(blockIdx.x - ret_blocks) * kTgtThreads + threadIdx.x;   // over N * kTgtPcCols
+  if (col >= (size_t)N * kTgtPcCols) return;
+  const int n = (int)(col / kTgtPcCols), q0 = (int)(col - (size_t)n * kTgtPcCols);
+  const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+  float4 R[kTgtPcPer];
+#pragma unroll
+  for (int p = 0; p < kTgtPcPer; ++p) R[p] = boot_q[(size_t)n * (kPcElems / 4) + q0 + p * kTgtPcCols];
+  for (int hi = T; hi > 0; hi -= kTgtPcChunk) {
+    const int lo = hi - kTgtPcChunk;
+    uint32_t cc[kTgtPcChunk];   // the record's two cells (its low 16 bits) | terminal << 16
+#pragma unroll
+    for (int k = 0; k < kTgtPcChunk; ++k) {
+      if (lo + k >= 0) {
+        const uint64_t r = valid_record(__ldg(rec + (size_t)(lo + k) * N + n));
+        cc[k] = (uint32_t)(r & 0xffffu) | ((uint32_t)frame_terminal(r) << 16);
+      }
+    }
+#pragma unroll
+    for (int k = kTgtPcChunk - 1; k >= 0; --k) {
+      if (lo + k >= 0) {
+        const uint64_t r = cc[k];
+#pragma unroll
+        for (int p = 0; p < kTgtPcPer; ++p) {
+          const int q = q0 + p * kTgtPcCols;
+          const float4 pc = pc_value4(frame_x0(r), frame_y0(r), frame_x1(r), frame_y1(r), q);
+          if (r >> 16) R[p] = zero;
+          R[p].x = __fadd_rn(pc.x, __fmul_rn(gamma_pc, R[p].x));   // pc_R = pixel_change + gamma_pc * pc_R   (:361)
+          R[p].y = __fadd_rn(pc.y, __fmul_rn(gamma_pc, R[p].y));
+          R[p].z = __fadd_rn(pc.z, __fmul_rn(gamma_pc, R[p].z));
+          R[p].w = __fadd_rn(pc.w, __fmul_rn(gamma_pc, R[p].w));
+          __stcs(tgt + (size_t)(lo + k) * per_t + (size_t)n * (kPcElems / 4) + q, R[p]);
+        }
+      }
+    }
+  }
+}
+
 __global__ void maze_reset_kernel(int32_t* pos, int32_t* last_action, float* last_reward, const uint8_t* mask,
                                   int n) {
   int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -820,6 +922,25 @@ extern "C" int unreal_maze_pc_targets(const int32_t* pos0, const int32_t* pos1, 
       reinterpret_cast<const int2*>(pos0), reinterpret_cast<const int2*>(pos1), len, reinterpret_cast<const float4*>(boot),
       gamma_pc, reinterpret_cast<float4*>(tgt), t, n);
   UNREAL_LAUNCH_CHECK("maze_pc_targets_kernel");
+  return UNREAL_OK;
+}
+
+extern "C" int unreal_maze_rollout_targets(const uint64_t* rec, const float* values, const float* boot_value,
+                                           const float* boot_q, float gamma, float gamma_pc, float* out_R, float* out_adv,
+                                           float* pc_tgt, int t, int n, void* stream) {
+  UNREAL_REQUIRE(t >= 0 && n >= 0, "unreal_maze_rollout_targets: negative size");
+  if (t == 0 || n == 0) return UNREAL_OK;
+  UNREAL_REQUIRE(rec && values && boot_value && boot_q && out_R && out_adv && pc_tgt,
+                 "unreal_maze_rollout_targets: null argument");
+  UNREAL_REQUIRE(aligned16(boot_q) && aligned16(pc_tgt) && (reinterpret_cast<uintptr_t>(rec) & 7u) == 0,
+                 "unreal_maze_rollout_targets: alignment (boot_q / pc_tgt 16 bytes; rec 8)");
+  const long long cols = (long long)n * kTgtPcCols;
+  const int ret_blocks = (n + kTgtThreads - 1) / kTgtThreads;
+  const long long blocks = ret_blocks + (cols + kTgtThreads - 1) / kTgtThreads;
+  maze_rollout_targets_kernel<<<(unsigned)blocks, kTgtThreads, 0, as_stream(stream)>>>(
+      rec, values, boot_value, reinterpret_cast<const float4*>(boot_q), gamma, gamma_pc, out_R, out_adv,
+      reinterpret_cast<float4*>(pc_tgt), t, n, ret_blocks);
+  UNREAL_LAUNCH_CHECK("maze_rollout_targets_kernel");
   return UNREAL_OK;
 }
 

@@ -144,6 +144,23 @@ def maze_pc_targets(pos0, pos1, length, boot, gamma_pc, out=None):
   return out
 
 
+def maze_rollout_targets(rec, values, boot_value, boot_q, gamma, gamma_pc, R=None, adv=None, pc_tgt=None):
+  """rec int64 [T,N] (the frame records of a maze pass), values f32 [T,N], boot_value f32 [N], boot_q f32 [N,20,20]
+  -> (R, adv [T,N], pc_tgt [T,N,20,20]) = nstep_returns + pc_targets of the pass, without its pixel-change maps."""
+  t, n = rec.shape
+  if R is None:
+    R = torch.empty(t, n, dtype=torch.float32, device=rec.device)
+  if adv is None:
+    adv = torch.empty(t, n, dtype=torch.float32, device=rec.device)
+  if pc_tgt is None:
+    pc_tgt = torch.empty(t, n, PC, PC, dtype=torch.float32, device=rec.device)
+  call("unreal_maze_rollout_targets", ptr(rec, torch.int64, "rec"), ptr(values, torch.float32, "values"),
+       ptr(boot_value, torch.float32, "boot_value"), ptr(boot_q, torch.float32, "boot_q"), float(gamma), float(gamma_pc),
+       ptr(R, torch.float32, "R"), ptr(adv, torch.float32, "adv"), ptr(pc_tgt, torch.float32, "pc_tgt"), t, n,
+       stream_ptr())
+  return R, adv, pc_tgt
+
+
 # ---------------------------------------------------------------------------- pixel change (generic)
 def pixel_change(cur, prev, out=None):
   """cur, prev [M,H,W,C] float32 or uint8 -> [M,(H-4)//4,(W-4)//4] float32."""

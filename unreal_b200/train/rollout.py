@@ -2,10 +2,12 @@
 environment loop and reverse scans (train/trainer.py:218-336) and of the pixel-control
 target scan (trainer.py:352-372) for N mazes at once.
 
-One *pass* = T launches of K1 (step + render + pixel-change, one per rollout step, each
-writing its own [t] slice of the rollout buffers) followed by K3 (n-step returns and
-advantages) and K4 (PC Q-targets).  The T+2 launches are captured into CUDA graphs so a
-pass costs three graph launches.  All rollout buffers stay resident in HBM for the learner:
+One *pass* = K1 (step + render + pixel-change of all T rollout steps: one window launch, or
+T launches each writing its own [t] slice of the rollout buffers) followed by ONE targets
+launch (unreal_maze_rollout_targets: n-step returns, advantages and PC Q-targets from the
+frame records K1 wrote; the pixel-change maps are not read back).  The two phases are
+captured into CUDA graphs, so a pass costs two graph launches.  All rollout buffers stay
+resident in HBM for the learner:
 
   obs      [T, N, 84, 84, 3]  f32 | u8     model input of each step's *next* state
   pc       [T, N, 20, 20]     f32          pixel change caused by each step
@@ -64,10 +66,10 @@ class RolloutTargets(object):
   # launches per pass, by kernel
   @property
   def launches_per_pass(self):
-    # window form: u8 = one warp-per-env kernel; f32 = one CTA-per-item kernel + the state kernel
-    return ((1 if self.obs.dtype == torch.uint8 else 2) if self.window_kernel else self.t) + 2
+    # window form: u8 = one warp-per-env kernel; f32 = one CTA-per-item kernel + the state kernel; + the targets kernel
+    return ((1 if self.obs.dtype == torch.uint8 else 2) if self.window_kernel else self.t) + 1
 
-  # ---- the three phases, eager --------------------------------------------------------
+  # ---- the two phases, eager ----------------------------------------------------------
   def _steps(self):
     if self.window_kernel:
       K.maze_window(self.state, self.actions, obs=self.obs, pc=self.pc, reward=self.reward, terminal=self.terminal,
@@ -77,19 +79,17 @@ class RolloutTargets(object):
       K.maze_step(self.state, self.actions[t], obs=self.obs[t], pc=self.pc[t], reward=self.reward[t],
                   terminal=self.terminal[t], frame_rec=self.frame_rec[t], auto_reset=self.auto_reset)
 
-  def _returns(self):
-    K.nstep_returns(self.reward, self.values, self.terminal, self.boot_value, self.gamma, self.R, self.adv)
-
-  def _pc_targets(self):
-    K.pc_targets(self.pc, self.terminal, None, self.boot_q, self.gamma_pc, self.pc_tgt)
+  def _targets(self):
+    K.maze_rollout_targets(self.frame_rec, self.values, self.boot_value, self.boot_q, self.gamma, self.gamma_pc,
+                           self.R, self.adv, self.pc_tgt)
 
   def _capture(self):
     torch.cuda.synchronize(self.device)
-    self._steps(); self._returns(); self._pc_targets()       # warm the lazy init paths before capture
+    self._steps(); self._targets()                            # warm the lazy init paths before capture
     K.maze_reset(self.state)
     torch.cuda.synchronize(self.device)
     graphs = []
-    for fn in (self._steps, self._returns, self._pc_targets):
+    for fn in (self._steps, self._targets):
       g = torch.cuda.CUDAGraph()
       with _lib.graph_capture(g):
         fn()
@@ -98,18 +98,21 @@ class RolloutTargets(object):
 
   def run_device(self, events=None):
     """One pass with inputs already in HBM.  `events`: optional list of 4 CUDA events recorded
-    before K1s / after K1s / after K3 / after K4 on the current stream."""
+    on the current stream before K1 / after K1 / after the targets launch / again after it (the
+    targets of K3 and K4 are one launch; the fourth event keeps the K1 / K3 / K4 timing layout,
+    with a K4 span of ~0)."""
     with torch.cuda.device(self.device):
       if self.use_graphs and self._graphs is None:
         self._capture()
-      phases = ([g.replay for g in self._graphs] if self.use_graphs
-                else [self._steps, self._returns, self._pc_targets])
+      phases = [g.replay for g in self._graphs] if self.use_graphs else [self._steps, self._targets]
       if events is not None:
         events[0].record()
       for i, ph in enumerate(phases):
         ph()
         if events is not None:
           events[i + 1].record()
+      if events is not None:
+        events[3].record()
 
   # ---- host-buffer entry point (what a CPU-side caller of the reference API would use) --
   def _ensure_host(self):
@@ -148,9 +151,10 @@ class RolloutTargets(object):
     as numpy views of pinned memory (valid until the next call).  Frames, pixel-change maps
     and PC targets stay on the device for the learner.
 
-    The copies are pipelined around the three phases on a second stream: only the actions
-    (T*N*4 bytes) gate the first K1 launch; values / bootstraps travel while the T steps run,
-    rewards / terminals return under K3+K4 and returns / advantages under K4."""
+    The copies are pipelined around the two phases on a second stream: only the actions
+    (T*N*4 bytes) gate K1; values / bootstraps travel while K1 runs and are waited for just
+    before the targets launch, rewards / terminals return under the targets kernel and
+    returns / advantages after it."""
     self._ensure_host()
     hi, ho = self._h_in, self._h_out
     for name, arr in (("actions", actions), ("values", values), ("boot_value", boot_value), ("boot_q", boot_q)):
@@ -167,7 +171,7 @@ class RolloutTargets(object):
         self._ev = [torch.cuda.Event() for _ in range(5)]
       main = torch.cuda.current_stream()
       if self.use_graphs and self.host_graph:
-        # the whole pass -- the H2D copies, the three phases and the D2H copies with their cross-stream overlap -- as ONE
+        # the whole pass -- the H2D copies, the two phases and the D2H copies with their cross-stream overlap -- as ONE
         # CUDA graph over the pinned staging buffers: one launch and one synchronisation per call instead of ~15 API calls
         if self._host_graph is None:
           self._pipeline(main)                                # THIS call's pass, eagerly (creates every lazy resource)
@@ -187,9 +191,9 @@ class RolloutTargets(object):
     """The copies and phases of one host-buffer pass on `main` + the copy stream (see run_host)."""
     hi, ho = self._h_in, self._h_out
     side = self._copy_stream
-    ev_start, ev_in, ev_k1, ev_k3, ev_out = self._ev
+    ev_start, ev_in, ev_k1, ev_tg, ev_out = self._ev
     phases = ([g.replay for g in self._graphs] if (self.use_graphs and replay_graphs)
-              else [self._steps, self._returns, self._pc_targets])
+              else [self._steps, self._targets])
     ev_start.record(main)
     self.actions.copy_(hi["actions"], non_blocking=True)
     side.wait_event(ev_start)                      # previous pass has finished with the inputs
@@ -205,12 +209,11 @@ class RolloutTargets(object):
       ho["reward"].copy_(self.reward, non_blocking=True)
       ho["terminal"].copy_(self.terminal, non_blocking=True)
     main.wait_event(ev_in)
-    phases[1]()                                    # K3
-    ev_k3.record(main)
+    phases[1]()                                    # targets: R, adv, PC targets
+    ev_tg.record(main)
     with torch.cuda.stream(side):
-      side.wait_event(ev_k3)
+      side.wait_event(ev_tg)
       ho["R"].copy_(self.R, non_blocking=True)
       ho["adv"].copy_(self.adv, non_blocking=True)
       ev_out.record(side)
-    phases[2]()                                    # K4
     main.wait_event(ev_out)
