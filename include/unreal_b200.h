@@ -18,6 +18,8 @@
  *     The only library-owned memory is what *_create() returns handles to.
  *   - layouts are C-contiguous; [T, N] means time-major (one row per rollout step).
  *   - a handle must not be used from two host threads at once; distinct handles are independent.
+ *   - work runs on the current device; the maze map is process-wide and applies on every device,
+ *     and the library's lazy set-up (kernel attributes, device queries, the map upload) is per device.
  */
 #ifndef UNREAL_B200_H_
 #define UNREAL_B200_H_

@@ -4,7 +4,9 @@
 
 #include <map>
 #include <mutex>
+#include <set>
 #include <string>
+#include <utility>
 
 #include "common.cuh"
 
@@ -24,17 +26,32 @@ int cuda_fail(cudaError_t e, const char* what) {
   return UNREAL_ECUDA;
 }
 
+// Lazy set-up is per device: a process may drive several devices, and function attributes and device properties belong to
+// the device that was current when they were set or queried.
+static std::mutex g_dev_mu;
+
 int sm_count() {
-  static int cached = 0;
-  if (cached > 0) return cached;
+  static std::map<int, int> cached;   // device -> SM count
   int dev = 0, n = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess ||
-      cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
-    set_error("cannot query the SM count (no CUDA device?)");
-    return 0;
+  if (cudaGetDevice(&dev) == cudaSuccess) {
+    std::lock_guard<std::mutex> lk(g_dev_mu);
+    auto it = cached.find(dev);
+    if (it != cached.end()) return it->second;
+    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess) return cached[dev] = n;
   }
-  cached = n;
-  return n;
+  set_error("cannot query the SM count (no CUDA device?)");
+  return 0;
+}
+
+int allow_dynamic_smem(const void* kernel, int bytes) {
+  static std::set<std::pair<const void*, int>> done;
+  int dev = 0;
+  UNREAL_CUDA(cudaGetDevice(&dev));
+  std::lock_guard<std::mutex> lk(g_dev_mu);
+  if (done.count({kernel, dev})) return UNREAL_OK;
+  UNREAL_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  done.insert({kernel, dev});
+  return UNREAL_OK;
 }
 
 static std::mutex g_tun_mu;

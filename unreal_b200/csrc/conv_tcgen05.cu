@@ -24,15 +24,11 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "maze_core.cuh"
 #include "tc05.cuh"
 
 namespace unreal {
 using namespace tc05;
-
-int make_tma_nd_bf16(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                     const uint32_t* box, int swizzle_bytes);   // gemm_tcgen05.cu
-
-int maze_walls49(uint64_t* out);     // maze.cu
 
 // Render-fused conv1 input (maze env type): the x'' tile of a work item (6 planes x 126 pixel rows x 16 B, rows
 // rb*105.. of the 21x21 space-to-depth grid) is a pure function of the agent cell and the constant wall map --
@@ -61,8 +57,7 @@ __device__ __forceinline__ void maze_tile_to_smem(uint32_t dst, uint64_t walls49
           const uint32_t ag = (c0 == 1 ? 0x3f80u : 0u) | (c1 == 1 ? 0x3f800000u : 0u);
           v[k] = (wl & mw) | (ag & ma);
         }
-        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst + (uint32_t)(q * 126 * 16 + p * 16)), "r"(v[0]),
-                     "r"(v[1]), "r"(v[2]), "r"(v[3]) : "memory");
+        st_shared_v4(dst + (uint32_t)(q * 126 * 16 + p * 16), v[0], v[1], v[2], v[3]);
       }
     }
   }
@@ -98,17 +93,6 @@ struct ConvArgs {
   const __nv_bfloat16* mask_y;   // MASKED build: [items][rows][N] activations of the layer the result is a gradient of
   float* db;                     // MASKED build: [rows][N] += the masked, rounded result summed over items (its bias gradient)
 };
-
-__device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* m, uint32_t src, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
 
 // MASKED: the result is the gradient w.r.t. a ReLU layer's output `mask_y` (pc_fc1 seen as [S,9,9,32] behind the pixel-control
 // deconv): the epilogue zeroes it where mask_y <= 0 and sums the rounded values over items into db -- the ReLU-gradient /
@@ -158,8 +142,7 @@ conv_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+  const uint32_t tmem_base = tmem_base_at(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -246,7 +229,7 @@ conv_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_
         tmem_ld_wait();
         const uint32_t buf = ebuf + (ebuf_it & 1u) * 4096u;
         ++ebuf_it;
-        if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+        if (lane == 0) bulk_wait_read<1>();
         __syncwarp();
         const uint32_t rowp = buf + (uint32_t)lane * 128u;
 #pragma unroll
@@ -274,14 +257,13 @@ conv_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_
             }
           }
           const uint32_t chunk = (uint32_t)q ^ (uint32_t)(lane & 7);
-          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(rowp + chunk * 16u), "r"(pk[0]), "r"(pk[1]),
-                       "r"(pk[2]), "r"(pk[3]) : "memory");
+          st_shared_v4(rowp + chunk * 16u, pk[0], pk[1], pk[2], pk[3]);
         }
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) {
           tma_store_3d(&tma_c, buf, 0, quarter * 32, it);
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+          bulk_commit();
         }
       }
       fence_before_sync();
@@ -295,7 +277,7 @@ conv_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_
         for (int j = 0; j < N; ++j) atomicAdd(g.db + row * N + j, b[j]);
       }
     }
-    if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+    if (lane == 0) bulk_wait_all();
   }
   __syncwarp();
   fence_before_sync();
@@ -457,18 +439,15 @@ conv1_fwd_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfloa
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+  const uint32_t tmem_base = tmem_base_at(tmem_slot);
 
   if (warp == 0 && maze_pos != nullptr) {
     // ===== render-fused producer (maze): the warp WRITES each item's x'' tile from the agent cell =====
     if (lane == 0) {
       mbar_arrive_expect_tx(w_bar, kWB);
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                   ::"r"(w_smem), "l"(w_planes), "r"(kC1WBytes), "r"(w_bar) : "memory");
+      bulk_load(w_smem, w_planes, kC1WBytes, w_bar);
       if constexpr (SPLIT)
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"(w_smem + kC1WBytes), "l"(w_planes_lo), "r"(kC1WBytes), "r"(w_bar) : "memory");
+        bulk_load(w_smem + kC1WBytes, w_planes_lo, kC1WBytes, w_bar);
     }
     int stage = 0; uint32_t phase = 0;
     for (int it = blockIdx.x; it < items; it += gridDim.x) {
@@ -484,11 +463,9 @@ conv1_fwd_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfloa
     if (lane == 0) {
       // ===== producer: resident filters (one bulk copy), then ONE box per item =====
       mbar_arrive_expect_tx(w_bar, kWB);
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                   ::"r"(w_smem), "l"(w_planes), "r"(kC1WBytes), "r"(w_bar) : "memory");
+      bulk_load(w_smem, w_planes, kC1WBytes, w_bar);
       if constexpr (SPLIT)
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"(w_smem + kC1WBytes), "l"(w_planes_lo), "r"(kC1WBytes), "r"(w_bar) : "memory");
+        bulk_load(w_smem + kC1WBytes, w_planes_lo, kC1WBytes, w_bar);
       int stage = 0; uint32_t phase = 0;
       for (int it = blockIdx.x; it < items; it += gridDim.x) {
         mbar_wait(empty_bar(stage), phase ^ 1u);
@@ -499,16 +476,12 @@ conv1_fwd_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfloa
         const uint32_t dst = a_smem + stage * kStageBytes;
 #pragma unroll
         for (int q = 0; q < 6; ++q)
-          asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                       ::"r"(dst + q * kC1PlaneBytes), "l"(src + (int64_t)q * 441 * 16), "r"(kC1PlaneBytes),
-                         "r"(full_bar(stage)) : "memory");
+          bulk_load(dst + q * kC1PlaneBytes, src + (int64_t)q * 441 * 16, kC1PlaneBytes, full_bar(stage));
         if (has_lo) {
           const uint8_t* src_lo = reinterpret_cast<const uint8_t*>(xpp_lo) + (src - reinterpret_cast<const uint8_t*>(xpp));
 #pragma unroll
           for (int q = 0; q < 6; ++q)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(dst + kC1StageBytes + q * kC1PlaneBytes), "l"(src_lo + (int64_t)q * 441 * 16),
-                           "r"(kC1PlaneBytes), "r"(full_bar(stage)) : "memory");
+            bulk_load(dst + kC1StageBytes + q * kC1PlaneBytes, src_lo + (int64_t)q * 441 * 16, kC1PlaneBytes, full_bar(stage));
         }
         if (++stage == kStages) { stage = 0; phase ^= 1u; }
       }
@@ -640,7 +613,7 @@ conv1_wgrad_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfl
 
   // zero every tile byte once: padding rows of the x'' tiles and the never-written rows of the dY tiles
   for (uint32_t off = threadIdx.x * 16u; off < (uint32_t)(kWgStages * kWgStageBytes + kWgTail); off += 96u * 16u)
-    asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(smem_base + off), "r"(0u) : "memory");
+    st_shared_v4(smem_base + off, 0u, 0u, 0u, 0u);
   if (warp == 0 && lane == 0) {
     for (int s = 0; s < kWgStages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     mbar_init(done_bar, 1);
@@ -652,8 +625,7 @@ conv1_wgrad_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfl
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+  const uint32_t tmem_base = tmem_base_at(tmem_slot);
 
   if (warp == 0 && maze_pos != nullptr) {
     // ===== render-fused producer (maze): the x'' tile is written by the warp, only dY comes from HBM =====
@@ -674,9 +646,7 @@ conv1_wgrad_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfl
           const uint8_t* ds = reinterpret_cast<const uint8_t*>(dyp) + ((int64_t)c * dy_plane_elems / 8 + smp * 420 + rb * 105) * 16;
 #pragma unroll
           for (int t = 0; t < 4; ++t)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(dst + kWgDyOff + (t * 2 + c) * kWgDyPlane + ((t >> 1) * 21 + (t & 1)) * 16), "l"(ds), "r"(1680),
-                           "r"(full_bar(stage)) : "memory");
+            bulk_load(dst + kWgDyOff + (t * 2 + c) * kWgDyPlane + ((t >> 1) * 21 + (t & 1)) * 16, ds, 1680, full_bar(stage));
         }
       }
       if (++stage == kWgStages) { stage = 0; phase ^= 1u; }
@@ -693,9 +663,7 @@ conv1_wgrad_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfl
         const uint8_t* xs = reinterpret_cast<const uint8_t*>(xpp) + (smp * 6 * 441 + rb * 105) * 16;
 #pragma unroll
         for (int q = 0; q < 6; ++q)
-          asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                       ::"r"(dst + q * kC1PlaneBytes), "l"(xs + (int64_t)q * 441 * 16), "r"(kC1PlaneBytes),
-                         "r"(full_bar(stage)) : "memory");
+          bulk_load(dst + q * kC1PlaneBytes, xs + (int64_t)q * 441 * 16, kC1PlaneBytes, full_bar(stage));
         if (pitch21) {
           // planes already on the x'' grid's 21-pixel row pitch (column 20 zero): ONE 1680-byte copy per plane
 #pragma unroll
@@ -703,9 +671,7 @@ conv1_wgrad_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfl
             const uint8_t* ds = reinterpret_cast<const uint8_t*>(dyp) + ((int64_t)c * dy_plane_elems / 8 + smp * 420 + rb * 105) * 16;
 #pragma unroll
             for (int t = 0; t < 4; ++t)
-              asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                           ::"r"(dst + kWgDyOff + (t * 2 + c) * kWgDyPlane + ((t >> 1) * 21 + (t & 1)) * 16), "l"(ds), "r"(1680),
-                             "r"(full_bar(stage)) : "memory");
+              bulk_load(dst + kWgDyOff + (t * 2 + c) * kWgDyPlane + ((t >> 1) * 21 + (t & 1)) * 16, ds, 1680, full_bar(stage));
           }
         } else {
 #pragma unroll
@@ -715,9 +681,8 @@ conv1_wgrad_tcgen05_kernel(const __nv_bfloat16* __restrict__ xpp, const __nv_bfl
             for (int t = 0; t < 4; ++t)
 #pragma unroll
               for (int oyl = 0; oyl < 5; ++oyl)
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                             ::"r"(dst + kWgDyOff + (t * 2 + c) * kWgDyPlane + ((t >> 1) * 21 + (t & 1) + oyl * 21) * 16),
-                               "l"(ds + oyl * 320), "r"(320), "r"(full_bar(stage)) : "memory");
+                bulk_load(dst + kWgDyOff + (t * 2 + c) * kWgDyPlane + ((t >> 1) * 21 + (t & 1) + oyl * 21) * 16, ds + oyl * 320,
+                          320, full_bar(stage));
           }
         }
         if (++stage == kWgStages) { stage = 0; phase ^= 1u; }
@@ -823,7 +788,7 @@ conv2_wgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __gr
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   for (uint32_t off = threadIdx.x * 16u; off < (uint32_t)(kW2AStages * kW2ABytes + kW2BStages * kW2BBytes + kW2Tail); off += 128u * 16u)
-    asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(smem_base + off), "r"(0u) : "memory");
+    st_shared_v4(smem_base + off, 0u, 0u, 0u, 0u);
   if (warp == 0 && lane == 0) {
     prefetch_tensormap(&tma_a); prefetch_tensormap(&tma_a2); prefetch_tensormap(&tma_dy);
     for (int s = 0; s < kW2AStages; ++s) { mbar_init(fullA(s), 1); mbar_init(emptyA(s), 1); }
@@ -837,8 +802,7 @@ conv2_wgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __gr
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+  const uint32_t tmem_base = tmem_base_at(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -910,8 +874,7 @@ conv2_wgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __gr
         // thread kept the LSU queue full (ncu: lg_throttle 5.7 stalled warps per issue at the end of the kernel)
 #pragma unroll
         for (int j = 0; j < 32; j += 4)
-          asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(o + j), "f"(__uint_as_float(v[j])),
-                       "f"(__uint_as_float(v[j + 1])), "f"(__uint_as_float(v[j + 2])), "f"(__uint_as_float(v[j + 3])) : "memory");
+          red_add_v4(o + j, __uint_as_float(v[j]), __uint_as_float(v[j + 1]), __uint_as_float(v[j + 2]), __uint_as_float(v[j + 3]));
       }
     }
   }
@@ -1005,8 +968,7 @@ conv2_dgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __gr
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+  const uint32_t tmem_base = tmem_base_at(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -1460,22 +1422,19 @@ pc_planes_conv_tcgen05_kernel(const __nv_bfloat16* __restrict__ dyp, const __nv_
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+  const uint32_t tmem_base = tmem_base_at(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0) {
       // ===== producer: resident filters (one bulk copy), then ONE 6400-byte bulk copy per sample =====
       mbar_arrive_expect_tx(w_bar, kPpWBytes);
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                   ::"r"(w_smem), "l"(w_planes), "r"(kPpWBytes), "r"(w_bar) : "memory");
+      bulk_load(w_smem, w_planes, kPpWBytes, w_bar);
       int stage = 0; uint32_t phase = 0;
       for (int it = blockIdx.x; it < samples; it += gridDim.x) {
         mbar_wait(empty_bar(stage), phase ^ 1u);
         mbar_arrive_expect_tx(full_bar(stage), kPpTileBytes);
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"(a_smem + stage * kPpTileBytes), "l"(reinterpret_cast<const uint8_t*>(dyp) + (int64_t)it * kPpTileBytes),
-                       "r"(kPpTileBytes), "r"(full_bar(stage)) : "memory");
+        bulk_load(a_smem + stage * kPpTileBytes, reinterpret_cast<const uint8_t*>(dyp) + (int64_t)it * kPpTileBytes, kPpTileBytes,
+                  full_bar(stage));
         if (++stage == kPpStages) { stage = 0; phase ^= 1u; }
       }
     }
@@ -1612,7 +1571,7 @@ pc_planes_wgrad_tcgen05_kernel(const __nv_bfloat16* __restrict__ dyp, const __gr
 
   // zero every tile byte once: the never-written rows of the B tiles, and whatever A reads before its first copies land
   for (uint32_t off = threadIdx.x * 16u; off < (uint32_t)(kPwBStages * kPwBBytes + kPwAStages * kPpTileBytes + kPwTail); off += 128u * 16u)
-    asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(smem_base + off), "r"(0u) : "memory");
+    st_shared_v4(smem_base + off, 0u, 0u, 0u, 0u);
   if (warp == 0 && lane == 0) {
     prefetch_tensormap(&tma_hp);
     for (int s = 0; s < kPwAStages; ++s) { mbar_init(fullA(s), 1); mbar_init(emptyA(s), 1); }
@@ -1626,8 +1585,7 @@ pc_planes_wgrad_tcgen05_kernel(const __nv_bfloat16* __restrict__ dyp, const __gr
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+  const uint32_t tmem_base = tmem_base_at(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -1639,9 +1597,7 @@ pc_planes_wgrad_tcgen05_kernel(const __nv_bfloat16* __restrict__ dyp, const __gr
         if (++sb == kPwBStages) { sb = 0; pb ^= 1u; }
         mbar_wait(emptyA(sa), pa ^ 1u);
         mbar_arrive_expect_tx(fullA(sa), kPpTileBytes);
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"(a_smem + sa * kPpTileBytes), "l"(reinterpret_cast<const uint8_t*>(dyp) + (int64_t)it * kPpTileBytes),
-                       "r"(kPpTileBytes), "r"(fullA(sa)) : "memory");
+        bulk_load(a_smem + sa * kPpTileBytes, reinterpret_cast<const uint8_t*>(dyp) + (int64_t)it * kPpTileBytes, kPpTileBytes, fullA(sa));
         if (++sa == kPwAStages) { sa = 0; pa ^= 1u; }
       }
     }
@@ -1696,8 +1652,7 @@ pc_planes_wgrad_tcgen05_kernel(const __nv_bfloat16* __restrict__ dyp, const __gr
       if (lane < 16 && m < 32) {
 #pragma unroll
         for (int j = 0; j < 32; j += 4)
-          asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(o + j), "f"(__uint_as_float(v[j])),
-                       "f"(__uint_as_float(v[j + 1])), "f"(__uint_as_float(v[j + 2])), "f"(__uint_as_float(v[j + 3])) : "memory");
+          red_add_v4(o + j, __uint_as_float(v[j]), __uint_as_float(v[j + 1]), __uint_as_float(v[j + 2]), __uint_as_float(v[j + 3]));
       }
     }
   }
@@ -1719,12 +1674,9 @@ static int launch_conv(const CUtensorMap& ta, const CUtensorMap& ta2, const CUte
   // + 5 KB: the last stage's 128-row UMMA read runs 40 rows past its 88-row stage into barriers / epilogue buffers
   constexpr int kSmem = kWBytes + (SPLIT ? 2 * 2 * Cfg::kStageBytes : Cfg::kStages * Cfg::kStageBytes) + 1024 +
                         Cfg::kEpiWarps * 2 * 4096 + 1024;
-  static bool configured = false;
   auto kern = conv_fwd_tcgen05_kernel<N, MODE, MASKED, C, SPLIT>;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem));
-    configured = true;
-  }
+  const int rc = allow_dynamic_smem((const void*)kern, kSmem);
+  if (rc != UNREAL_OK) return rc;
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   const int grid = g.items < 2 * sms ? g.items : 2 * sms;
@@ -1773,17 +1725,10 @@ extern "C" int unreal_s2d_frames_split(const void* frames, int dtype, void* out_
 template <bool SPLIT>
 static int conv1_fwd_launch(const void* xpp, const int32_t* pos, const void* w_taps, const float* bias, void* out, int s,
                             void* stream, const void* xpp_lo = nullptr, const void* w_lo = nullptr, void* out_lo = nullptr) {
-  uint64_t walls = 0;
-  if (pos != nullptr) {
-    int rc = maze_walls49(&walls);
-    if (rc != UNREAL_OK) return rc;
-  }
+  const uint64_t walls = pos != nullptr ? maze_walls49() : 0;
   constexpr int kSmem = SPLIT ? kC1SplitSmem : kC1Smem;
-  static bool configured = false;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(conv1_fwd_tcgen05_kernel<SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem));
-    configured = true;
-  }
+  const int rc = allow_dynamic_smem((const void*)conv1_fwd_tcgen05_kernel<SPLIT>, kSmem);
+  if (rc != UNREAL_OK) return rc;
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   const int items = s * 4;
@@ -1926,18 +1871,11 @@ static int conv1_wgrad_launch(const void* xpp_bf16, const void* dy_planes_bf16, 
   UNREAL_REQUIRE(xpp_bf16 && dy_planes_bf16 && dw_taps && s > 0, "unreal_conv1_wgrad: null buffer or s <= 0");
   UNREAL_REQUIRE(aligned16(xpp_bf16) && aligned16(dy_planes_bf16) && aligned16(dw_taps),
                  "unreal_conv1_wgrad: buffers must be 16-byte aligned");
-  static bool configured = false;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(conv1_wgrad_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem));
-    configured = true;
-  }
+  const int rc = allow_dynamic_smem((const void*)conv1_wgrad_tcgen05_kernel, kWgSmem);
+  if (rc != UNREAL_OK) return rc;
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
-  uint64_t walls = 0;
-  if (maze_pos != nullptr) {
-    int rc = maze_walls49(&walls);
-    if (rc != UNREAL_OK) return rc;
-  }
+  const uint64_t walls = maze_pos != nullptr ? maze_walls49() : 0;
   const int items = s * 4;
   conv1_wgrad_tcgen05_kernel<<<items < 3 * sms ? items : 3 * sms, 96, kWgSmem, as_stream(stream)>>>(
       reinterpret_cast<const __nv_bfloat16*>(xpp_bf16), reinterpret_cast<const __nv_bfloat16*>(dy_planes_bf16), dw_taps,
@@ -1983,11 +1921,8 @@ static int conv2_wgrad_launch(const void* h1_bf16, const void* dy_bf16, float* d
     int rc = make_tma_nd_bf16(&td, dy_bf16, 3, dims, strides, box, 64);
     if (rc != UNREAL_OK) return rc;
   }
-  static bool configured = false;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(conv2_wgrad_tcgen05_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, W2Cfg<C>::kSmem));
-    configured = true;
-  }
+  const int rc = allow_dynamic_smem((const void*)conv2_wgrad_tcgen05_kernel<C>, W2Cfg<C>::kSmem);
+  if (rc != UNREAL_OK) return rc;
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   conv2_wgrad_tcgen05_kernel<C><<<s < 2 * sms ? s : 2 * sms, 128, W2Cfg<C>::kSmem, as_stream(stream)>>>(ta, ta2, td, dw_taps, s);
@@ -2022,11 +1957,8 @@ static int launch_deconv(const void* dy_bf16, const void* w_dtaps_bf16, void* ou
     int rc = make_tma_nd_bf16(&tw, w_dtaps_bf16, 2, dims, strides, box, 64);
     if (rc != UNREAL_OK) return rc;
   }
-  static bool configured = false;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(conv2_dgrad_tcgen05_kernel<CO, EPI, NA, PC>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDgSmem));
-    configured = true;
-  }
+  const int rc = allow_dynamic_smem((const void*)conv2_dgrad_tcgen05_kernel<CO, EPI, NA, PC>, kDgSmem);
+  if (rc != UNREAL_OK) return rc;
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   conv2_dgrad_tcgen05_kernel<CO, EPI, NA, PC><<<s < 2 * sms ? s : 2 * sms, 64 + 32 * EPI, kDgSmem, as_stream(stream)>>>(
@@ -2097,11 +2029,8 @@ extern "C" int unreal_pc_planes_conv(const void* dy_planes_bf16, const void* w_p
   UNREAL_REQUIRE(dy_planes_bf16 && w_planes_bf16 && mask_y_bf16 && out_bf16 && s > 0, "unreal_pc_planes_conv: null buffer or s <= 0");
   UNREAL_REQUIRE(aligned16(dy_planes_bf16) && aligned16(w_planes_bf16) && aligned16(mask_y_bf16) && aligned16(out_bf16),
                  "unreal_pc_planes_conv: 16-byte alignment");
-  static bool configured = false;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(pc_planes_conv_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPpSmem));
-    configured = true;
-  }
+  const int rc = allow_dynamic_smem((const void*)pc_planes_conv_tcgen05_kernel, kPpSmem);
+  if (rc != UNREAL_OK) return rc;
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   pc_planes_conv_tcgen05_kernel<<<s < 2 * sms ? s : 2 * sms, kConvThreads, kPpSmem, as_stream(stream)>>>(
@@ -2122,11 +2051,8 @@ extern "C" int unreal_pc_planes_wgrad(const void* dy_planes_bf16, const void* hp
     int rc = make_tma_nd_bf16(&th, hp_bf16, 4, dims, strides, box, 64);
     if (rc != UNREAL_OK) return rc;
   }
-  static bool configured = false;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(pc_planes_wgrad_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPwSmem));
-    configured = true;
-  }
+  const int rc = allow_dynamic_smem((const void*)pc_planes_wgrad_tcgen05_kernel, kPwSmem);
+  if (rc != UNREAL_OK) return rc;
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   pc_planes_wgrad_tcgen05_kernel<<<s < 2 * sms ? s : 2 * sms, 128, kPwSmem, as_stream(stream)>>>(

@@ -18,8 +18,6 @@
 
 namespace unreal {
 
-int maze_layout_host(MazeLayout* out);  // maze.cu
-
 namespace {
 
 constexpr int kEvalEnvs = 32;                          // envs per block: phase 1 is one warp
@@ -128,9 +126,7 @@ extern "C" int unreal_maze_eval_act(const float* pi, int a, int greedy, uint32_t
   UNREAL_REQUIRE(aligned16(lstm_c) && aligned16(lstm_h) && aligned16(fc_tab_bf16) && aligned16(xh_bf16),
                  "unreal_maze_eval_act: LSTM state, table and operand must be 16-byte aligned");
   if (n == 0) return UNREAL_OK;
-  MazeLayout L;
-  int rc = maze_layout_host(&L);
-  if (rc != UNREAL_OK) return rc;
+  const MazeLayout L = maze_layout_host();
   EvalState S{pos, last_action, last_reward, ep_score, ep_length, ep_index, active, res_score, res_length, res_finished,
               n, episodes, max_steps};
   EvalRows R{lstm_c, lstm_h, reinterpret_cast<const __nv_bfloat16*>(fc_tab_bf16), reinterpret_cast<__nv_bfloat16*>(xh_bf16),

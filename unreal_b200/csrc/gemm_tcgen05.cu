@@ -73,29 +73,6 @@ struct GemmCfg {
   static constexpr int kSmemBytes = kStages * kStageBytes + 1024 /*barriers, tmem slot*/ + kEpiBytes + 1024 /*alignment slack*/;
 };
 
-// ---- epilogue stores -------------------------------------------------------------------
-__device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, float d) {
-  asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
-}
-
-__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, uint32_t src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tma_reduce_add_2d(const CUtensorMap* m, uint32_t src, int c0, int c1) {
-  asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int kPending>
-__device__ __forceinline__ void bulk_wait_read() {
-  asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(kPending) : "memory");
-}
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
 // One accumulator tile [32 rows of this warp x BN columns]: TMEM -> registers -> bias / addend /
 // ReLU -> C.  `lead` = this work item applies bias / addend (first K split).  TMA-store path: the
 // warp stages [32 rows x 128 bytes] (64 bf16 or 32 f32 columns) in its own double-buffered,
@@ -255,8 +232,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+  const uint32_t tmem_base = tmem_base_at(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -399,8 +375,7 @@ gemm2sm_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_c
   fence_before_sync();
   cluster_sync_all();                 // both CTAs' barriers exist before any remote arrive / TMA signal
   fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+  const uint32_t tmem_base = tmem_base_at(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -512,7 +487,6 @@ static EncodeTiledFn encode_tiled() {
   return fn;
 }
 
-// row-major [rows, cols] matrix with leading dimension ld; box = [box_rows, 128 bytes], 128-byte swizzle
 int make_tma_2d(CUtensorMap* map, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f32) {
   EncodeTiledFn fn = encode_tiled();
   if (fn == nullptr) {
@@ -534,9 +508,6 @@ int make_tma_2d(CUtensorMap* map, const void* base, int64_t rows, int64_t cols, 
   return UNREAL_OK;
 }
 
-
-// rank-N tensor map, bf16 or f32 elements, swizzle 0 / 32 / 64 / 128 bytes (conv_tcgen05.cu: 4-D / 5-D im2col boxes;
-// lstm_tcgen05.cu: narrow staging boxes of the cell warps)
 int make_tma_nd(CUtensorMap* map, bool f32, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                 const uint32_t* box, int swizzle_bytes) {
   EncodeTiledFn fn = encode_tiled();
@@ -569,12 +540,9 @@ template <int BN, bool A_MN, bool B_MN, bool DEEP = false>
 static int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, const GemmArgs& g,
                        cudaStream_t st) {
   using Cfg = GemmCfg<BN, DEEP>;
-  static bool configured = false;
   auto kern = gemm_tcgen05_kernel<BN, A_MN, B_MN, DEEP>;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
-    configured = true;
-  }
+  const int rc = allow_dynamic_smem((const void*)kern, Cfg::kSmemBytes);
+  if (rc != UNREAL_OK) return rc;
   const int num_m = (g.m + kBM - 1) / kBM, num_n = (g.n + BN - 1) / BN;
   const int64_t work = (int64_t)num_m * num_n * g.split_k;
   const int sms = sm_count();
@@ -588,12 +556,9 @@ static int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUten
 template <int BN, bool A_MN, bool B_MN>
 static int launch_gemm_2sm(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, const GemmArgs& g,
                            cudaStream_t st) {
-  static bool configured = false;
   auto kern = gemm2sm_tcgen05_kernel<BN, A_MN, B_MN>;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg2<BN>::kSmemBytes));
-    configured = true;
-  }
+  const int rc = allow_dynamic_smem((const void*)kern, Cfg2<BN>::kSmemBytes);
+  if (rc != UNREAL_OK) return rc;
   const int num_m = (g.m + 2 * kBM - 1) / (2 * kBM), num_n = (g.n + BN - 1) / BN;
   const int64_t work = (int64_t)num_m * num_n * g.split_k;
   const int sms = sm_count();

@@ -40,27 +40,12 @@
 namespace unreal {
 using namespace tc05;
 
-int make_tma_2d(CUtensorMap* map, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f32);  // gemm_tcgen05.cu
-int make_tma_nd(CUtensorMap* map, bool f32, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                const uint32_t* box, int swizzle_bytes);                                                               // gemm_tcgen05.cu
-
 namespace {
 
 constexpr int kLsCellWarps = 16;
 constexpr int kLsThreads = 32 * (2 + kLsCellWarps);
 constexpr int kLsBM = 128, kLsBK = 64;
 constexpr uint32_t kLsDescHi = (1024u >> 4) | (1u << 14) | (2u << 29);   // SBO 1024 B, version 1, 128-byte swizzle
-
-// 32 lanes x 8 consecutive fp32 columns
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&r)[8]) {
-  uint32_t u[8];
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(u[0]), "=r"(u[1]), "=r"(u[2]), "=r"(u[3]), "=r"(u[4]), "=r"(u[5]), "=r"(u[6]), "=r"(u[7])
-               : "r"(taddr)
-               : "memory");
-#pragma unroll
-  for (int j = 0; j < 8; ++j) r[j] = __uint_as_float(u[j]);
-}
 
 // Branch-free activations.  What hides latency in a cell warp is instruction-level parallelism over a lane's 8 units --
 // which tanhf (a branch between its polynomial and exponential ranges) and the IEEE division (a branch to its
@@ -106,29 +91,14 @@ __device__ __forceinline__ size_t tiled_off(int row_block, int chunks_per_row, i
   return ((size_t)(row_block * chunks_per_row + chunk) * 32 + lane);        // in 16-byte chunks
 }
 
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, uint32_t src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void sts_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-__device__ __forceinline__ float4 lds_v4(uint32_t addr) {
-  float4 v;
-  asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr) : "memory");
-  return v;
-}
 // Staging tiles of one cell warp (its 32 rows x 16 units), lane = row.  f32: [32 rows x 64 B] with the 64-byte swizzle
 // (16-byte chunk j of row r at chunk j ^ ((r >> 1) & 3)); bf16: [32 rows x 32 B] with the 32-byte swizzle (chunk j at
 // j ^ ((r >> 2) & 1)).  Both are what a TMA box {16 columns, 32 rows} of that swizzle mode reads / writes, and both are
 // bank-conflict free for lane = row.  `ch` = which 8-unit half of the warp's 16 units.
 __device__ __forceinline__ void stage8f(uint32_t tile, int lane, int ch, const float (&v)[8]) {
   const uint32_t rowp = tile + (uint32_t)lane * 64u, sw = (uint32_t)((lane >> 1) & 3);
-  sts_v4(rowp + (((uint32_t)(2 * ch)) ^ sw) * 16u, __float_as_uint(v[0]), __float_as_uint(v[1]), __float_as_uint(v[2]), __float_as_uint(v[3]));
-  sts_v4(rowp + (((uint32_t)(2 * ch + 1)) ^ sw) * 16u, __float_as_uint(v[4]), __float_as_uint(v[5]), __float_as_uint(v[6]), __float_as_uint(v[7]));
+  st_shared_v4(rowp + (((uint32_t)(2 * ch)) ^ sw) * 16u, __float_as_uint(v[0]), __float_as_uint(v[1]), __float_as_uint(v[2]), __float_as_uint(v[3]));
+  st_shared_v4(rowp + (((uint32_t)(2 * ch + 1)) ^ sw) * 16u, __float_as_uint(v[4]), __float_as_uint(v[5]), __float_as_uint(v[6]), __float_as_uint(v[7]));
 }
 __device__ __forceinline__ void unstage8f(uint32_t tile, int lane, int ch, float (&v)[8]) {
   const uint32_t rowp = tile + (uint32_t)lane * 64u, sw = (uint32_t)((lane >> 1) & 3);
@@ -137,7 +107,7 @@ __device__ __forceinline__ void unstage8f(uint32_t tile, int lane, int ch, float
 }
 __device__ __forceinline__ void stage8h(uint32_t tile, int lane, int ch, const float (&v)[8]) {
   const uint4 p = pack8(v);
-  sts_v4(tile + (uint32_t)lane * 32u + (((uint32_t)ch) ^ (uint32_t)((lane >> 2) & 1)) * 16u, p.x, p.y, p.z, p.w);
+  st_shared_v4(tile + (uint32_t)lane * 32u + (((uint32_t)ch) ^ (uint32_t)((lane >> 2) & 1)) * 16u, p.x, p.y, p.z, p.w);
 }
 
 struct LstmFwdArgs {
@@ -193,8 +163,7 @@ lstm_step_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+  const uint32_t tmem_base = tmem_base_at(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -265,7 +234,7 @@ lstm_step_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __
         if (on) ld8f(g.c_prev + (g.tiled ? tiled_off(m_blk * 4 + quarter, 64, u >> 2, lane) * 4 : (size_t)row * 256 + u), c[ch], cstep);
       }
       if (g.tiled) {                         // the staging tiles are free once the previous tile's stores have read them
-        if (lane == 0) bulk_wait_read0();
+        if (lane == 0) bulk_wait_read<0>();
         __syncwarp();
       }
       mbar_wait(tfull_bar(acc), acc_phase);
@@ -401,8 +370,7 @@ lstm_step_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+  const uint32_t tmem_base = tmem_base_at(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0 && !g.skip_gemm) {
@@ -460,7 +428,7 @@ lstm_step_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __
       const int u0 = n_blk * BN + part * 16;
       if (g.tiled) {
         if (lane == 0) {
-          bulk_wait_read0();                 // the previous tile's dgates stores have read the staging tiles
+          bulk_wait_read<0>();              // the previous tile's dgates stores have read the staging tiles
           mbar_arrive_expect_tx(dh_bar(cw), 2048);
           tma_load_2d(s_dh, &tma_dh, dh_bar(cw), u0, row0);     // rows >= n arrive as zeros
         }
@@ -588,11 +556,8 @@ extern "C" int unreal_lstm_step_fwd(const void* xh, int64_t ld_xh, const void* w
     rc = make_tma_nd(&th16, false, h16_out, 2, dims, strides, box, 32);     // 32-byte rows, 32-byte swizzle
     if (rc != UNREAL_OK) return rc;
   }
-  static bool configured = false;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(lstm_step_fwd_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFwdSmem));
-    configured = true;
-  }
+  rc = allow_dynamic_smem((const void*)lstm_step_fwd_tcgen05_kernel, kFwdSmem);
+  if (rc != UNREAL_OK) return rc;
   LstmFwdArgs g{bias, c_prev, c_out, h_out, h_copy, static_cast<__nv_bfloat16*>(h16_out), static_cast<__nv_bfloat16*>(acts),
                 active, n, k, h16_ld, tiled ? 1 : 0};
   const int work = (n + kLsBM - 1) / kLsBM * 4;
@@ -630,11 +595,8 @@ extern "C" int unreal_lstm_step_bwd(const void* dgates_next, const void* wh, int
     rc = make_tma_nd(&tdg, false, dgates, 2, dims_g, strides_g, box, 32);
     if (rc != UNREAL_OK) return rc;
   }
-  static bool configured = false;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(lstm_step_bwd_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBwdSmem));
-    configured = true;
-  }
+  rc = allow_dynamic_smem((const void*)lstm_step_bwd_tcgen05_kernel, kBwdSmem);
+  if (rc != UNREAL_OK) return rc;
   LstmBwdArgs g{static_cast<const __nv_bfloat16*>(acts), c_prev, c, dh, dc, static_cast<__nv_bfloat16*>(dgates), dh2, n,
                 tiled ? 1 : 0, skip ? 1 : 0};
   const int work = (n + kLsBM - 1) / kLsBM * (256 / kBwdBN);

@@ -13,14 +13,17 @@
 //     cp.async.bulk (shared -> global), multi-buffered so patching overlaps the store.
 //   variant 2: one warp per env, same mask-built words, no shared memory or barriers.
 // The default is whichever measured fastest on B200 (profiles/, DESIGN.md).
+#include <map>
+#include <mutex>
+
 #include "common.cuh"
 #include "maze_core.cuh"
+#include "tc05.cuh"
 
 namespace unreal {
+using namespace tc05;
 
 __constant__ MazeLayout c_maze;
-static MazeLayout h_maze;
-static bool h_maze_ready = false;
 
 static const char kReferenceMap[] =
     "--+---G"
@@ -133,19 +136,6 @@ template <> struct One<uint8_t> { static __device__ __forceinline__ uint8_t v() 
 // ------------------------------------------------------------------------------------
 // variant 1: shared-memory frame templates + TMA bulk stores.
 // ------------------------------------------------------------------------------------
-__device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, uint32_t bytes) {
-  uint32_t s = (uint32_t)__cvta_generic_to_shared(ssrc);
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(s), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int kPending>
-__device__ __forceinline__ void bulk_wait_read() {
-  asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(kPending) : "memory");
-}
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
 template <typename T>
 __device__ __forceinline__ void set_agent(T* buf, int x, int y, int t, T val) {
   // t in [0,144): pixel (12x + t%12, 12y + t/12), channel 1   (_put_pixel :57-60)
@@ -175,7 +165,7 @@ __global__ void __launch_bounds__(kThreads) maze_tma_kernel(StepArgs a) {
   int drawn[kBufs];  // agent cell currently patched into buffer b (x | y<<4), -1 none
 #pragma unroll
   for (int b = 0; b < kBufs; ++b) drawn[b] = -1;
-  fence_async_smem();  // template writes must be visible to the TMA engine too
+  fence_proxy_async_smem();  // template writes must be visible to the TMA engine too
   __syncthreads();
 
   int it = 0;
@@ -198,7 +188,7 @@ __global__ void __launch_bounds__(kThreads) maze_tma_kernel(StepArgs a) {
       if (have != want && tid < 144) {
         if (have >= 0) set_agent<T>(buf, have & 15, have >> 4, tid, (T)0);
         set_agent<T>(buf, f.rx, f.ry, tid, One<T>::v());
-        fence_async_smem();  // generic-proxy writes -> visible to the async (TMA) proxy
+        fence_proxy_async_smem();  // generic-proxy writes -> visible to the async (TMA) proxy
       }
 #pragma unroll
       for (int k = 0; k < kBufs; ++k) drawn[k] = (k == b) ? want : drawn[k];
@@ -734,9 +724,49 @@ __global__ void maze_reset_kernel(int32_t* pos, int32_t* last_action, float* las
   if (last_reward) last_reward[e] = 0.f;
 }
 
+static int parse_map(const char* m, MazeLayout* out) {
+  MazeLayout L;
+  for (int y = 0; y < UNREAL_MAZE_GRID; ++y) L.wall_rows[y] = 0;
+  L.start_x = L.start_y = L.goal_x = L.goal_y = -1;
+  for (int i = 0; i < UNREAL_MAZE_GRID * UNREAL_MAZE_GRID; ++i) {
+    char c = m[i];
+    UNREAL_REQUIRE(c != 0, "maze map shorter than 49 characters");
+    int x = i % UNREAL_MAZE_GRID, y = i / UNREAL_MAZE_GRID;
+    if (c == '+') L.wall_rows[y] |= 1u << x;
+    else if (c == 'S') { L.start_x = x; L.start_y = y; }
+    else if (c == 'G') { L.goal_x = x; L.goal_y = y; }
+  }
+  UNREAL_REQUIRE(L.start_x >= 0, "maze map has no 'S' cell");
+  *out = L;
+  return UNREAL_OK;
+}
+
+// The map is process-wide and h_maze is its one copy on the host.  Each device holds its own c_maze, so a device gets
+// h_maze uploaded the first time it needs the map and again after the map changed: h_maze_gen counts the maps set,
+// g_dev_gen records the generation each device holds.  Uploads happen in the eager calls that precede a graph capture.
+static std::mutex g_maze_mu;
+static MazeLayout h_maze = [] {
+  MazeLayout L;
+  parse_map(kReferenceMap, &L);
+  return L;
+}();
+static unsigned h_maze_gen = 1;
+static std::map<int, unsigned> g_dev_gen;
+
+static int upload_map_locked() {
+  int dev = 0;
+  UNREAL_CUDA(cudaGetDevice(&dev));
+  unsigned& have = g_dev_gen[dev];
+  if (have == h_maze_gen) return UNREAL_OK;
+  UNREAL_CUDA(cudaMemcpyToSymbol(c_maze, &h_maze, sizeof(h_maze)));
+  have = h_maze_gen;
+  return UNREAL_OK;
+}
+
+// every entry point whose kernels read c_maze calls this first
 static int ensure_map() {
-  if (h_maze_ready) return UNREAL_OK;
-  return unreal_maze_set_map(nullptr);
+  std::lock_guard<std::mutex> lk(g_maze_mu);
+  return upload_map_locked();
 }
 
 template <bool kStep>
@@ -787,7 +817,8 @@ static int launch_render(const StepArgs& a, int obs_dtype, cudaStream_t st) {
     constexpr int kBufs = 2;
     size_t smem = (size_t)kBufs * kFrameElems * sizeof(float);
     auto k = maze_tma_kernel<float, kBufs, kStep>;
-    UNREAL_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int rc = allow_dynamic_smem((const void*)k, (int)smem);
+    if (rc != UNREAL_OK) return rc;
     int grid = a.n < sms ? a.n : sms;
     k<<<grid, kThreads, smem, st>>>(a);
     UNREAL_LAUNCH_CHECK("maze_tma_kernel<f32>");
@@ -795,7 +826,8 @@ static int launch_render(const StepArgs& a, int obs_dtype, cudaStream_t st) {
     constexpr int kBufs = 4;
     size_t smem = (size_t)kBufs * kFrameElems * sizeof(uint8_t);
     auto k = maze_tma_kernel<uint8_t, kBufs, kStep>;
-    UNREAL_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int rc = allow_dynamic_smem((const void*)k, (int)smem);
+    if (rc != UNREAL_OK) return rc;
     int per_sm = get_tunable("maze_u8_ctas_per_sm", 2);
     int grid = a.n < sms * per_sm ? a.n : sms * per_sm;
     k<<<grid, kThreads, smem, st>>>(a);
@@ -809,56 +841,39 @@ static int launch_render(const StepArgs& a, int obs_dtype, cudaStream_t st) {
 using namespace unreal;
 
 extern "C" int unreal_maze_set_map(const char* map49_host) {
-  const char* m = map49_host ? map49_host : kReferenceMap;
   MazeLayout L;
-  for (int y = 0; y < UNREAL_MAZE_GRID; ++y) L.wall_rows[y] = 0;
-  L.start_x = L.start_y = L.goal_x = L.goal_y = -1;
-  for (int i = 0; i < UNREAL_MAZE_GRID * UNREAL_MAZE_GRID; ++i) {
-    char c = m[i];
-    UNREAL_REQUIRE(c != 0, "maze map shorter than 49 characters");
-    int x = i % UNREAL_MAZE_GRID, y = i / UNREAL_MAZE_GRID;
-    if (c == '+') L.wall_rows[y] |= 1u << x;
-    else if (c == 'S') { L.start_x = x; L.start_y = y; }
-    else if (c == 'G') { L.goal_x = x; L.goal_y = y; }
-  }
-  UNREAL_REQUIRE(L.start_x >= 0, "maze map has no 'S' cell");
-  UNREAL_CUDA(cudaMemcpyToSymbol(c_maze, &L, sizeof(L)));
+  int rc = parse_map(map49_host ? map49_host : kReferenceMap, &L);
+  if (rc != UNREAL_OK) return rc;
+  std::lock_guard<std::mutex> lk(g_maze_mu);
   h_maze = L;
-  h_maze_ready = true;
-  return UNREAL_OK;
+  ++h_maze_gen;
+  return upload_map_locked();
 }
 
 namespace unreal {
-// the 7x7 wall map as 49 bits (bit cy*7 + cx), for the render-fused conv1 kernels in conv_tcgen05.cu
-int maze_walls49(uint64_t* out) {
-  if (!h_maze_ready) {
-    int rc = unreal_maze_set_map(nullptr);
-    if (rc != UNREAL_OK) return rc;
-  }
-  uint64_t w = 0;
-  for (int cy = 0; cy < UNREAL_MAZE_GRID; ++cy) w |= (uint64_t)(h_maze.wall_rows[cy] & 0x7fu) << (7 * cy);
-  *out = w;
-  return UNREAL_OK;
+MazeLayout maze_layout_host() {
+  std::lock_guard<std::mutex> lk(g_maze_mu);
+  return h_maze;
 }
 
-// the layout K1 steps with (the host copy of c_maze), for kernels of other translation units (evaluate.cu)
-int maze_layout_host(MazeLayout* out) {
-  int rc = ensure_map();
-  if (rc != UNREAL_OK) return rc;
-  *out = h_maze;
-  return UNREAL_OK;
+uint64_t maze_walls49() {
+  const MazeLayout L = maze_layout_host();
+  uint64_t w = 0;
+  for (int cy = 0; cy < UNREAL_MAZE_GRID; ++cy) w |= (uint64_t)(L.wall_rows[cy] & 0x7fu) << (7 * cy);
+  return w;
 }
 }  // namespace unreal
 
 extern "C" int unreal_maze_get_layout(int* sx, int* sy, int* gx, int* gy, uint8_t* walls49_host) {
   int rc = ensure_map();
   if (rc) return rc;
-  if (sx) *sx = h_maze.start_x;
-  if (sy) *sy = h_maze.start_y;
-  if (gx) *gx = h_maze.goal_x;
-  if (gy) *gy = h_maze.goal_y;
+  const MazeLayout L = maze_layout_host();
+  if (sx) *sx = L.start_x;
+  if (sy) *sy = L.start_y;
+  if (gx) *gx = L.goal_x;
+  if (gy) *gy = L.goal_y;
   if (walls49_host)
-    for (int i = 0; i < 49; ++i) walls49_host[i] = (h_maze.wall_rows[i / 7] >> (i % 7)) & 1u;
+    for (int i = 0; i < 49; ++i) walls49_host[i] = (L.wall_rows[i / 7] >> (i % 7)) & 1u;
   return UNREAL_OK;
 }
 

@@ -10,6 +10,11 @@ struct MazeLayout {
   int32_t start_x, start_y, goal_x, goal_y;
 };
 
+// Host copies of the process-wide map (maze.cu) for kernels of other translation units: the layout K1 steps with
+// (evaluate.cu), and its walls as 49 bits, bit cy*7 + cx (the render-fused conv1 kernels of conv_tcgen05.cu).
+MazeLayout maze_layout_host();
+uint64_t maze_walls49();
+
 struct MazeStep {
   int x1, y1;     // cell after the move (before any reset)
   int reward;     // +1 goal, -1 hit, 0 otherwise

@@ -1203,12 +1203,9 @@ extern "C" int unreal_cell_segment_sum(const void* dy, int dy_dtype, const int32
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   constexpr int kSmem = 49 * 256 * 4;
-  static bool configured = false;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(cell_segment_sum_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem));
-    UNREAL_CUDA(cudaFuncSetAttribute(cell_segment_sum_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem));
-    configured = true;
-  }
+  int rc = allow_dynamic_smem((const void*)cell_segment_sum_kernel<float>, kSmem);
+  if (rc == UNREAL_OK) rc = allow_dynamic_smem((const void*)cell_segment_sum_kernel<__nv_bfloat16>, kSmem);
+  if (rc != UNREAL_OK) return rc;
   int64_t ctas = (int64_t)sms * 4;
   if (ctas > (s + 63) / 64) ctas = (s + 63) / 64;
   const int64_t rows_per_cta = (s + ctas - 1) / ctas;

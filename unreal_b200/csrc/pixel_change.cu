@@ -14,10 +14,6 @@
 
 namespace unreal {
 
-// pixel_change84.cu: HBM-rate path for 84x84x3 frames; -100 = not applicable
-int pixel_change84(const void* p0, int64_t stride0, const void* p1, int64_t stride1, int dtype, float* pc,
-                   int sequences, int l, cudaStream_t st);
-
 constexpr int kMaxCellsPerCta = 64;  // 4 rows x 256 pixels = 1024 threads
 
 template <typename T> struct Px;

@@ -118,8 +118,7 @@ __global__ void __launch_bounds__(Pc84<T, PR>::kThreads) pixel_change84_kernel(c
     const uint8_t* src = frame + (2 + 4 * PR * part) * P::kRowBytes - P::kLead;
     const uint32_t bar = bar0 + 8u * (k % 3);
     mbar_arrive_expect_tx(bar, P::kCopyBytes);
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(base + (uint32_t)(k % 3) * P::kBufBytes), "l"(src), "r"(P::kCopyBytes), "r"(bar) : "memory");
+    bulk_load(base + (uint32_t)(k % 3) * P::kBufBytes, src, P::kCopyBytes, bar);
   };
   if (tid == 0) {
     if (total > 0) issue(0);
@@ -295,8 +294,7 @@ __global__ void __launch_bounds__(Pc84U8::kThreads, 1) pixel_change84_u8_kernel(
         const uint8_t* src = frame + 2 * P::kRowBytes - P::kLead;
         const uint32_t bar = full0 + 8u * b;
         mbar_arrive_expect_tx(bar, P::kCopyBytes);
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"(base + (uint32_t)b * P::kBufBytes), "l"(src), "r"(P::kCopyBytes), "r"(bar) : "memory");
+        bulk_load(base + (uint32_t)b * P::kBufBytes, src, P::kCopyBytes, bar);
       }
     }
     return;
@@ -332,12 +330,9 @@ __global__ void __launch_bounds__(Pc84U8::kThreads, 1) pixel_change84_u8_kernel(
 template <int kXuBytes>
 static int launch84_u8(const Pc84Args& g, cudaStream_t st) {
   using P = Pc84U8;
-  static bool configured = false;
   auto kern = pixel_change84_u8_kernel<kXuBytes>;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, P::kSmem));
-    configured = true;
-  }
+  const int rc = allow_dynamic_smem((const void*)kern, P::kSmem);
+  if (rc != UNREAL_OK) return rc;
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   const int grid = g.sequences < sms ? g.sequences : sms;
@@ -383,12 +378,9 @@ __global__ void selfcheck_arith_kernel(unsigned long long* out, uint32_t mg) {
 template <typename T, int PR>
 static int launch84(const Pc84Args& g, cudaStream_t st) {
   using P = Pc84<T, PR>;
-  static bool configured = false;
   auto kern = pixel_change84_kernel<T, PR>;
-  if (!configured) {
-    UNREAL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, P::kSmem));
-    configured = true;
-  }
+  const int rc = allow_dynamic_smem((const void*)kern, P::kSmem);
+  if (rc != UNREAL_OK) return rc;
   const int sms = sm_count();
   if (sms <= 0) return UNREAL_ECUDA;
   const int per_sm = (227 * 1024) / (P::kSmem + 1024);

@@ -1,5 +1,6 @@
-// Thin inline-PTX layer for the sm_100a tensor path: mbarrier, TMA (cp.async.bulk.tensor),
-// tcgen05 (alloc / mma / commit / ld) and the UMMA shared-memory / instruction descriptors.
+// Thin inline-PTX layer for the sm_100a kernels: mbarrier, TMA (cp.async.bulk.tensor) and plain bulk copies,
+// tcgen05 (alloc / mma / commit / ld), the UMMA shared-memory / instruction descriptors and the vector shared /
+// global accesses of the epilogues.  Every inline asm statement of the library lives here; the .cu files call these.
 // Bit layouts follow the PTX ISA "tcgen05" chapter (matrix descriptor: start address, leading /
 // stride byte offsets in 16-byte units, version 1, swizzle mode in bits 61-63; instruction
 // descriptor for .kind::f16: D format bits 4-5, A/B format bits 7-9/10-12, A/B major bits 15/16,
@@ -61,6 +62,58 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* m, 
       ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
       : "memory");
 }
+__device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2, int c3) {
+  asm volatile(
+      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
+      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+      : "memory");
+}
+// shared -> global tile stores / reductions, completion tracked by bulk groups (bulk_commit / bulk_wait_*)
+__device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, uint32_t src, int c0, int c1) {
+  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
+               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src), "r"(c0), "r"(c1) : "memory");
+}
+__device__ __forceinline__ void tma_store_3d(const CUtensorMap* m, uint32_t src, int c0, int c1, int c2) {
+  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
+               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src), "r"(c0), "r"(c1), "r"(c2) : "memory");
+}
+__device__ __forceinline__ void tma_reduce_add_2d(const CUtensorMap* m, uint32_t src, int c0, int c1) {
+  asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3}], [%1];"
+               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src), "r"(c0), "r"(c1) : "memory");
+}
+
+// ---- plain bulk copies (cp.async.bulk, no tensor map) ------------------------------------
+// `bytes` contiguous bytes global -> shared, completion counted in bytes on `bar`
+__device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
+}
+// `bytes` contiguous bytes shared -> global, in the current bulk group
+__device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, uint32_t bytes) {
+  uint32_t s = (uint32_t)__cvta_generic_to_shared(ssrc);
+  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(s), "r"(bytes)
+               : "memory");
+}
+__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// until at most kPending committed groups still read their shared-memory source
+template <int kPending>
+__device__ __forceinline__ void bulk_wait_read() {
+  asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(kPending) : "memory");
+}
+__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+
+// ---- vector accesses -------------------------------------------------------------------
+__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
+  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
+}
+__device__ __forceinline__ float4 lds_v4(uint32_t addr) {
+  float4 v;
+  asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr) : "memory");
+  return v;
+}
+__device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, float d) {
+  asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
+}
 
 // ---- tcgen05 ---------------------------------------------------------------------------
 __device__ __forceinline__ void fence_before_sync() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
@@ -73,6 +126,12 @@ __device__ __forceinline__ void tmem_alloc(uint32_t slot) {
   static_assert(kCols >= 32 && kCols <= 512 && (kCols & (kCols - 1)) == 0, "TMEM columns: power of two in [32,512]");
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot), "n"(kCols) : "memory");
   asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+// the base address tmem_alloc / tmem_alloc_2sm wrote to `slot`, read once the allocation is published to the CTA
+__device__ __forceinline__ uint32_t tmem_base_at(uint32_t slot) {
+  uint32_t base;
+  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(base) : "r"(slot));
+  return base;
 }
 template <int kCols>
 __device__ __forceinline__ void tmem_dealloc(uint32_t base) {
@@ -131,6 +190,16 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* r) {
         "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
       : "r"(taddr)
       : "memory");
+}
+// 32 lanes x 8 consecutive fp32 columns
+__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&r)[8]) {
+  uint32_t u[8];
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+               : "=r"(u[0]), "=r"(u[1]), "=r"(u[2]), "=r"(u[3]), "=r"(u[4]), "=r"(u[5]), "=r"(u[6]), "=r"(u[7])
+               : "r"(taddr)
+               : "memory");
+#pragma unroll
+  for (int j = 0; j < 8; ++j) r[j] = __uint_as_float(u[j]);
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
@@ -224,4 +293,14 @@ __device__ __forceinline__ void mma_commit_2sm(uint32_t bar, uint16_t cta_mask) 
 }
 
 }  // namespace tc05
+
+// ---- host: tensor maps for the TMA loads / stores above (gemm_tcgen05.cu) --------------------
+// row-major [rows, cols] matrix with leading dimension ld; box = [box_rows, 128 bytes], 128-byte swizzle
+int make_tma_2d(CUtensorMap* map, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f32);
+// rank-N tensor map, bf16 or f32 elements, swizzle 0 / 32 / 64 / 128 bytes
+int make_tma_nd(CUtensorMap* map, bool f32, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
+                const uint32_t* box, int swizzle_bytes);
+int make_tma_nd_bf16(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
+                     const uint32_t* box, int swizzle_bytes);
+
 }  // namespace unreal
