@@ -12,7 +12,8 @@
  *   - every function returns UNREAL_OK (0) or a negative UNREAL_E* code and never throws;
  *     unreal_last_error() returns a thread-local message for the last failure.
  *   - all array arguments are caller-owned DEVICE pointers (e.g. torch.Tensor.data_ptr())
- *     unless the name ends in _host; "nullable" arguments may be NULL.
+ *     unless the name ends in _host (pinned host memory where the function says so); "nullable"
+ *     arguments may be NULL.
  *   - functions only enqueue work on `stream` (a cudaStream_t passed as void*, NULL = the
  *     legacy default stream); they do not synchronise, allocate, or keep caller pointers.
  *     The only library-owned memory is what *_create() returns handles to.
@@ -223,6 +224,32 @@ int unreal_rows_select(void* out, const void* src, const int64_t* idx, const uin
  * all seq_len), zeros beyond and for start[e] < 0.  out is [L,N,item] when time_major else [N,L,item]. */
 int unreal_replay_gather(unreal_replay_t* r, const void* payload, long long item_bytes, const int32_t* start,
                          const int32_t* len /*nullable*/, int seq_len, int time_major, void* out, void* stream);
+
+/* ---- host simulators (HostEnvProducer, environment/frame_environment.py) -----------------------------------------
+ * What BatchedFrameEnvironment.process does after N host envs (lab / gym / indoor, environment/{lab,gym,indoor}
+ * _environment.py process() / reset()) have stepped, in one launch.  Replaces, per env: the upload of the new frame
+ * (lab_environment.py:99-102 `image / 255.0` inverted), Environment._calc_pixel_change (environment.py:93-99), the
+ * record of the step, the `if terminal: reset()` of trainer.py:201-202 and the last_action / last_reward of
+ * indoor_environment.py:117-139 / lab_environment.py:120-131.
+ * The *_host arguments are PINNED HOST memory (cudaHostAlloc, torch pin_memory), read in place by the kernel; the
+ * caller must not rewrite them until the launch has completed.  Staging frames are [N,H,W,C] of stage_dtype:
+ * UNREAL_U8 as is, or UNREAL_F32 in [0,1] converted to u8 as rint(double(x) * 255) (round half to even) clipped to
+ * [0,255] -- finite values only.  Frame buffers 16-byte aligned; H, W, C as unreal_pixel_change.
+ * mode 0, step (rows e with active[e] != 0, active NULL: all):
+ *   out[e] <- step frame (inactive: prev[e] when copy_inactive, else untouched); pc[e] <- K2 over (out[e], prev[e]) for
+ *   EVERY row; reward / terminal <- step_*_host (0 for inactive); rec as unreal_frame_pack with the last_action /
+ *   last_reward from before the step; terminal active rows: out[e] <- reset frame, objective[e] <- reset objective,
+ *   last_action / last_reward <- 0; other active rows: objective[e] <- step objective, last_* <- action / reward.
+ * mode 1, reset (rows with active[e] != 0, NULL: all): out[e] <- reset frame, objective[e] <- reset objective,
+ *   last_action / last_reward (nullable) <- 0; the step arguments may be NULL.
+ * Objective arrays [N,G] f32 (G = 0: all NULL).  Only the rows a mode needs are read from the staging. */
+int unreal_host_frames_ingest(int mode, const void* step_frames_host, const void* reset_frames_host, int stage_dtype,
+                              const float* step_reward_host, const uint8_t* step_terminal_host,
+                              const float* step_objective_host, const float* reset_objective_host,
+                              const int32_t* action, const uint8_t* active /*nullable*/, const uint8_t* prev,
+                              uint8_t* out, int copy_inactive, float* pc, uint64_t* rec, float* reward,
+                              uint8_t* terminal, int32_t* last_action, float* last_reward, float* objective, int n,
+                              int h, int w, int c, int g, void* stream);
 
 /* ---- rollout bookkeeping (Trainer._process_base, trainer.py:228-296), fused ------------------------------------
  * unreal_rollout_lar: ExperienceFrame.concat_action_and_reward (experience.py:34-46) for every env:

@@ -71,6 +71,8 @@ SIGNATURES = {
     "unreal_ring_store": (c_int, [P, P, P, c_int, c_int, c_int64, P]),
     "unreal_rows_select": (c_int, [P, P, P, P, c_int, c_int64, P]),
     "unreal_replay_gather": (c_int, [c_void_p, P, c_int64, P, P, c_int, c_int, P, P]),
+    "unreal_host_frames_ingest": (c_int, [c_int, P, P, c_int, P, P, P, P, P, P, P, P, c_int, P, P, P, P, P, P, P,
+                                          c_int, c_int, c_int, c_int, c_int, P]),
     "unreal_rollout_lar": (c_int, [P, P, P, c_int, c_int, c_int, P, P]),
     "unreal_rollout_post": (c_int, [P, P, P, c_int, P, P, P, P, P, P, P, P]),
     "unreal_maze_eval_act": (c_int, [P, c_int, c_int, P, P, P, P, P, P, P, P, P, P, P, P, c_int, c_int, P, P, P, P, c_int64,
@@ -184,6 +186,19 @@ def ptr(t, dtype=None, name="tensor"):
   if not t.is_contiguous():
     raise UnrealError("%s must be contiguous" % name)
   if dtype is not None and t.dtype != dtype:
+    raise UnrealError("%s must be %s, got %s" % (name, dtype, t.dtype))
+  return t.data_ptr()
+
+
+def host_ptr(t, dtype, name="tensor"):
+  """data_ptr of a contiguous pinned host tensor (None -> NULL), with dtype check."""
+  if t is None:
+    return None
+  if not isinstance(t, torch.Tensor) or t.is_cuda or not t.is_pinned():
+    raise UnrealError("%s must be a pinned host tensor" % name)
+  if not t.is_contiguous():
+    raise UnrealError("%s must be contiguous" % name)
+  if t.dtype != dtype:
     raise UnrealError("%s must be %s, got %s" % (name, dtype, t.dtype))
   return t.data_ptr()
 

@@ -15,7 +15,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libunreal_b200.so")
 
-SOURCES = ["api.cu", "maze.cu", "returns.cu", "rng.cu", "pixel_change.cu", "pixel_change84.cu", "replay.cu", "rmsprop.cu", "gemm_tcgen05.cu", "model_ops.cu", "conv_tcgen05.cu", "lstm_tcgen05.cu", "rollout_ops.cu", "evaluate.cu"]
+SOURCES = ["api.cu", "maze.cu", "returns.cu", "rng.cu", "pixel_change.cu", "pixel_change84.cu", "replay.cu", "rmsprop.cu", "gemm_tcgen05.cu", "model_ops.cu", "conv_tcgen05.cu", "lstm_tcgen05.cu", "rollout_ops.cu", "evaluate.cu", "host_ingest.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -63,6 +63,11 @@ UNREAL_HD uint64_t frame_pack(int x0, int y0, int x1, int y1, int action, int re
   r |= (uint64_t)((uint8_t)(int8_t)last_reward) << 48;
   return r;
 }
+// the record of a generic-frame env step (no cells): rewards stored as their sign
+UNREAL_HD uint64_t framed_record(int action, float reward, int terminal, int last_action, float last_reward) {
+  return frame_pack(0, 0, 0, 0, action, (reward > 0.f) - (reward < 0.f), terminal, last_action,
+                    (last_reward > 0.f) - (last_reward < 0.f));
+}
 UNREAL_HD int frame_valid(uint64_t r) { return (int)((r >> 39) & 1); }
 UNREAL_HD int frame_terminal(uint64_t r) { return (int)((r >> 32) & 1); }
 UNREAL_HD int frame_reward(uint64_t r) { return (int)(int8_t)((r >> 24) & 255); }

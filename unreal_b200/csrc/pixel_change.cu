@@ -10,35 +10,9 @@
 // frames give bit-identical maps to the reference's float32 evaluation.
 // The stream form walks L+1 consecutive frames of a sequence with the previous frame's pixel
 // held in registers: every frame is read from HBM exactly once.
-#include "common.cuh"
+#include "pixel_change_core.cuh"
 
 namespace unreal {
-
-constexpr int kMaxCellsPerCta = 64;  // 4 rows x 256 pixels = 1024 threads
-
-template <typename T> struct Px;
-template <> struct Px<float> { static __device__ __forceinline__ float load(const float* p) { return __ldcs(p); } };
-template <> struct Px<uint8_t> {
-  // frames arrive as uint8 and are scaled by /255 like lab_environment.py:99-102
-  static __device__ __forceinline__ float load(const uint8_t* p) { return __fdiv_rn((float)__ldcs(p), 255.0f); }
-};
-
-// |a-b| channel mean of one pixel, numpy order: ((d0 + d1) + d2) / C
-template <int C>
-__device__ __forceinline__ float pixel_mean(const float (&a)[C], const float (&b)[C]) {
-  float s = fabsf(__fsub_rn(a[0], b[0]));
-#pragma unroll
-  for (int c = 1; c < C; ++c) s = __fadd_rn(s, fabsf(__fsub_rn(a[c], b[c])));
-  return __fdiv_rn(s, (float)C);
-}
-
-// after this every lane with (px & 3) == 0 holds the mean of its 4-pixel cell row
-__device__ __forceinline__ float cell_row_mean(float m) {
-  float v1 = __shfl_down_sync(0xffffffffu, m, 1);
-  float v2 = __shfl_down_sync(0xffffffffu, m, 2);
-  float v3 = __shfl_down_sync(0xffffffffu, m, 3);
-  return __fmul_rn(__fadd_rn(__fadd_rn(__fadd_rn(m, v1), v2), v3), 0.25f);
-}
 
 // grid: (frames-or-sequences x pool rows, column tiles); block: 4 rows x 4*cells pixels, rounded
 // up to whole warps (the padding threads only take part in the shuffles)
@@ -50,33 +24,20 @@ __global__ void __launch_bounds__(1024) pixel_change_kernel(const T* __restrict_
   const size_t m = blockIdx.x / ph;               // frame (or sequence)
   const int i = blockIdx.x - (int)m * ph;         // pool row
   const int j0 = blockIdx.y * kMaxCellsPerCta;    // first cell of this tile
-  const int cells = min(kMaxCellsPerCta, pw - j0);
-  const int tile_px = cells * 4;
-  const bool live = threadIdx.x < 4 * tile_px;
-  const int r = live ? threadIdx.x / tile_px : 0;  // pixel row inside the pool row, 0..3
-  const int p = threadIdx.x - r * tile_px;        // pixel inside the tile
   const size_t frame_elems = (size_t)H * W * C;
-  const size_t off = ((size_t)(4 * i + 2 + r) * W + (size_t)(4 * j0 + 2 + p)) * C;
-  float a[C], b[C];
-#pragma unroll
-  for (int c = 0; c < C; ++c) a[c] = b[c] = 0.f;
   if (!kStream) {
-    if (live) {
-#pragma unroll
-      for (int c = 0; c < C; ++c) {
-        a[c] = Px<T>::load(cur_or_frames + m * frame_elems + off + c);
-        b[c] = Px<T>::load(prev + m * frame_elems + off + c);
-      }
-    }
-    float row = cell_row_mean(pixel_mean<C>(a, b));
-    if (live && (p & 3) == 0) s_rows[r][p >> 2] = row;
-    __syncthreads();
-    if (threadIdx.x < cells) {
-      const int j = threadIdx.x;
-      float v = __fadd_rn(__fadd_rn(__fadd_rn(s_rows[0][j], s_rows[1][j]), s_rows[2][j]), s_rows[3][j]);
-      pc[(m * ph + i) * pw + j0 + j] = __fmul_rn(v, 0.25f);
-    }
+    pool_row_change<T, C>(cur_or_frames + m * frame_elems, prev + m * frame_elems, pc + (m * ph + i) * pw, W, i, j0, pw,
+                          s_rows);
   } else {
+    const int cells = min(kMaxCellsPerCta, pw - j0);
+    const int tile_px = cells * 4;
+    const bool live = threadIdx.x < 4 * tile_px;
+    const int r = live ? threadIdx.x / tile_px : 0;  // pixel row inside the pool row, 0..3
+    const int p = threadIdx.x - r * tile_px;        // pixel inside the tile
+    const size_t off = ((size_t)(4 * i + 2 + r) * W + (size_t)(4 * j0 + 2 + p)) * C;
+    float a[C], b[C];
+#pragma unroll
+    for (int c = 0; c < C; ++c) a[c] = b[c] = 0.f;
     const T* seq = cur_or_frames + m * (size_t)(L + 1) * frame_elems + off;
     float nx[C];
 #pragma unroll
@@ -113,9 +74,8 @@ template <typename T, bool kStream>
 static int launch_c(const void* x, const void* y, float* pc, int m, int l, int h, int w, int c, cudaStream_t st) {
   const int ph = (h - 4) / 4, pw = (w - 4) / 4;
   const int tiles = (pw + kMaxCellsPerCta - 1) / kMaxCellsPerCta;
-  const int cells = pw < kMaxCellsPerCta ? pw : kMaxCellsPerCta;
   // every tile but the last is full; the last may be narrower: size the block for the widest
-  dim3 grid((unsigned)((size_t)m * ph), tiles), block((16 * cells + 31) / 32 * 32);
+  dim3 grid((unsigned)((size_t)m * ph), tiles), block(pool_row_threads(w));
   UNREAL_REQUIRE(tiles == 1 || pw % kMaxCellsPerCta == 0,
                  "unreal_pixel_change: frames wider than 260 px need (W-4)/4 to be a multiple of 64");
   const T* a = static_cast<const T*>(x);

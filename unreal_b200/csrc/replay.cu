@@ -182,9 +182,8 @@ __global__ void frame_pack_kernel(const int32_t* __restrict__ action, const floa
   int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= n) return;
   if (active && !active[e]) { rec[e] = 0ull; return; }
-  const float r = reward[e], lr = last_reward ? last_reward[e] : 0.f;
-  rec[e] = frame_pack(0, 0, 0, 0, action[e], (r > 0.f) - (r < 0.f), terminal[e], last_action ? last_action[e] : 0,
-                      (lr > 0.f) - (lr < 0.f));
+  rec[e] = framed_record(action[e], reward[e], terminal[e], last_action ? last_action[e] : 0,
+                         last_reward ? last_reward[e] : 0.f);
 }
 
 // payload[e, slot[e], :] <- src[e, :]; one CTA per env walks the item in W-sized words

@@ -12,8 +12,13 @@ around the simulator call:
 
 Frames are uint8 [N,H,W,3] on the device (1 = 255, the reference's `image / 255.0` preprocessing is
 applied on load by K2 and by the network's frame kernel); 21 168 B per 84x84 frame instead of the
-reference's 84 672 B float32 state.
+reference's 84 672 B float32 state.  Host simulators that return float32 frames are staged as float32
+and converted to uint8 on the device by the ingest kernel (HostEnvProducer).
 """
+import queue
+import threading
+import weakref
+
 import numpy as np
 import torch
 
@@ -42,10 +47,6 @@ class FrameProducer(object):
 
   def step(self, action, active, out, reward, terminal, objective=None):
     raise NotImplementedError
-
-
-def _rows(mask, like):
-  return mask.to(torch.bool).view(-1, *([1] * (like.dim() - 1)))
 
 
 class TableFrameProducer(FrameProducer):
@@ -139,66 +140,199 @@ class RandomFrameProducer(FrameProducer):
     terminal.copy_(done.to(torch.uint8))
 
 
+class _EnvThreads(object):
+  """k long-lived daemon threads; thread i owns the envs [lo_i, hi_i) for its whole life, so a simulator object is only
+  ever called from one thread.  `run(job)` hands every thread job(lo, hi) and returns what each returned, in order."""
+
+  def __init__(self, n, k):
+    self.slices = [(i * n // k, (i + 1) * n // k) for i in range(k)]
+    self._jobs = [queue.SimpleQueue() for _ in range(k)]
+    self._done = [queue.SimpleQueue() for _ in range(k)]
+    self._threads = [threading.Thread(target=_env_thread, args=(self._jobs[i], self._done[i], lo, hi), daemon=True,
+                                      name="unreal-env-%d" % i) for i, (lo, hi) in enumerate(self.slices)]
+    for t in self._threads:
+      t.start()
+    self._finalizer = weakref.finalize(self, _EnvThreads._stop, self._jobs)
+    self._finalizer.atexit = False      # daemon threads end with the interpreter; never join one stuck in an env
+
+  @staticmethod
+  def _stop(jobs):
+    for q in jobs:
+      q.put(None)
+
+  def run(self, job):
+    for q in self._jobs:
+      q.put(job)
+    return [d.get() for d in self._done]
+
+  def close(self):
+    self._finalizer()
+    for t in self._threads:
+      t.join()
+
+
+def _env_thread(jobs, done, lo, hi):
+  while True:
+    job = jobs.get()
+    if job is None:
+      return
+    done.put(job(lo, hi))
+    job = None          # a finished job keeps no reference to its producer
+
+
 class HostEnvProducer(FrameProducer):
   """N reference-style env objects on the host (anything with the Environment instance contract of
   environment.py:76-86: `process(action) -> (state, reward, terminal, pixel_change)`, `reset()`,
-  `last_state['image']` as float [0,1] or uint8 [H,W,3]) feeding the device path: actions come back
-  to the host once per step, frames go up through one pinned staging buffer.  The envs' own
-  pixel_change is ignored -- the adapter recomputes it on the device (K2) from the same two frames."""
+  `last_state['image']` as float [0,1] or uint8 [H,W,3]) feeding the device path.
 
-  def __init__(self, envs, device, action_size, objective_size=0, frame_shape=(84, 84, 3)):
+  `workers=1` calls every env from the calling thread (simulators bound to a thread, such as GL contexts, keep
+  working); `workers=k` starts k daemon threads, each owning a fixed contiguous slice of the envs, which step their
+  envs concurrently (the reference's lab / gym envs block in a Pipe `recv()`, which releases the GIL).  An env whose
+  step is terminal is reset by its thread right away (trainer.py:201-202).  The threads write frames, rewards,
+  terminals and objectives into pinned staging, and one kernel (unreal_host_frames_ingest) reads it in place and does
+  everything the adapter does around the simulator call.  Per step the action (and the active mask) come back to the
+  host once; nothing is uploaded.  Staging holds frames as the envs produce them: uint8, or float32 for float frames
+  (float64 frames are rounded to float32 on the way in), fixed by the first env's first frame (its `last_state`
+  after construction).  The envs' own pixel_change is
+  ignored -- the kernel recomputes it from the same two frames (K2).
+
+  A failing env call raises UnrealError naming the env, after every thread has stopped writing; the producer then
+  refuses further calls.  `close()` (BatchedFrameEnvironment.stop()) ends the threads."""
+
+  def __init__(self, envs, device, action_size, objective_size=0, frame_shape=(84, 84, 3), workers=1):
     self.envs = list(envs)
-    self.num_envs = len(self.envs)
+    self.num_envs = n = len(self.envs)
     self.device = torch.device(device)
     self.action_size = int(action_size)
-    self.objective_size = int(objective_size)
+    self.objective_size = g = int(objective_size)
     self.frame_shape = tuple(frame_shape)
-    n = self.num_envs
-    self._stage = torch.empty(n, *self.frame_shape, dtype=torch.uint8).pin_memory()
-    self._rt = torch.zeros(n, 2, dtype=torch.float32).pin_memory()
-    self._obj = torch.zeros(n, max(1, self.objective_size), dtype=torch.float32).pin_memory()
+    first = getattr(self.envs[0], 'last_state', None) if n else None
+    if first is None or 'image' not in first:
+      raise _lib.UnrealError("HostEnvProducer: env 0 has no last_state['image'] after construction; its first frame "
+                             "fixes the staging dtype")
+    self.stage_dtype = torch.uint8 if np.asarray(first['image']).dtype == np.uint8 else torch.float32
+    pin = lambda *shape, dtype=torch.float32: torch.zeros(*shape, dtype=dtype).pin_memory()  # noqa: E731
+    self._step_frames = pin(n, *self.frame_shape, dtype=self.stage_dtype)
+    self._reset_frames = pin(n, *self.frame_shape, dtype=self.stage_dtype)
+    self._reward = pin(n)
+    self._terminal = pin(n, dtype=torch.uint8)
+    self._step_obj = pin(n, max(1, g))
+    self._reset_obj = pin(n, max(1, g))
+    self._action = pin(n, dtype=torch.int32)
+    self._mask = pin(n, dtype=torch.uint8)
+    self._np = {k: getattr(self, '_' + k).numpy() for k in ('step_frames', 'reset_frames', 'reward', 'terminal',
+                                                            'step_obj', 'reset_obj', 'action', 'mask')}
+    self._copied = torch.cuda.Event()       # the action / mask read-back has landed
+    self._ingested = torch.cuda.Event()     # the last ingest has read the staging
+    self._failed = None
+    k = max(1, min(int(workers), n))
+    self._threads = _EnvThreads(n, k) if k > 1 else None
+    self.workers = k
 
   @staticmethod
   def _u8(image):
+    """The host twin of the kernel's float conversion (the inverse of `image / 255.0`)."""
     a = np.asarray(image)
     if a.dtype == np.uint8:
       return a
-    return np.rint(a.astype(np.float64) * 255.0).clip(0, 255).astype(np.uint8)   # inverse of `image / 255.0`
+    return np.rint(a.astype(np.float64) * 255.0).clip(0, 255).astype(np.uint8)
 
-  def _put(self, e, state):
-    self._stage[e].copy_(torch.from_numpy(np.ascontiguousarray(self._u8(state['image']))))
+  def close(self):
+    if self._threads is not None:
+      self._threads.close()
+      self._threads = None
+
+  # ---- host side: runs on the env's own thread -------------------------------------------------------------------
+  def _put(self, frames, obj, e, state):
+    img = np.asarray(state['image'])
+    if (img.dtype == np.uint8) != (self.stage_dtype == torch.uint8):
+      raise _lib.UnrealError("env %d produced a %s frame; the staging holds %s frames (fixed by env 0's first frame)"
+                             % (e, img.dtype, self.stage_dtype))
+    if img.shape != self.frame_shape:
+      raise _lib.UnrealError("env %d produced a frame of shape %s, not %s" % (e, img.shape, self.frame_shape))
+    frames[e] = img
     if self.objective_size:
-      self._obj[e, :self.objective_size] = torch.as_tensor(np.asarray(state['objective'], dtype=np.float32))
+      obj[e, :self.objective_size] = np.asarray(state['objective'], dtype=np.float32)
 
-  def _upload(self, mask_host, out, objective):
-    m = torch.from_numpy(mask_host).to(self.device)
-    K.rows_select(out, self._stage.to(self.device, non_blocking=True), None, m)
-    if objective is not None and self.objective_size:
-      fresh = self._obj[:, :self.objective_size].to(self.device, non_blocking=True)
-      objective.copy_(torch.where(_rows(m, objective), fresh, objective))
-    torch.cuda.current_stream().synchronize()      # the staging buffers are reused by the next call
+  def _step_rows(self, lo, hi):
+    s = self._np
+    for e in range(lo, hi):
+      if not s['mask'][e]:
+        continue
+      try:
+        state, r, t, _ = self.envs[e].process(int(s['action'][e]))
+        self._put(s['step_frames'], s['step_obj'], e, state if isinstance(state, dict) else {'image': state})
+        s['reward'][e] = r
+        s['terminal'][e] = 1 if t else 0
+        if t:
+          self.envs[e].reset()
+          self._put(s['reset_frames'], s['reset_obj'], e, self.envs[e].last_state)
+      except BaseException as ex:   # noqa: B902 -- handed to the calling thread
+        return e, ex
+    return None
+
+  def _reset_rows(self, lo, hi):
+    s = self._np
+    for e in range(lo, hi):
+      if not s['mask'][e]:
+        continue
+      try:
+        self.envs[e].reset()
+        self._put(s['reset_frames'], s['reset_obj'], e, self.envs[e].last_state)
+      except BaseException as ex:   # noqa: B902
+        return e, ex
+    return None
+
+  # ---- calling thread ---------------------------------------------------------------------------------------------
+  def _run(self, job, action, mask):
+    if self._failed is not None:
+      raise _lib.UnrealError("HostEnvProducer: env %d failed earlier; the producer takes no further calls" % self._failed)
+    self._ingested.synchronize()           # the previous ingest has finished reading the staging
+    if action is not None:
+      self._action.copy_(action, non_blocking=True)
+    if mask is not None:
+      self._mask.copy_(mask, non_blocking=True)
+    else:
+      self._np['mask'].fill(1)
+    if action is not None or mask is not None:
+      self._copied.record()
+      self._copied.synchronize()
+    out = [job(0, self.num_envs)] if self._threads is None else self._threads.run(job)
+    errors = [x for x in out if x is not None]
+    if errors:
+      e, ex = min(errors, key=lambda x: x[0])
+      self._failed = e
+      raise _lib.UnrealError("HostEnvProducer: env %d raised %s: %s" % (e, type(ex).__name__, ex)) from ex
+
+  @staticmethod
+  def _u8_mask(mask):
+    return mask if mask is None or mask.dtype == torch.uint8 else mask.to(torch.uint8)
+
+  def fused_reset(self, mask, out, objective=None, last_action=None, last_reward=None):
+    """reset() of the envs with mask[e] != 0 (None: all): first frame into out[e], objective, last_action /
+    last_reward zeroed (both nullable)."""
+    mask = self._u8_mask(mask)
+    self._run(self._reset_rows, None, mask)
+    K.host_frames_ingest(self._reset_frames, out, reset_objective=self._reset_obj, active=mask,
+                         last_action=last_action, last_reward=last_reward,
+                         objective=objective if self.objective_size else None)
+    self._ingested.record()
 
   def reset(self, mask, out, objective=None):
-    mask_host = np.ones(self.num_envs, bool) if mask is None else mask.to(torch.bool).cpu().numpy()
-    for e in np.flatnonzero(mask_host):
-      self.envs[e].reset()
-      self._put(e, self.envs[e].last_state)
-    if mask_host.any():
-      self._upload(mask_host, out, objective)
+    self.fused_reset(mask, out, objective)
 
-  def step(self, action, active, out, reward, terminal, objective=None):
-    act = action.cpu().numpy()
-    mask_host = np.ones(self.num_envs, bool) if active is None else active.to(torch.bool).cpu().numpy()
-    self._rt.zero_()
-    for e in np.flatnonzero(mask_host):
-      state, r, t, _ = self.envs[e].process(int(act[e]))
-      self._put(e, state if isinstance(state, dict) else {'image': state})
-      self._rt[e, 0] = float(r)
-      self._rt[e, 1] = 1.0 if t else 0.0
-    rt = self._rt.to(self.device, non_blocking=True)
-    reward.copy_(rt[:, 0])
-    terminal.copy_(rt[:, 1].to(torch.uint8))
-    self._upload(mask_host, out, objective)
+  def fused_step(self, action, active, prev, out, copy_inactive, pc, reward, terminal, rec, last_action, last_reward,
+                 objective=None):
+    """One step of the envs with active[e] != 0 (None: all) and everything BatchedFrameEnvironment.process does
+    around it, in one launch (unreal_host_frames_ingest)."""
+    active = self._u8_mask(active)
+    self._run(self._step_rows, action, active)
+    K.host_frames_ingest(self._reset_frames, out, step_frames=self._step_frames, step_reward=self._reward,
+                         step_terminal=self._terminal, step_objective=self._step_obj, reset_objective=self._reset_obj,
+                         action=action, active=active, prev=prev, copy_inactive=copy_inactive, pc=pc, rec=rec,
+                         reward=reward, terminal=terminal, last_action=last_action, last_reward=last_reward,
+                         objective=objective if self.objective_size else None)
+    self._ingested.record()
 
 
 class BatchedFrameEnvironment(environment.Environment):
@@ -227,6 +361,11 @@ class BatchedFrameEnvironment(environment.Environment):
       self._cur = self._obs
       self.reset()
 
+  def stop(self):
+    """Ends the producer's worker threads, if it has any."""
+    if hasattr(self.producer, 'close'):
+      self.producer.close()
+
   def _state(self, frame):
     s = {'image': frame}
     if self.objective is not None:
@@ -236,6 +375,10 @@ class BatchedFrameEnvironment(environment.Environment):
   def reset(self, mask=None):
     """reset() of the reference env classes for every env (or those with mask != 0)."""
     with torch.cuda.device(self.device):
+      if hasattr(self.producer, 'fused_reset'):
+        self.producer.fused_reset(mask, self._cur, self.objective, self.last_action, self.last_reward)
+        self.last_state = self._state(self._cur)
+        return
       self.producer.reset(mask, self._cur, self.objective)
       if mask is None:
         self.last_action.zero_(); self.last_reward.zero_()
@@ -279,8 +422,15 @@ class BatchedFrameEnvironment(environment.Environment):
     pc = self._pc if out_pc is None else out_pc
     reward = self._reward if out_reward is None else out_reward
     terminal = self._terminal if out_terminal is None else out_terminal
+    own = out_obs is self._obs or out_obs is self._next
     with torch.cuda.device(self.device):
-      if out_obs is self._obs or out_obs is self._next:
+      if hasattr(self.producer, 'fused_step'):
+        self.producer.fused_step(action, active, prev, out_obs, own, pc, reward, terminal, self.frame_rec,
+                                 self.last_action, self.last_reward, self.objective)
+        self._cur = out_obs
+        self.last_state = self._state(out_obs)
+        return self.last_state, reward, terminal, pc
+      if own:
         out_obs.copy_(prev)                    # inactive envs keep their frame (caller-supplied buffers: untouched rows)
       self.producer.step(action, active, out_obs, reward, terminal, self.objective)
       K.pixel_change(out_obs, prev, out=pc)    # environment.py:93-99

@@ -437,6 +437,38 @@ def frame_pack(action, reward, terminal, last_action=None, last_reward=None, act
   return rec
 
 
+def host_frames_ingest(reset_frames, out, step_frames=None, step_reward=None, step_terminal=None, step_objective=None,
+                       reset_objective=None, action=None, active=None, prev=None, copy_inactive=False, pc=None, rec=None,
+                       reward=None, terminal=None, last_action=None, last_reward=None, objective=None):
+  """One launch of unreal_host_frames_ingest: step mode when `prev` is given, else reset mode.  Staging (frames
+  [N,H,W,C] u8 or f32, reward [N] f32, terminal [N] u8, objectives [N,G] f32) is pinned host memory read in place;
+  everything else is on the device.  `active` [N] u8 (None: all rows) selects the stepped / reset envs."""
+  n, h, w, c = out.shape
+  if reset_frames.shape != out.shape or (step_frames is not None and step_frames.shape != out.shape):
+    raise _lib.UnrealError("host_frames_ingest: staging %s and out %s shapes differ" % (tuple(reset_frames.shape), tuple(out.shape)))
+  if step_frames is not None and step_frames.dtype != reset_frames.dtype:
+    raise _lib.UnrealError("host_frames_ingest: step and reset staging dtypes differ")
+  g = 0 if objective is None else objective.shape[1]
+  rows = [(active, (n,)), (objective, (n, g)), (reset_objective if g else None, (n, g))]
+  if prev is not None:
+    rows += [(prev, out.shape), (pc, (n, (h - 4) // 4, (w - 4) // 4)), (step_objective if g else None, (n, g))]
+    rows += [(t, (n,)) for t in (action, step_reward, step_terminal, rec, reward, terminal, last_action, last_reward)]
+  for t, shape in rows:
+    if t is not None and tuple(t.shape) != tuple(shape):
+      raise _lib.UnrealError("host_frames_ingest: a buffer of shape %s where %s is needed" % (tuple(t.shape), tuple(shape)))
+  sd = reset_frames.dtype
+  hp = _lib.host_ptr
+  call("unreal_host_frames_ingest", 1 if prev is None else 0, hp(step_frames, sd, "step_frames"),
+       hp(reset_frames, sd, "reset_frames"), _lib.dtype_tag(reset_frames), hp(step_reward, torch.float32, "step_reward"),
+       hp(step_terminal, torch.uint8, "step_terminal"), hp(step_objective if g else None, torch.float32, "step_objective"),
+       hp(reset_objective if g else None, torch.float32, "reset_objective"), ptr(action, torch.int32, "action"),
+       ptr(active, torch.uint8, "active"), ptr(prev, torch.uint8, "prev"), ptr(out, torch.uint8, "out"),
+       1 if copy_inactive else 0, ptr(pc, torch.float32, "pc"), ptr(rec, torch.int64, "rec"),
+       ptr(reward, torch.float32, "reward"), ptr(terminal, torch.uint8, "terminal"),
+       ptr(last_action, torch.int32, "last_action"), ptr(last_reward, torch.float32, "last_reward"),
+       ptr(objective, torch.float32, "objective"), n, h, w, c, g, stream_ptr())
+
+
 # ---------------------------------------------------------------------------- optimiser
 def grad_sumsq(grad, out=None):
   """sum(grad^2) as a device double; `out` (1-element float64) is accumulated into."""
